@@ -3,11 +3,15 @@
 full GFS model eval forward (DGCNN + attention + GW head, 13 classes, 150 geometric words), batch = 32 blocks of
 2048 points x 9 channels per GPU, k = 20, random-init weights.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl gfs3d|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl gfs3d|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one eval forward of the model over one batch of 32 blocks.  Blocks are independent (SURVEY.md section 8e): every
 rank processes its own 32 blocks, no data-path collective (weak scaling).  Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes the logits of the last timed step as DIR/logits.npy (float32, (blocks, classes, points);
+DIR/logits_rank<r>.npy per rank when N > 1).  Inputs and weights come from fixed seeds, so two builds run with the same
+arguments can be compared output for output.  Above 64 MB in all, a fixed seeded sample of whole blocks is written.
 """
 import argparse
 import json
@@ -395,6 +399,22 @@ def emit(line):
     out.flush()
 
 
+DUMP_BYTES = 63_000_000                  # under 64 MB (either unit) with the .npy headers
+
+
+def dump_logits(out_dir, logits, name, budget):
+    """logits (B, classes, N) -> out_dir/<name>.npy as float32; whole blocks, a fixed seeded sample of them when the batch is
+    larger than `budget` bytes (the kept block indices go to out_dir/<name>_blocks.npy as float64)"""
+    import numpy as np
+    a = logits.detach().float().cpu().numpy()
+    keep = max(1, budget // (a[0].nbytes + 8))
+    if a.shape[0] > keep:
+        blocks = np.sort(np.random.RandomState(0).choice(a.shape[0], keep, replace=False))
+        a = a[blocks]
+        np.save(os.path.join(out_dir, name + "_blocks.npy"), blocks.astype(np.float64))
+    np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def main():
     claim_stdout()
     ap = argparse.ArgumentParser()
@@ -410,7 +430,13 @@ def main():
     ap.add_argument("--kmeans-points", type=int, default=4_000_000, help="total points of the k-means leg (sharded over the ranks)")
     ap.add_argument("--e2e-serial", action="store_true",
                     help="end-to-end leg without prefetch: H2D, forward and D2H of a step strictly one after the other")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the logits of the last timed step to DIR as .npy (float32), for comparing two builds")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.impl == "reference" and a.dump_outputs:
+        ap.error("--dump-outputs writes what the gfs3d path computed; --impl reference does not support it")
     if a.impl == "reference":
         return run_reference(a)
     a.warmup = max(a.warmup, 3)
@@ -467,10 +493,14 @@ def main():
     for i in range(a.steps):
         flush.zero_()
         ev[i][0].record()
-        run(xs[i % NROT])
+        last = run(xs[i % NROT])
         ev[i][1].record()
     barrier()
     wall = time.perf_counter() - w0
+    if a.dump_outputs:                          # before the next replay overwrites the graph's static output
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        dump_logits(a.dump_outputs, last, "logits" if world == 1 else f"logits_rank{rank}", DUMP_BYTES // world)
+    last = None
     launches = (ops.LAUNCHES - l0) if graphed is None else graphed.kernels_per_replay * a.steps
     dev_ms = sum(s.elapsed_time(e) for s, e in ev)
 

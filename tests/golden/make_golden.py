@@ -215,6 +215,20 @@ def make_kmeanspp(name, n, D, K, seed, rs_seed):
          idx=idx.astype(np.int32), x_checksum=np.float64(X.astype(np.float64).sum()))
 
 
+def make_kmeans_fit_pp(name, n, D, K, seed, rs_seed):
+    """sklearn KMeans(init='k-means++', n_init=1).fit(X) end to end, as get_basis.py:210 drives it: seeding and Lloyd
+    iterations together (X regenerated from the seed by the test, not mean-centred: fit centres it itself)"""
+    import sklearn
+    from sklearn.cluster import KMeans
+    rs = np.random.RandomState(seed)
+    cent = rs.randn(K, D).astype(np.float32)
+    X = (cent[rs.randint(0, K, n)] + 0.35 * rs.randn(n, D)).astype(np.float32)
+    km = KMeans(n_clusters=K, init="k-means++", n_init=1, random_state=rs_seed).fit(X)
+    print(f"{name}: sklearn {sklearn.__version__} n_iter={km.n_iter_}")
+    save(name, seed=np.int32(seed), rs_seed=np.int32(rs_seed), n=np.int32(n), D=np.int32(D), K=np.int32(K),
+         labels=km.labels_.astype(np.int16), n_iter=np.int32(km.n_iter_), x_checksum=np.float64(X.astype(np.float64).sum()))
+
+
 def make_metric(name, seed, scannet):
     """runs/eval.py of the reference (pure numpy/Python, importable as is) on random labels"""
     from runs.eval import evaluate_metric_GFS  # noqa: E402  (reference)
@@ -373,3 +387,4 @@ if __name__ == "__main__":
     if "kmeanspp" in todo:
         make_kmeanspp("kmeanspp_n3000_k50", 3000, 192, 50, seed=2, rs_seed=102)
         make_kmeanspp("kmeanspp_n6000_k150", 6000, 192, 150, seed=5, rs_seed=105)
+        make_kmeans_fit_pp("kmeans_fit_pp_n3000_k50", 3000, 192, 50, seed=2, rs_seed=102)

@@ -137,18 +137,19 @@ def test_kmeans_plusplus_picks_sklearns_centres(golden, name):
 
 
 def test_kmeans_fit_with_plusplus_init_matches_sklearn_end_to_end(golden):
-    """get_basis.py:210 as written -- KMeans(n_clusters, init='k-means++').fit(X).labels_ -- against sklearn run with the same
-    RandomState: same seeding picks (pinned above) + same Lloyd trajectory => the same labels"""
-    from sklearn.cluster import KMeans as SK
+    """get_basis.py:210 as written -- KMeans(n_clusters, init='k-means++').fit(X).labels_ -- against the labels sklearn 1.9.0
+    gave with the same RandomState (tests/golden/make_golden.py:make_kmeans_fit_pp): same seeding picks (pinned above) + same
+    Lloyd trajectory => the same labels"""
     from gfs3d.kmeans import KMeans
-    rs = np.random.RandomState(2)
-    n, D, K = 3000, 192, 50
+    g = golden("kmeans_fit_pp_n3000_k50")
+    n, D, K = int(g["n"]), int(g["D"]), int(g["K"])
+    rs = np.random.RandomState(int(g["seed"]))
     cent = rs.randn(K, D).astype(np.float32)
     X = (cent[rs.randint(0, K, n)] + 0.35 * rs.randn(n, D)).astype(np.float32)
-    ref = SK(n_clusters=K, init="k-means++", n_init=1, random_state=102).fit(X)
-    got = KMeans(n_clusters=K, init="k-means++", random_state=102).fit(X)
-    agree = float((ref.labels_ == got.labels_).mean())
-    print(f"k-means++ + Lloyd vs sklearn: label agreement {agree:.5f}, iterations {got.n_iter_} vs {ref.n_iter_}")
+    assert abs(float(X.astype(np.float64).sum()) - float(g["x_checksum"])) < 1e-9
+    got = KMeans(n_clusters=K, init="k-means++", random_state=int(g["rs_seed"])).fit(X)
+    agree = float((g["labels"] == got.labels_).mean())
+    print(f"k-means++ + Lloyd vs sklearn: label agreement {agree:.5f}, iterations {got.n_iter_} vs {int(g['n_iter'])}")
     assert agree >= 0.999
 
 
