@@ -315,7 +315,8 @@ bn_stats_partials_kernel(const float2* __restrict__ part, int P, int64_t M, cons
 // A CTA owns ES_PPB consecutive points = ES_PPB*k consecutive edges, staged channel-major through shared memory.  The Q half
 // needs no atomics (all k edges of a point are in the tile: one plain store per channel, fixed summation order); the P half goes
 // out as 16-byte vector reductions (red.global.add.v4.f32, sm_90+): 16 per edge instead of 64 scalar atomics.  The order in which
-// different CTAs add into one dP row is not fixed -- the only non-deterministic summation of the training path.
+// different CTAs add into one dP row is not fixed -- the only non-deterministic summation of the training path; the ordered
+// scatter below (gfs_edge_scatter_bn_ordered) replaces it when the caller asks for reproducible bits.
 constexpr int ES_PPB = 8;
 
 __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
@@ -355,11 +356,15 @@ edge_scatter_kernel(const float* __restrict__ dH, const int32_t* __restrict__ id
 // The same scatter with the BatchNorm + activation backward of the layer in front of it applied on the fly: the tile is
 //   dH[c, e] = gamma[c] invstd[c] (g - sum_g[c]/E - xhat sum_gx[c]/E),   g = dy[c, e] * act'(gamma xhat + beta),  xhat = (x - mean) invstd
 // computed from dy (= d h1) and x (= H) while staging, so the (64, E) tensor dH is never written or re-read.
+// ORDERED = false: the P half goes out as red.global.add.v4.f32 (dpq's P half zeroed by the caller).
+// ORDERED = true (phase 1 of gfs_edge_scatter_bn_ordered): the P-half terms are stored edge-major instead, terms[e, 0:64] (rows of
+// 256 B, 16-byte stores); edge_gather_rows_kernel then sums them per target in ascending edge order.
+template <bool ORDERED>
 __global__ void __launch_bounds__(256)
 edge_scatter_bn_kernel(const float* __restrict__ dy, const float* __restrict__ x, const int32_t* __restrict__ idx, int N, int k, int64_t Mp,
                        int64_t E, const float* __restrict__ mean, const float* __restrict__ invstd, const float* __restrict__ gamma,
                        const float* __restrict__ beta, float slope, const float* __restrict__ sum_g, const float* __restrict__ sum_gx,
-                       float* __restrict__ dpq) {
+                       float* __restrict__ dpq, float* __restrict__ terms) {
     extern __shared__ float T[];                        // [64][EL + 1]
     __shared__ float cf[5][64];                         // mean, invstd, gamma, beta | gamma*invstd ; a ; b  (packed below)
     __shared__ float ca[64], cb[64];
@@ -401,11 +406,127 @@ edge_scatter_bn_kernel(const float* __restrict__ dy, const float* __restrict__ x
     }
     for (int t = threadIdx.x; t < ne * 16; t += 256) {
         const int el = t >> 4, q = t & 15;
-        const int64_t i = i0 + el / k;
-        const int64_t j = (i / N) * N + __ldg(idx + e0 + el);
         const float* r = T + (4 * q) * LD + el;
-        red_add_v4(dpq + j * 128 + 4 * q, r[0], r[LD], r[2 * LD], r[3 * LD]);
+        if (ORDERED) {
+            reinterpret_cast<float4*>(terms + (e0 + el) * 64)[q] = make_float4(r[0], r[LD], r[2 * LD], r[3 * LD]);
+        } else {
+            const int64_t i = i0 + el / k;
+            const int64_t j = (i / N) * N + __ldg(idx + e0 + el);
+            red_add_v4(dpq + j * 128 + 4 * q, r[0], r[LD], r[2 * LD], r[3 * LD]);
+        }
     }
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// Ordered (deterministic) scatter: reverse index of the graph + per-target sums in ascending edge order
+// ------------------------------------------------------------------------------------------------------------------
+// CSR of the incoming edges of every target, identical to a stable sort of the targets: rev_ptr[j] = sum of the in-degrees of
+// the targets before j, rev_edge[rev_ptr[j] .. rev_ptr[j+1]) = the edges e with target j in ascending order.  Every edge of block b
+// targets block b, so block b's edges fill rev_edge[b*N*k, (b+1)*N*k) and one CTA builds its block alone.  Its NW warps split the
+// block's edges into NW consecutive segments: pass 1 counts per (segment, target) in shared memory, a scan over (target, segment)
+// turns the counts into write cursors, pass 2 walks each segment again 32 edges at a time and places every edge at its cursor
+// plus its rank among the lanes with the same target (__match_any_sync).  No atomics decide an order: the result is the same
+// on every run.
+constexpr int RI_THREADS = 512;
+constexpr size_t RI_SMEM_MAX = 226 * 1024;           // dynamic part; the static wsum and the 227 KB cap leave room
+
+__global__ void __launch_bounds__(RI_THREADS)
+edge_reverse_index_kernel(const int32_t* __restrict__ idx, int N, int k, int NW, int32_t* __restrict__ rev_ptr,
+                          int32_t* __restrict__ rev_edge) {
+    extern __shared__ int32_t cnt[];                    // [NW][N]
+    __shared__ int32_t wsum[RI_THREADS / 32];
+    const int b = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int64_t EB = (int64_t)N * k, base = (int64_t)b * EB;
+    const int32_t* ib = idx + base;
+    const int64_t seg = (EB + NW - 1) / NW;
+    const int64_t lo = warp < NW ? (int64_t)warp * seg : EB, hi = lo + seg < EB ? lo + seg : EB;
+    for (int i = tid; i < NW * N; i += RI_THREADS) cnt[i] = 0;
+    __syncthreads();
+    for (int64_t e = lo + lane; e < hi; e += 32) atomicAdd(&cnt[warp * N + __ldg(ib + e)], 1);   // integer counts: order-free
+    __syncthreads();
+    // thread t owns targets [t*R, t*R + R): exclusive prefix over the segments, then over the targets (block-wide scan)
+    const int R = (N + RI_THREADS - 1) / RI_THREADS;
+    const int l0 = tid * R < N ? tid * R : N, l1 = l0 + R < N ? l0 + R : N;
+    int own = 0;
+    for (int l = l0; l < l1; ++l) {
+        int run = 0;
+        for (int w = 0; w < NW; ++w) {
+            const int c = cnt[w * N + l];
+            cnt[w * N + l] = run;
+            run += c;
+        }
+        rev_ptr[(int64_t)b * N + l] = run;              // in-degree, replaced by the start below
+        own += run;
+    }
+    int inc = own;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += v;
+    }
+    if (lane == 31) wsum[warp] = inc;
+    __syncthreads();
+    int before = inc - own;
+    for (int w = 0; w < warp; ++w) before += wsum[w];
+    int64_t start = base + before;
+    for (int l = l0; l < l1; ++l) {
+        const int deg = rev_ptr[(int64_t)b * N + l];
+        rev_ptr[(int64_t)b * N + l] = (int32_t)start;
+        for (int w = 0; w < NW; ++w) cnt[w * N + l] += (int32_t)start;
+        start += deg;
+    }
+    if (b == gridDim.x - 1 && tid == 0) rev_ptr[(int64_t)gridDim.x * N] = (int32_t)(base + EB);
+    __syncthreads();
+    if (warp >= NW) return;
+    const unsigned lt = (1u << lane) - 1u;
+    for (int64_t e0 = lo; e0 < hi; e0 += 32) {
+        const int64_t e = e0 + lane;
+        const int l = e < hi ? __ldg(ib + e) : -1 - lane;          // lanes past the segment: a key no other lane has
+        const unsigned same = __match_any_sync(0xffffffffu, l);
+        if (e < hi) {
+            const int at = cnt[warp * N + l];
+            rev_edge[at + __popc(same & lt)] = (int32_t)(base + e);
+            __syncwarp(same);
+            if ((same & lt) == 0) cnt[warp * N + l] = at + __popc(same);   // the lowest lane of each group advances the cursor
+        }
+        __syncwarp();
+    }
+}
+
+// Phase 2 of the ordered scatter: dpq[j, 0:64] = sum over r of terms[rev_edge[r], 0:64], r ascending from rev_ptr[j], starting
+// from +0.0.  Half a warp per target, a float4 (four channels) per lane; the edge ids and rows of ES_AHEAD edges are loaded
+// before their adds, so a long list is bound by load latency per batch, not per edge.
+constexpr int ES_AHEAD = 8;
+
+__global__ void __launch_bounds__(256)
+edge_gather_rows_kernel(const float* __restrict__ terms, const int32_t* __restrict__ rev_ptr, const int32_t* __restrict__ rev_edge,
+                        int64_t Mp, float* __restrict__ dpq) {
+    const int64_t j = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 4;
+    const int q = threadIdx.x & 15;
+    if (j >= Mp) return;
+    const int32_t s = __ldg(rev_ptr + j), t = __ldg(rev_ptr + j + 1);
+    float4 acc = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    int32_t r = s;
+    for (; r + ES_AHEAD <= t; r += ES_AHEAD) {
+        float4 v[ES_AHEAD];
+#pragma unroll
+        for (int u = 0; u < ES_AHEAD; ++u) v[u] = __ldg(reinterpret_cast<const float4*>(terms + (int64_t)__ldg(rev_edge + r + u) * 64) + q);
+#pragma unroll
+        for (int u = 0; u < ES_AHEAD; ++u) {
+            acc.x += v[u].x;
+            acc.y += v[u].y;
+            acc.z += v[u].z;
+            acc.w += v[u].w;
+        }
+    }
+    for (; r < t; ++r) {
+        const float4 v = __ldg(reinterpret_cast<const float4*>(terms + (int64_t)__ldg(rev_edge + r) * 64) + q);
+        acc.x += v.x;
+        acc.y += v.y;
+        acc.z += v.z;
+        acc.w += v.w;
+    }
+    reinterpret_cast<float4*>(dpq + j * 128)[q] = acc;
 }
 
 // y[c, i] = max_slot a[c, i*k + slot] (first maximum), arg[c, i] = slot
@@ -642,10 +763,56 @@ extern "C" int gfs_edge_scatter_bn(const float* dy, const float* x, const int32_
     GFS_REQUIRE(k <= 64, GFS_ERR_UNSUPPORTED, "gfs_edge_scatter_bn: k <= 64");
     const int64_t Mp = (int64_t)B * N, E = Mp * k;
     const size_t smem = (size_t)64 * (ES_PPB * k + 1) * sizeof(float);
-    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(edge_scatter_bn_kernel), (size_t)64 * (ES_PPB * 64 + 1) * sizeof(float)));
-    edge_scatter_bn_kernel<<<(unsigned)((Mp + ES_PPB - 1) / ES_PPB), 256, smem, static_cast<cudaStream_t>(stream)>>>(
-        dy, x, idx, N, k, Mp, E, mean, invstd, gamma, beta, slope, sum_g, sum_gx, dpq);
+    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(edge_scatter_bn_kernel<false>), (size_t)64 * (ES_PPB * 64 + 1) * sizeof(float)));
+    edge_scatter_bn_kernel<false><<<(unsigned)((Mp + ES_PPB - 1) / ES_PPB), 256, smem, static_cast<cudaStream_t>(stream)>>>(
+        dy, x, idx, N, k, Mp, E, mean, invstd, gamma, beta, slope, sum_g, sum_gx, dpq, nullptr);
     GFS_LAUNCH_OK("edge_scatter_bn_kernel");
+    return GFS_OK;
+}
+
+// shared-memory budget of the reverse index: NW segment counters of N ints per CTA
+static int reverse_index_segments(int N) {
+    const int64_t fit = (int64_t)(RI_SMEM_MAX / sizeof(int32_t)) / N;
+    return (int)(fit < RI_THREADS / 32 ? fit : RI_THREADS / 32);
+}
+
+extern "C" int gfs_edge_reverse_index(const int32_t* idx, int B, int N, int k, int32_t* rev_ptr, int32_t* rev_edge, void* stream) {
+    GFS_REQUIRE(idx && rev_ptr && rev_edge, GFS_ERR_BAD_ARG, "gfs_edge_reverse_index: null pointer");
+    GFS_REQUIRE(B > 0 && N > 0 && k > 0, GFS_ERR_BAD_ARG, "gfs_edge_reverse_index: non-positive size (B=%d N=%d k=%d)", B, N, k);
+    GFS_REQUIRE(k <= 64, GFS_ERR_UNSUPPORTED, "gfs_edge_reverse_index: k=%d > 64 is not built", k);
+    GFS_REQUIRE((int64_t)B * N * k < ((int64_t)1 << 31), GFS_ERR_UNSUPPORTED,
+                "gfs_edge_reverse_index: E = B*N*k = %lld edges >= 2^31 (int32 edge ids)", (long long)B * N * k);
+    const int NW = reverse_index_segments(N);
+    GFS_REQUIRE(NW >= 1, GFS_ERR_UNSUPPORTED, "gfs_edge_reverse_index: N=%d > %d (per-target counters live in shared memory)", N,
+                (int)(RI_SMEM_MAX / sizeof(int32_t)));
+    const size_t smem = (size_t)NW * N * sizeof(int32_t);
+    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(edge_reverse_index_kernel), RI_SMEM_MAX));
+    edge_reverse_index_kernel<<<B, RI_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(idx, N, k, NW, rev_ptr, rev_edge);
+    GFS_LAUNCH_OK("edge_reverse_index_kernel");
+    return GFS_OK;
+}
+
+extern "C" int gfs_edge_scatter_bn_ordered(const float* dy, const float* x, const int32_t* idx, const int32_t* rev_ptr,
+                                           const int32_t* rev_edge, int B, int N, int k, const float* mean, const float* invstd,
+                                           const float* gamma, const float* beta, float slope, const float* sum_g, const float* sum_gx,
+                                           float* edge_terms, float* dpq, void* stream) {
+    GFS_REQUIRE(dy && x && idx && rev_ptr && rev_edge && mean && invstd && gamma && beta && sum_g && sum_gx && edge_terms && dpq,
+                GFS_ERR_BAD_ARG, "gfs_edge_scatter_bn_ordered: null pointer");
+    GFS_REQUIRE(B > 0 && N > 0 && k > 0, GFS_ERR_BAD_ARG, "gfs_edge_scatter_bn_ordered: non-positive size (B=%d N=%d k=%d)", B, N, k);
+    GFS_REQUIRE(k <= 64, GFS_ERR_UNSUPPORTED, "gfs_edge_scatter_bn_ordered: k=%d > 64 is not built", k);
+    GFS_REQUIRE((int64_t)B * N * k < ((int64_t)1 << 31), GFS_ERR_UNSUPPORTED,
+                "gfs_edge_scatter_bn_ordered: E = B*N*k = %lld edges >= 2^31 (int32 edge ids)", (long long)B * N * k);
+    GFS_REQUIRE(((reinterpret_cast<uintptr_t>(edge_terms) | reinterpret_cast<uintptr_t>(dpq)) & 15) == 0, GFS_ERR_BAD_ARG,
+                "gfs_edge_scatter_bn_ordered: edge_terms and dpq must be 16-byte aligned");
+    const int64_t Mp = (int64_t)B * N, E = Mp * k;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t smem = (size_t)64 * (ES_PPB * k + 1) * sizeof(float);
+    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(edge_scatter_bn_kernel<true>), (size_t)64 * (ES_PPB * 64 + 1) * sizeof(float)));
+    edge_scatter_bn_kernel<true><<<(unsigned)((Mp + ES_PPB - 1) / ES_PPB), 256, smem, st>>>(
+        dy, x, idx, N, k, Mp, E, mean, invstd, gamma, beta, slope, sum_g, sum_gx, dpq, edge_terms);
+    GFS_LAUNCH_OK("edge_scatter_bn_kernel<ordered>");
+    edge_gather_rows_kernel<<<(unsigned)((Mp * 16 + 255) / 256), 256, 0, st>>>(edge_terms, rev_ptr, rev_edge, Mp, dpq);
+    GFS_LAUNCH_OK("edge_gather_rows_kernel");
     return GFS_OK;
 }
 

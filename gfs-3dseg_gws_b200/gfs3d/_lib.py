@@ -45,6 +45,8 @@ SIGNATURES = {
     "gfs_bn_act_max_fwd": [_p, _i, _i64, _i, _p, _p, _f, _p, _i64, _p, _p],
     "gfs_bn_bwd_sums": [_p, _i64, _p, _i64, _i, _i64, _p, _p, _p, _p, _f, _p, _p, _p, _p],
     "gfs_edge_scatter_bn": [_p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _f, _p, _p, _p, _p],
+    "gfs_edge_reverse_index": [_p, _i, _i, _i, _p, _p, _p],
+    "gfs_edge_scatter_bn_ordered": [_p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p],
     "gfs_bn_act_bwd": [_p, _i64, _p, _i64, _p, _i64, _i, _i64, _p, _p, _p, _p, _f, _p, _p, _p, _p],
     "gfs_bn_act_bwd_argmax": [_p, _i64, _p, _i, _p, _i64, _p, _i64, _i, _i64, _p, _p, _p, _p, _f, _p, _p, _p, _p],
     "gfs_edge_gather": [_p, _p, _i, _i, _i, _p, _p],

@@ -541,12 +541,36 @@ def bn_bwd_sums(dy, x, mean, invstd, gamma, beta, slope):
     return sg, sgx
 
 
-def edge_scatter_bn(dy, x, idx, B, N, k, mean, invstd, gamma, beta, slope, sg, sgx):
-    """edge_scatter(bn_act_bwd(dy, x, ...).dx) without the (64, E) tensor in between; dy, x (64, E) contiguous"""
+def edge_reverse_index(idx, B, N):
+    """incoming edges of every target of the graph idx (B, N, k) int32 -> rev_ptr (B*N + 1), rev_edge (B*N*k) int32: the edges of
+    target j = b*N + idx[e] are rev_edge[rev_ptr[j]:rev_ptr[j+1]] in ascending edge index (a stable sort of the targets)"""
+    _need_cuda(idx)
+    k = idx.shape[-1]
+    assert idx.dtype == torch.int32 and idx.is_contiguous() and idx.numel() == B * N * k
+    rev_ptr = torch.empty(B * N + 1, dtype=torch.int32, device=idx.device)
+    rev_edge = torch.empty(B * N * k, dtype=torch.int32, device=idx.device)
+    _call("gfs_edge_reverse_index", 1, _ptr(idx), B, N, k, _ptr(rev_ptr), _ptr(rev_edge), _stream())
+    return rev_ptr, rev_edge
+
+
+def edge_scatter_bn(dy, x, idx, B, N, k, mean, invstd, gamma, beta, slope, sg, sgx, ordered=False, rev=None, edge_terms=None):
+    """edge_scatter(bn_act_bwd(dy, x, ...).dx) without the (64, E) tensor in between; dy, x (64, E) contiguous.
+    ordered=True: the P half is summed per target in ascending edge order (gfs_edge_scatter_bn_ordered), the same bits on every
+    run.  rev: the graph's edge_reverse_index (built here if None); edge_terms: optional (E, 64) fp32 buffer for the per-edge terms"""
     assert dy.is_contiguous() and x.is_contiguous() and dy.shape == x.shape and dy.shape[0] == 64
-    dpq = torch.zeros(B * N, 128, dtype=torch.float32, device=dy.device)
-    _call("gfs_edge_scatter_bn", 1, _ptr(dy), _ptr(x), _ptr(idx), B, N, k, _ptr(mean), _ptr(invstd), _ptr(gamma), _ptr(beta),
-          float(slope), _ptr(sg), _ptr(sgx), _ptr(dpq), _stream())
+    if not ordered:
+        dpq = torch.zeros(B * N, 128, dtype=torch.float32, device=dy.device)
+        _call("gfs_edge_scatter_bn", 1, _ptr(dy), _ptr(x), _ptr(idx), B, N, k, _ptr(mean), _ptr(invstd), _ptr(gamma), _ptr(beta),
+              float(slope), _ptr(sg), _ptr(sgx), _ptr(dpq), _stream())
+        return dpq
+    rev_ptr, rev_edge = edge_reverse_index(idx, B, N) if rev is None else rev
+    E = B * N * k
+    if edge_terms is None:
+        edge_terms = torch.empty(E, 64, dtype=torch.float32, device=dy.device)
+    assert edge_terms.dtype == torch.float32 and edge_terms.is_contiguous() and edge_terms.shape == (E, 64)
+    dpq = torch.empty(B * N, 128, dtype=torch.float32, device=dy.device)
+    _call("gfs_edge_scatter_bn_ordered", 2, _ptr(dy), _ptr(x), _ptr(idx), _ptr(rev_ptr), _ptr(rev_edge), B, N, k, _ptr(mean),
+          _ptr(invstd), _ptr(gamma), _ptr(beta), float(slope), _ptr(sg), _ptr(sgx), _ptr(edge_terms), _ptr(dpq), _stream())
     return dpq
 
 

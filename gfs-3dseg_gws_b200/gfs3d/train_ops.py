@@ -139,7 +139,13 @@ class EdgeConvTrain(torch.autograd.Function):
         del dZ
         # BN1 / LeakyReLU backward is applied inside the scatter while its tile is staged: dH (64, E) is never built
         sg1, sgx1 = ops.bn_bwd_sums(dh1, H, m1, is1, g1, b1, 0.2)
-        dpq = ops.edge_scatter_bn(dh1, H, idx, B, N, k, m1, is1, g1, b1, 0.2, sg1, sgx1)   # (M, 128): scatter-add over the graph
+        if torch.are_deterministic_algorithms_enabled():
+            # reproducible bits: each dP row is summed in ascending edge order instead of by atomics (one (E, 64) buffer of
+            # per-edge terms lives until the scatter returns)
+            dpq = ops.edge_scatter_bn(dh1, H, idx, B, N, k, m1, is1, g1, b1, 0.2, sg1, sgx1, ordered=True,
+                                      rev=ops.edge_reverse_index(idx, B, N))
+        else:
+            dpq = ops.edge_scatter_bn(dh1, H, idx, B, N, k, m1, is1, g1, b1, 0.2, sg1, sgx1)   # (M, 128): scatter-add over the graph
         del dh1
         dWpq = torch.empty(128, C, dtype=torch.float32, device=x.device)
         ops.gemm_f32(dpq, 128, False, x, M, True, 128, C, M, dWpq, C, splitk=ops._splitk(M), impl=_exact())

@@ -264,14 +264,23 @@ class mpti_net_Point_GeoAsWeight_v2(nn.Module):
         ori_proto, fake_novel = self.generate_fake_proto(x=point_feat[fake_num:], y=y[fake_num:], main_proto=self.main_proto.clone(),
                                                          xn=xn[fake_num:])
         x_pre_1 = self.get_pred(x=point_feat, proto=ori_proto, use_bg_proto=True, xn=xn)
-        loss_ce_1 = self.criterion(x_pre_1, y)
+        loss_ce_1 = self._loss(x_pre_1, y)
         refine_proto = self.post_refine_proto_v2(proto=self.main_proto.clone(), x=point_feat, point_feat=point_feat, use_bg_proto=True, xn=xn)
         post_refine_proto = refine_proto.clone()
         post_refine_proto[:, :base_num] = post_refine_proto[:, :base_num] + ori_proto[:base_num].unsqueeze(0)
         post_refine_proto[:, base_num:] = post_refine_proto[:, base_num:] * 0 + ori_proto[base_num:].unsqueeze(0)
         x_pre_2 = self.get_pred(x=point_feat, proto=post_refine_proto, use_bg_proto=True, xn=xn)
-        loss_ce_2 = self.criterion(x_pre_2, y)
+        loss_ce_2 = self._loss(x_pre_2, y)
         return x_pre_2.max(1)[1], 0.5 * loss_ce_2 + 0.5 * loss_ce_1
+
+    def _loss(self, logits, y):
+        """self.criterion(logits (b, cls, n), y (b, n)).  torch's CUDA loss for the (b, cls, n) layout (nll_loss2d) adds the
+        per-block partial sums with atomics; under torch.use_deterministic_algorithms a CrossEntropyLoss is evaluated on the
+        (b*n, cls) view instead, whose reduction runs in a fixed order: the same loss, reproducible to the bit."""
+        if (torch.are_deterministic_algorithms_enabled() and logits.is_cuda and isinstance(self.criterion, nn.CrossEntropyLoss)
+                and self.criterion.reduction != "none"):
+            return self.criterion(logits.transpose(1, 2).reshape(-1, logits.shape[1]), y.reshape(-1))
+        return self.criterion(logits, y)
 
     def generate_fake_proto(self, x, y, main_proto, fake_novel=None, post_processing=False, xn=None):
         """model/capl.py:364-411 (training only): half of the classes present in the support half-batch are declared

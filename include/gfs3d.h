@@ -308,6 +308,23 @@ int gfs_edge_scatter_bn(const float* dy, const float* x, const int32_t* idx, int
                         const float* invstd, const float* gamma, const float* beta, float slope, const float* sum_g,
                         const float* sum_gx, float* dpq, void* stream);
 
+/* Deterministic variant of gfs_edge_scatter_bn: the backward of the neighbour gather of model/dgcnn.py:38-41 summed in a fixed order.
+ * Edge e = i*k + slot of point i (block b = i / N) targets j = b*N + idx[e]; idx values lie in [0, N).
+ *   gfs_edge_reverse_index       CSR of the incoming edges, identical to a stable sort of the targets: rev_ptr (B*N + 1 int32)
+ *                                holds the exclusive scan of the in-degrees, rev_edge (E = B*N*k int32) the edges of each target in
+ *                                ascending edge index.  Built without order-dependent atomics: the same on every run.
+ *                                N <= 57 856 (per-target counters in shared memory).
+ *   gfs_edge_scatter_bn_ordered  dpq (M, 128), every element written (no zeroing needed).  Q half (c >= 64): exactly as
+ *                                gfs_edge_scatter_bn.  P half: dpq[j, c] = fp32 sum, left to right from +0.0, of t[e, c] over the
+ *                                edges of target j in ascending edge index (a target without incoming edges gets +0.0), where
+ *                                t[e, c] is the per-edge BatchNorm / activation backward term gfs_edge_scatter_bn adds.  The terms
+ *                                are first stored to edge_terms (E x 64 fp32, caller-owned, 16-byte aligned), then summed per target.
+ * Both reject k > 64 and E >= 2^31 with GFS_ERR_UNSUPPORTED.                                                                      */
+int gfs_edge_reverse_index(const int32_t* idx, int B, int N, int k, int32_t* rev_ptr, int32_t* rev_edge, void* stream);
+int gfs_edge_scatter_bn_ordered(const float* dy, const float* x, const int32_t* idx, const int32_t* rev_ptr, const int32_t* rev_edge,
+                                int B, int N, int k, const float* mean, const float* invstd, const float* gamma, const float* beta,
+                                float slope, const float* sum_g, const float* sum_gx, float* edge_terms, float* dpq, void* stream);
+
 /* edge tensor of model/dgcnn.py:35-41 after the split first conv: H[c, e] = P[j(e), c] + Q[i(e), c]  (pq point-major (M,128)) */
 int gfs_edge_gather(const float* pq, const int32_t* idx, int B, int N, int k, float* H, void* stream);
 /* the same plus the batch statistics of H and the BatchNorm coefficients (as gfs_bn_stats_coeffs) taken while the tiles are on

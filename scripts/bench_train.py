@@ -4,8 +4,12 @@ forward + backward + Adam, data-parallel with one flat-bucket NCCL gradient all-
 
     python scripts/bench_train.py [--batch 32] [--steps 10]
     torchrun --nproc-per-node N scripts/bench_train.py
+    python scripts/bench_train.py --deterministic
 
-Prints one JSON line (ms/step max over ranks, blocks/s whole job).  Attention dropout stays ON (p = 0.1) as in training."""
+Prints one JSON line (ms/step max over ranks, blocks/s whole job).  Attention dropout stays ON (p = 0.1) as in training.
+--deterministic (one GPU): times the default step and the step under torch.use_deterministic_algorithms(True, warn_only=True),
+with torch's NaN fill of uninitialised memory on and off, alternately for three rounds, and reports the ordered-scatter
+entry points' times next to the atomic scatter's."""
 import argparse
 import json
 import os
@@ -28,6 +32,7 @@ ap.add_argument("--batch", type=int, default=32)
 ap.add_argument("--steps", type=int, default=10)
 ap.add_argument("--warmup", type=int, default=3)
 ap.add_argument("--npts", type=int, default=2048)
+ap.add_argument("--deterministic", action="store_true", help="compare the default and the deterministic step (one GPU)")
 a = ap.parse_args()
 world, rank, local = int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0))
 torch.cuda.set_device(local)
@@ -60,6 +65,59 @@ def step(i):
     opt.step()
     return loss, n
 
+
+def bench_deterministic():
+    import subprocess
+    import warnings
+    warnings.filterwarnings("ignore", message=".*deterministic.*")        # torch's alerts for its own ops (warn_only)
+    modes = {"default": (False, True), "deterministic": (True, True), "deterministic_no_fill": (True, False)}
+
+    def set_mode(name):
+        on, fill = modes[name]
+        torch.use_deterministic_algorithms(on, warn_only=True)
+        torch.utils.deterministic.fill_uninitialized_memory = fill
+
+    for name in modes:
+        set_mode(name)
+        for i in range(a.warmup):
+            step(i)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    rounds = {name: [] for name in modes}
+    for _ in range(3):
+        for name in modes:
+            set_mode(name)
+            torch.cuda.synchronize()
+            e0.record()
+            for i in range(a.steps):
+                step(i)
+            e1.record()
+            torch.cuda.synchronize()
+            rounds[name].append(round(e0.elapsed_time(e1) / a.steps, 3))
+    scatter = {}
+    for name in ("default", "deterministic"):
+        set_mode(name)
+        ops.PROFILE = {}
+        step(0)
+        torch.cuda.synchronize()
+        scatter[name] = {k: round(sum(s_.elapsed_time(e_) for s_, e_ in v), 3) for k, v in ops.PROFILE.items()
+                         if k.startswith(("gfs_edge_scatter", "gfs_edge_reverse"))}
+        ops.PROFILE = None
+    set_mode("default")
+    smi = subprocess.run(["nvidia-smi", "-i", str(local), "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                         text=True).stdout.strip()
+    print(json.dumps({"metric": "gfs_train_step_ms_deterministic", "ms_per_step_rounds": rounds,
+                      "ms_per_step_median": {k: sorted(v)[1] for k, v in rounds.items()},
+                      "scatter_entry_ms_per_step": scatter, "steps_per_round": a.steps, "batch": a.batch, "npts": a.npts,
+                      "gpu": torch.cuda.get_device_name(dev), "nvidia_smi_name_power_limit": smi,
+                      "peak_mem_gb": torch.cuda.max_memory_allocated() / 1e9,
+                      "config": "ScanNet-shaped: 21 classes, 180 GWs, base_num 15, fwd+bwd+Adam, attention dropout 0.1"}))
+
+
+if a.deterministic:
+    if world > 1:
+        sys.exit("--deterministic runs on one GPU")
+    bench_deterministic()
+    sys.exit(0)
 
 for i in range(a.warmup):
     step(i)
