@@ -14,20 +14,33 @@ constexpr int KM_THREADS = 288;    // warps 0-7: one thread per feature column; 
 
 // X is row-major, so a chunk of 32 points is ONE contiguous cp.async.bulk (TMA) of 32*D*4 bytes; two chunks are in flight
 // while the column threads add the current one into the shared-memory table.
+//
+// WEIGHTED (sklearn _k_means_lloyd.pyx:216-218, sums[l] += x * w, wsum[l] += w): the helper warp stages the chunk's 32
+// weights next to its labels, the column threads add __fmul_rn(x, w) with __fadd_rn (a product, then an add: no fused
+// multiply-add, as sklearn's C), and the helper warp's lane 0 adds the weights into a per-CTA fp64 table in ascending
+// point order instead of counting.  The unweighted instance is the kernel as it was.
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(KM_THREADS, 1)
-kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32_t* __restrict__ labels, int K,
-                      float* __restrict__ partial, int32_t* __restrict__ pcount) {
+kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32_t* __restrict__ labels,
+                      const float* __restrict__ weights, int K, float* __restrict__ partial, int32_t* __restrict__ pcount,
+                      double* __restrict__ pweight) {
     extern __shared__ __align__(128) unsigned char sm_raw[];
     float* stg = reinterpret_cast<float*>(sm_raw);                          // [2][KM_CH][D]   (first: keeps 128 B alignment)
     float* tab = stg + 2 * KM_CH * D;                                       // [K][D]
-    int* cnt = reinterpret_cast<int*>(tab + (size_t)K * D);                 // [K]
-    int* lab = cnt + ((K + 3) & ~3);                                        // [2][KM_CH]
-    uint64_t* full = reinterpret_cast<uint64_t*>(lab + 2 * KM_CH);          // [2]
+    int* cnt = reinterpret_cast<int*>(tab + (size_t)K * D);                 // [K]            (unweighted)
+    double* wtab = reinterpret_cast<double*>(tab + (size_t)K * D);          // [K] fp64       (weighted)
+    int* lab = WEIGHTED ? reinterpret_cast<int*>(wtab + K) : cnt + ((K + 3) & ~3);   // [2][KM_CH]
+    float* wst = reinterpret_cast<float*>(lab + 2 * KM_CH);                 // [2][KM_CH]     (weighted)
+    uint64_t* full = reinterpret_cast<uint64_t*>(WEIGHTED ? reinterpret_cast<int*>(wst + 2 * KM_CH) : lab + 2 * KM_CH);  // [2]
     const int tid = threadIdx.x, lane = tid & 31;
     const bool helper = tid >= 256;
 
     for (int i = tid; i < K * D; i += KM_THREADS) tab[i] = 0.0f;
-    for (int i = tid; i < K; i += KM_THREADS) cnt[i] = 0;
+    if constexpr (WEIGHTED) {
+        for (int i = tid; i < K; i += KM_THREADS) wtab[i] = 0.0;
+    } else {
+        for (int i = tid; i < K; i += KM_THREADS) cnt[i] = 0;
+    }
     if (tid == 0) {
         mbar_init(&full[0], 1);
         mbar_init(&full[1], 1);
@@ -46,6 +59,7 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
             const int64_t p0 = i0 + (int64_t)c * KM_CH;
             const int cc = (int)((i1 - p0) < KM_CH ? (i1 - p0) : KM_CH);
             lab[(c & 1) * KM_CH + lane] = lane < cc ? labels[p0 + lane] : 0;
+            if constexpr (WEIGHTED) wst[(c & 1) * KM_CH + lane] = lane < cc ? weights[p0 + lane] : 0.0f;
             if (lane == 0) {
                 const uint32_t bytes = (uint32_t)cc * (uint32_t)D * 4u;
                 mbar_arrive_expect_tx(&full[c & 1], bytes);
@@ -68,19 +82,41 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
             const int d = tid;
             if (d < D) {
                 const float* S = stg + (size_t)(c & 1) * KM_CH * D + d;
-                int j = 0;
-                for (; j + 1 < cc; j += 2) {      // ascending point order; two independent read-modify-writes when labels differ
-                    const int l0 = L[j], l1 = L[j + 1];
-                    const float v0 = S[j * D], v1 = S[(j + 1) * D];
-                    if (l0 != l1) {
-                        const float a = tab[l0 * D + d], b = tab[l1 * D + d];
-                        tab[l0 * D + d] = a + v0;
-                        tab[l1 * D + d] = b + v1;
-                    } else {
-                        tab[l0 * D + d] = (tab[l0 * D + d] + v0) + v1;
+                if constexpr (WEIGHTED) {
+                    const float* W = wst + (c & 1) * KM_CH;
+                    int j = 0;
+                    for (; j + 1 < cc; j += 2) {  // the same pairwise order as the unweighted instance
+                        const int l0 = L[j], l1 = L[j + 1];
+                        const float v0 = __fmul_rn(S[j * D], W[j]), v1 = __fmul_rn(S[(j + 1) * D], W[j + 1]);
+                        if (l0 != l1) {
+                            const float a = tab[l0 * D + d], b = tab[l1 * D + d];
+                            tab[l0 * D + d] = __fadd_rn(a, v0);
+                            tab[l1 * D + d] = __fadd_rn(b, v1);
+                        } else {
+                            tab[l0 * D + d] = __fadd_rn(__fadd_rn(tab[l0 * D + d], v0), v1);
+                        }
                     }
+                    if (j < cc) tab[L[j] * D + d] = __fadd_rn(tab[L[j] * D + d], __fmul_rn(S[j * D], W[j]));
+                } else {
+                    int j = 0;
+                    for (; j + 1 < cc; j += 2) {      // ascending point order; two independent read-modify-writes when labels differ
+                        const int l0 = L[j], l1 = L[j + 1];
+                        const float v0 = S[j * D], v1 = S[(j + 1) * D];
+                        if (l0 != l1) {
+                            const float a = tab[l0 * D + d], b = tab[l1 * D + d];
+                            tab[l0 * D + d] = a + v0;
+                            tab[l1 * D + d] = b + v1;
+                        } else {
+                            tab[l0 * D + d] = (tab[l0 * D + d] + v0) + v1;
+                        }
+                    }
+                    if (j < cc) tab[L[j] * D + d] += S[j * D];
                 }
-                if (j < cc) tab[L[j] * D + d] += S[j * D];
+            }
+        } else if constexpr (WEIGHTED) {
+            if (lane == 0) {                      // fp64, ascending point order: no floating-point atomics
+                const float* W = wst + (c & 1) * KM_CH;
+                for (int j = 0; j < cc; ++j) wtab[L[j]] += (double)W[j];
             }
         } else if (lane < cc) {
             atomicAdd(&cnt[L[lane]], 1);
@@ -91,7 +127,11 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
     __syncthreads();
     float* o = partial + (size_t)blockIdx.x * K * D;
     for (int i = tid; i < K * D; i += KM_THREADS) o[i] = tab[i];
-    for (int i = tid; i < K; i += KM_THREADS) pcount[(size_t)blockIdx.x * K + i] = cnt[i];
+    if constexpr (WEIGHTED) {
+        for (int i = tid; i < K; i += KM_THREADS) pweight[(size_t)blockIdx.x * K + i] = wtab[i];
+    } else {
+        for (int i = tid; i < K; i += KM_THREADS) pcount[(size_t)blockIdx.x * K + i] = cnt[i];
+    }
 }
 
 __global__ void kmeans_reduce_kernel(const float* __restrict__ partial, const int32_t* __restrict__ pcount, int P, int KD, int K,
@@ -106,6 +146,22 @@ __global__ void kmeans_reduce_kernel(const float* __restrict__ partial, const in
         int64_t c = 0;
         for (int p = 0; p < P; ++p) c += pcount[(size_t)p * K + i];
         counts[i] = c;
+    }
+}
+
+// weighted: the same CTA-order fp64 reduction; the per-CTA weight sums are fp64 already
+__global__ void kmeans_reduce_weighted_kernel(const float* __restrict__ partial, const double* __restrict__ pweight, int P, int KD,
+                                              int K, double* __restrict__ sums, double* __restrict__ wsums) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < KD) {
+        double acc = 0.0;
+        for (int p = 0; p < P; ++p) acc += (double)partial[(size_t)p * KD + i];
+        sums[i] = acc;
+    }
+    if (i < K) {
+        double w = 0.0;
+        for (int p = 0; p < P; ++p) w += pweight[(size_t)p * K + i];
+        wsums[i] = w;
     }
 }
 
@@ -125,11 +181,32 @@ extern "C" int gfs_kmeans_accumulate(const float* X, int64_t n, int D, const int
     const int P = sm_count();
     GFS_REQUIRE(P > 0, GFS_ERR_CUDA, "gfs_kmeans_accumulate: cannot query the device");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_kernel), 220 * 1024));
-    kmeans_partial_kernel<<<P, KM_THREADS, smem, st>>>(X, n, D, labels, K, partial, pcount);
+    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_kernel<false>), 220 * 1024));
+    kmeans_partial_kernel<false><<<P, KM_THREADS, smem, st>>>(X, n, D, labels, nullptr, K, partial, pcount, nullptr);
     GFS_LAUNCH_OK("kmeans_partial_kernel");
     kmeans_reduce_kernel<<<(K * D + 255) / 256, 256, 0, st>>>(partial, pcount, P, K * D, K, sums, counts);
     GFS_LAUNCH_OK("kmeans_reduce_kernel");
+    return GFS_OK;
+}
+
+extern "C" int gfs_kmeans_accumulate_weighted(const float* X, int64_t n, int D, const int32_t* labels, const float* weights, int K,
+                                              float* partial, double* pweight, double* sums, double* wsums, void* stream) {
+    using namespace gfs;
+    GFS_REQUIRE(X && labels && weights && partial && pweight && sums && wsums, GFS_ERR_BAD_ARG,
+                "gfs_kmeans_accumulate_weighted: null pointer");
+    GFS_REQUIRE(n > 0 && D > 0 && K > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_accumulate_weighted: non-positive size");
+    GFS_REQUIRE(D <= 256 && D % 4 == 0, GFS_ERR_UNSUPPORTED, "gfs_kmeans_accumulate_weighted: D=%d must be a multiple of 4, <= 256", D);
+    GFS_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15) == 0, GFS_ERR_BAD_ARG, "gfs_kmeans_accumulate_weighted: X must be 16-byte aligned");
+    const size_t smem = (size_t)(2 * KM_CH + K) * D * sizeof(float) + (size_t)K * sizeof(double) + 2 * KM_CH * (sizeof(int) + sizeof(float)) + 64;
+    GFS_REQUIRE(smem <= 220 * 1024, GFS_ERR_UNSUPPORTED, "gfs_kmeans_accumulate_weighted: K*D=%d does not fit shared memory", K * D);
+    const int P = sm_count();
+    GFS_REQUIRE(P > 0, GFS_ERR_CUDA, "gfs_kmeans_accumulate_weighted: cannot query the device");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_kernel<true>), 220 * 1024));
+    kmeans_partial_kernel<true><<<P, KM_THREADS, smem, st>>>(X, n, D, labels, weights, K, partial, nullptr, pweight);
+    GFS_LAUNCH_OK("kmeans_partial_kernel<weighted>");
+    kmeans_reduce_weighted_kernel<<<(K * D + 255) / 256, 256, 0, st>>>(partial, pweight, P, K * D, K, sums, wsums);
+    GFS_LAUNCH_OK("kmeans_reduce_weighted_kernel");
     return GFS_OK;
 }
 
@@ -146,6 +223,9 @@ namespace gfs {
 //                         caller's), shift = sum (new - old)^2 (fp64, fixed order), #empty; also the transposed (D, Kp) copy of
 //                         the new centres that the next E-step reads.  result = [changed, shift, empty] (fp64) = one D2H read.
 // ---------------------------------------------------------------------------------------------------------------
+// WEIGHTED: the weight slot packed[K*D : K*D+K] is already filled (gfs_kmeans_accumulate_weighted wrote it), so only the
+// changed-label count is written; WEIGHTED update divides by the fp64 weight sums as they are (no rounding to a count).
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(256)
 kmeans_pack_kernel(const int32_t* __restrict__ labels, const int32_t* __restrict__ labels_old, int64_t n, const int64_t* __restrict__ counts,
                    int K, int KD, double* __restrict__ packed, unsigned long long* __restrict__ scratch) {
@@ -163,7 +243,8 @@ kmeans_pack_kernel(const int32_t* __restrict__ labels, const int32_t* __restrict
     __syncthreads();
     if (!last) return;
     __threadfence();
-    for (int c = threadIdx.x; c < K; c += blockDim.x) packed[KD + c] = (double)counts[c];
+    if constexpr (!WEIGHTED)
+        for (int c = threadIdx.x; c < K; c += blockDim.x) packed[KD + c] = (double)counts[c];
     if (threadIdx.x == 0) {
         packed[KD + K] = (double)atomicAdd(&scratch[0], 0ull);
         scratch[0] = 0ull;
@@ -171,6 +252,7 @@ kmeans_pack_kernel(const int32_t* __restrict__ labels, const int32_t* __restrict
     }
 }
 
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(1024)
 kmeans_update_kernel(const double* __restrict__ packed, const float* __restrict__ centers_old, int K, int D, int Kp,
                      float* __restrict__ centers_new, float* __restrict__ ct, double* __restrict__ result) {
@@ -179,7 +261,7 @@ kmeans_update_kernel(const double* __restrict__ packed, const float* __restrict_
     double shift = 0.0;
     for (int i = threadIdx.x; i < KD; i += 1024) {
         const int c = i / D, d = i - c * D;
-        const double cnt = rint(packed[KD + c]);
+        const double cnt = WEIGHTED ? packed[KD + c] : rint(packed[KD + c]);
         const float nw = cnt > 0.0 ? (float)(packed[i] / cnt) : 0.0f;
         const double df = (double)(nw - centers_old[i]);
         shift += df * df;
@@ -187,7 +269,7 @@ kmeans_update_kernel(const double* __restrict__ packed, const float* __restrict_
         ct[(int64_t)d * Kp + c] = nw;
     }
     double empty = 0.0;
-    for (int c = threadIdx.x; c < K; c += 1024) empty += rint(packed[KD + c]) > 0.0 ? 0.0 : 1.0;
+    for (int c = threadIdx.x; c < K; c += 1024) empty += (WEIGHTED ? packed[KD + c] : rint(packed[KD + c])) > 0.0 ? 0.0 : 1.0;
 #pragma unroll
     for (int o = 16; o >= 1; o >>= 1) {
         shift += __shfl_xor_sync(0xffffffffu, shift, o);
@@ -220,9 +302,22 @@ extern "C" int gfs_kmeans_pack(const int32_t* labels, const int32_t* labels_old,
     GFS_REQUIRE(labels && labels_old && counts && packed && scratch16 && n > 0 && K > 0 && D > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_pack: bad argument");
     const int64_t want = (n + 256 * 8 - 1) / (256 * 8);
     const unsigned grid = (unsigned)(want < 1 ? 1 : want > 592 ? 592 : want);
-    kmeans_pack_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(labels, labels_old, n, counts, K, K * D, packed,
-                                                                           static_cast<unsigned long long*>(scratch16));
+    kmeans_pack_kernel<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(labels, labels_old, n, counts, K, K * D, packed,
+                                                                                  static_cast<unsigned long long*>(scratch16));
     GFS_LAUNCH_OK("kmeans_pack_kernel");
+    return GFS_OK;
+}
+
+extern "C" int gfs_kmeans_pack_weighted(const int32_t* labels, const int32_t* labels_old, int64_t n, int K, int D, double* packed,
+                                        void* scratch16, void* stream) {
+    using namespace gfs;
+    GFS_REQUIRE(labels && labels_old && packed && scratch16, GFS_ERR_BAD_ARG, "gfs_kmeans_pack_weighted: null pointer");
+    GFS_REQUIRE(n > 0 && K > 0 && D > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_pack_weighted: non-positive size");
+    const int64_t want = (n + 256 * 8 - 1) / (256 * 8);
+    const unsigned grid = (unsigned)(want < 1 ? 1 : want > 592 ? 592 : want);
+    kmeans_pack_kernel<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(labels, labels_old, n, nullptr, K, K * D, packed,
+                                                                                 static_cast<unsigned long long*>(scratch16));
+    GFS_LAUNCH_OK("kmeans_pack_kernel<weighted>");
     return GFS_OK;
 }
 
@@ -231,8 +326,20 @@ extern "C" int gfs_kmeans_update(const double* packed, const float* centers_old,
     using namespace gfs;
     GFS_REQUIRE(packed && centers_old && centers_new && centers_t && result3 && K > 0 && D > 0 && Kp >= K, GFS_ERR_BAD_ARG,
                 "gfs_kmeans_update: bad argument");
-    kmeans_update_kernel<<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(packed, centers_old, K, D, Kp, centers_new, centers_t, result3);
+    kmeans_update_kernel<false><<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(packed, centers_old, K, D, Kp, centers_new, centers_t,
+                                                                                   result3);
     GFS_LAUNCH_OK("kmeans_update_kernel");
+    return GFS_OK;
+}
+
+extern "C" int gfs_kmeans_update_weighted(const double* packed, const float* centers_old, int K, int D, int Kp, float* centers_new,
+                                          float* centers_t, double* result3, void* stream) {
+    using namespace gfs;
+    GFS_REQUIRE(packed && centers_old && centers_new && centers_t && result3, GFS_ERR_BAD_ARG, "gfs_kmeans_update_weighted: null pointer");
+    GFS_REQUIRE(K > 0 && D > 0 && Kp >= K, GFS_ERR_BAD_ARG, "gfs_kmeans_update_weighted: bad size");
+    kmeans_update_kernel<true><<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(packed, centers_old, K, D, Kp, centers_new, centers_t,
+                                                                                  result3);
+    GFS_LAUNCH_OK("kmeans_update_kernel<weighted>");
     return GFS_OK;
 }
 
@@ -252,10 +359,13 @@ namespace gfs {
 constexpr int PP_T = 8;
 constexpr int PP_THREADS = 256;
 
+// WEIGHTED (sklearn's `distance_to_candidates @ sample_weight`): pots[t] += sum_i w_i * m[t][i] in fp64 -- the product of two
+// fp32 values is exact in fp64, so with all weights 1 the sums are those of the unweighted instance.
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(PP_THREADS)
 kmeans_pp_trial_kernel(const float* __restrict__ xt, int64_t npad, int64_t n, int D, const double* __restrict__ xsq,
-                       const float* __restrict__ cand, int T, const float* __restrict__ closest, float* __restrict__ m_out,
-                       double* __restrict__ pots) {
+                       const float* __restrict__ cand, int T, const float* __restrict__ closest, const float* __restrict__ weights,
+                       float* __restrict__ m_out, double* __restrict__ pots) {
     extern __shared__ __align__(16) double csd[];   // [D][8] candidate coordinates, then [8] squared norms
     double* csq = csd + D * PP_T;
     for (int i = threadIdx.x; i < D * PP_T; i += PP_THREADS) {
@@ -292,6 +402,8 @@ kmeans_pp_trial_kernel(const float* __restrict__ xt, int64_t npad, int64_t n, in
     }
     const double xs = xsq[ii];
     const float cl = closest ? closest[ii] : INFINITY;
+    double wi = 1.0;
+    if constexpr (WEIGHTED) wi = (double)weights[ii];
     __shared__ double red[PP_T][PP_THREADS / 32];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
@@ -300,7 +412,9 @@ kmeans_pp_trial_kernel(const float* __restrict__ xt, int64_t npad, int64_t n, in
             const float d = fmaxf((float)((xs - 2.0 * dot[t]) + csq[t]), 0.0f);
             const float m = fminf(d, cl);
             if (on) m_out[(int64_t)t * npad + i] = m;
-            double s = on ? (double)m : 0.0;
+            double s;
+            if constexpr (WEIGHTED) s = on ? (double)m * wi : 0.0;
+            else s = on ? (double)m : 0.0;
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
             if (lane == 0) red[t][warp] = s;
@@ -326,8 +440,118 @@ extern "C" int gfs_kmeans_pp_trial(const float* xt, int64_t npad, int64_t n, int
     const size_t smem = (size_t)(D * PP_T + PP_T) * sizeof(double);
     const int64_t grid = (n + PP_THREADS - 1) / PP_THREADS;
     GFS_REQUIRE(grid < ((int64_t)1 << 31), GFS_ERR_UNSUPPORTED, "gfs_kmeans_pp_trial: n too large");
-    kmeans_pp_trial_kernel<<<(unsigned)grid, PP_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(xt, npad, n, D, xsq, cand, T, closest,
-                                                                                                m_out, pots);
+    kmeans_pp_trial_kernel<false><<<(unsigned)grid, PP_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(xt, npad, n, D, xsq, cand, T,
+                                                                                                       closest, nullptr, m_out, pots);
     GFS_LAUNCH_OK("kmeans_pp_trial_kernel");
+    return GFS_OK;
+}
+
+extern "C" int gfs_kmeans_pp_trial_weighted(const float* xt, int64_t npad, int64_t n, int D, const double* xsq, const float* cand, int T,
+                                            const float* closest, const float* weights, float* m_out, double* pots, void* stream) {
+    using namespace gfs;
+    GFS_REQUIRE(xt && xsq && cand && weights && m_out && pots, GFS_ERR_BAD_ARG, "gfs_kmeans_pp_trial_weighted: null pointer");
+    GFS_REQUIRE(n > 0 && npad >= n && D > 0 && T > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_pp_trial_weighted: non-positive size");
+    GFS_REQUIRE(T <= PP_T, GFS_ERR_UNSUPPORTED, "gfs_kmeans_pp_trial_weighted: T=%d candidates > %d is not built", T, PP_T);
+    GFS_REQUIRE(D <= 512, GFS_ERR_UNSUPPORTED, "gfs_kmeans_pp_trial_weighted: D=%d > 512 is not built", D);
+    const size_t smem = (size_t)(D * PP_T + PP_T) * sizeof(double);
+    const int64_t grid = (n + PP_THREADS - 1) / PP_THREADS;
+    GFS_REQUIRE(grid < ((int64_t)1 << 31), GFS_ERR_UNSUPPORTED, "gfs_kmeans_pp_trial_weighted: n too large");
+    kmeans_pp_trial_kernel<true><<<(unsigned)grid, PP_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(xt, npad, n, D, xsq, cand, T,
+                                                                                                      closest, weights, m_out, pots);
+    GFS_LAUNCH_OK("kmeans_pp_trial_kernel<weighted>");
+    return GFS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// inertia (sklearn _k_means_common.pyx:_inertia_dense):  sum_i w_i * |x_i - c_{label_i}|^2
+// The per-point squared distance is sklearn's fp32 chain (_euclidean_dense_dense): result += ((d0^2 + d1^2) + d2^2) + d3^2 over
+// groups of 4 features, every product and add rounded separately.  One warp per point: lane l loads feature groups l and l + 32
+// (one coalesced row read), the chain then runs in group order through shuffles.  Each CTA owns a contiguous range of points,
+// its warps take the points in a fixed interleave and add w_i * d_i (exact in fp64) in order; the per-CTA fp64 partials are
+// reduced in CTA order, so the result depends on n alone, not on scheduling.
+// ---------------------------------------------------------------------------------------------------------------
+namespace gfs {
+
+constexpr int KI_THREADS = 256;
+constexpr int KI_MAX_CTAS = 1024;   // the partial workspace holds this many doubles
+constexpr int KI_PTS = 4;           // points per warp step (independent loads in flight)
+
+__device__ __forceinline__ float ki_group(const float4 a, const float4 b) {
+    const float d0 = __fsub_rn(a.x, b.x), d1 = __fsub_rn(a.y, b.y), d2 = __fsub_rn(a.z, b.z), d3 = __fsub_rn(a.w, b.w);
+    return __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(d0, d0), __fmul_rn(d1, d1)), __fmul_rn(d2, d2)), __fmul_rn(d3, d3));
+}
+
+__global__ void __launch_bounds__(KI_THREADS)
+kmeans_inertia_kernel(const float* __restrict__ X, int64_t n, int D, const int32_t* __restrict__ labels,
+                      const float* __restrict__ centers, const float* __restrict__ weights, double* __restrict__ partial) {
+    __shared__ double red[KI_THREADS / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int G = D >> 2;                                     // feature groups of 4 (<= 64)
+    const int64_t per = (n + gridDim.x - 1) / gridDim.x;
+    const int64_t i0 = per * blockIdx.x;
+    const int64_t i1 = (i0 + per) < n ? (i0 + per) : n;
+    const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
+    double acc = 0.0;
+    for (int64_t base = i0 + (int64_t)warp * KI_PTS; base < i1; base += (int64_t)KI_PTS * (KI_THREADS / 32)) {
+        float t0[KI_PTS], t1[KI_PTS], w[KI_PTS];
+#pragma unroll
+        for (int q = 0; q < KI_PTS; ++q) {
+            const int64_t i = base + q;
+            const bool on = i < i1;
+            const int64_t ii = on ? i : i0;
+            const int l = labels[ii];
+            w[q] = weights ? weights[ii] : 1.0f;
+            const float4* xr = reinterpret_cast<const float4*>(X + ii * D);
+            const float4* cr = reinterpret_cast<const float4*>(centers + (int64_t)l * D);
+            t0[q] = lane < G ? ki_group(__ldg(xr + lane), __ldg(cr + lane)) : ki_group(zero4, zero4);
+            t1[q] = lane + 32 < G ? ki_group(__ldg(xr + lane + 32), __ldg(cr + lane + 32)) : ki_group(zero4, zero4);
+        }
+        float r[KI_PTS];
+#pragma unroll
+        for (int q = 0; q < KI_PTS; ++q) r[q] = 0.0f;
+        for (int g = 0; g < G; ++g) {                        // warp-uniform: sklearn's group order
+#pragma unroll
+            for (int q = 0; q < KI_PTS; ++q) r[q] = __fadd_rn(r[q], __shfl_sync(0xffffffffu, g < 32 ? t0[q] : t1[q], g & 31));
+        }
+#pragma unroll
+        for (int q = 0; q < KI_PTS; ++q)
+            if (base + q < i1) acc += (double)r[q] * (double)w[q];
+    }
+    if (lane == 0) red[warp] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s = 0.0;
+        for (int k = 0; k < KI_THREADS / 32; ++k) s += red[k];
+        partial[blockIdx.x] = s;
+    }
+}
+
+__global__ void kmeans_inertia_reduce_kernel(const double* __restrict__ partial, int P, double* __restrict__ out) {
+    if (threadIdx.x == 0) {
+        double s = 0.0;
+        for (int p = 0; p < P; ++p) s += partial[p];
+        out[0] = s;
+    }
+}
+
+}  // namespace gfs
+
+extern "C" int gfs_kmeans_inertia_partials(void) { return gfs::KI_MAX_CTAS; }
+
+extern "C" int gfs_kmeans_inertia(const float* X, int64_t n, int D, const int32_t* labels, const float* centers, int K,
+                                  const float* weights, double* partial, double* out, void* stream) {
+    using namespace gfs;
+    GFS_REQUIRE(X && labels && centers && partial && out, GFS_ERR_BAD_ARG, "gfs_kmeans_inertia: null pointer");
+    GFS_REQUIRE(n > 0 && D > 0 && K > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_inertia: non-positive size");
+    GFS_REQUIRE(D <= 256 && D % 4 == 0, GFS_ERR_UNSUPPORTED, "gfs_kmeans_inertia: D=%d must be a multiple of 4, <= 256", D);
+    GFS_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15) == 0 && (reinterpret_cast<uintptr_t>(centers) & 15) == 0, GFS_ERR_BAD_ARG,
+                "gfs_kmeans_inertia: X and centers must be 16-byte aligned");
+    const int64_t want = (n + 63) / 64;
+    const int P = (int)(want < KI_MAX_CTAS ? want : KI_MAX_CTAS);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    kmeans_inertia_kernel<<<P, KI_THREADS, 0, st>>>(X, n, D, labels, centers, weights, partial);
+    GFS_LAUNCH_OK("kmeans_inertia_kernel");
+    kmeans_inertia_reduce_kernel<<<1, 32, 0, st>>>(partial, P, out);
+    GFS_LAUNCH_OK("kmeans_inertia_reduce_kernel");
     return GFS_OK;
 }

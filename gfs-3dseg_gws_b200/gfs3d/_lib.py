@@ -35,6 +35,11 @@ SIGNATURES = {
     "gfs_kmeans_pack": [_p, _p, _i64, _p, _i, _i, _p, _p, _p],
     "gfs_kmeans_update": [_p, _p, _i, _i, _i, _p, _p, _p, _p],
     "gfs_kmeans_pp_trial": [_p, _i64, _i64, _i, _p, _p, _i, _p, _p, _p, _p],
+    "gfs_kmeans_accumulate_weighted": [_p, _i64, _i, _p, _p, _i, _p, _p, _p, _p, _p],
+    "gfs_kmeans_pack_weighted": [_p, _p, _i64, _i, _i, _p, _p, _p],
+    "gfs_kmeans_update_weighted": [_p, _p, _i, _i, _i, _p, _p, _p, _p],
+    "gfs_kmeans_pp_trial_weighted": [_p, _i64, _i64, _i, _p, _p, _i, _p, _p, _p, _p, _p],
+    "gfs_kmeans_inertia": [_p, _i64, _i, _p, _p, _i, _p, _p, _p, _p],
     # training path
     "gfs_gemm_f32": [_p, _i64, _i, _i64, _p, _i64, _i, _i64, _p, _i64, _i, _i64, _p, _i, _i, _i, _i, _i, _p, _i, _p],
     "gfs_gemm_tf32": [_p, _i64, _i, _i64, _p, _i64, _i, _i64, _p, _i64, _i, _i64, _p, _i, _i, _i, _i, _i, _p, _i, _i, _p],
@@ -60,6 +65,7 @@ SIGNATURES = {
 }
 UTILITIES = {"gfs_version": (_i, []), "gfs_last_error_string": (ctypes.c_char_p, []),
              "gfs_device_sm_count": (_i, []), "gfs_set_pdl": (_i, [_i]), "gfs_kmeans_partials": (_i, []),
+             "gfs_kmeans_inertia_partials": (_i, []),
              "gfs_knn_tc_workspace_bytes": (_i64, [_i, _i, _i]),
              "gfs_knn_tc_chains": (_i, [_i, _i, _i]), "gfs_knn_tc_set_split": (_i, [_i]),
              "gfs_rowsel_tc_workspace_bytes": (_i64, [_i64, _i])}

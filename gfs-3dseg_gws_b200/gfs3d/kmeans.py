@@ -8,8 +8,13 @@ Multi-GPU: pass `process_group` (or have torch.distributed initialised and shard
 the points; the only exchange per iteration is an NCCL all-reduce of the (K*D + K) fp64 sums/counts (+ the mean/variance
 once), every rank applies the identical centroid update.
 
+Beyond get_basis.py: the rest of sklearn's KMeans interface -- `sample_weight` (weighted seeding, M-step, relocation and
+inertia: _k_means_lloyd.pyx:216-218, _kmeans.py:_kmeans_plusplus), `init='random'`, the `n_init` loop (_kmeans.py:1504-1545),
+`inertia_`, `predict`, `transform`, `fit_transform` and `score`.  Numpy inputs give numpy results, tensors give tensors.
+
 Inject for the reference script without editing it:   import get_basis; get_basis.KMeans = gfs3d.kmeans.KMeans
 """
+import warnings
 from typing import Optional
 
 import numpy as np
@@ -54,7 +59,53 @@ class KMeans:
         d = _dist()
         return d.get_world_size(self.process_group), d.get_rank(self.process_group)
 
-    def _seed_plusplus(self, Xc, xt, rng, n=None):
+    def _gather_sizes(self, n, dev):
+        world, rank = self._world()
+        sizes = torch.tensor([n], dtype=torch.int64, device=dev)
+        if world > 1:
+            allsz = [torch.empty_like(sizes) for _ in range(world)]
+            _dist().all_gather(allsz, sizes, group=self.process_group)
+            sizes = torch.cat(allsz)
+        return sizes.tolist()
+
+    def _gather_weights(self, w, sizes):
+        """the weights of all ranks in rank order (4 bytes per point, once per seeding), as float32 numpy"""
+        world, _ = self._world()
+        if world == 1:
+            return w.cpu().numpy()
+        parts = [torch.empty(s_, dtype=torch.float32, device=w.device) for s_ in sizes]
+        _dist().all_gather(parts, w.contiguous(), group=self.process_group)
+        return torch.cat(parts).cpu().numpy()
+
+    def _broadcast0(self, t):
+        if self._world()[0] > 1:
+            _dist().broadcast(t, src=_dist().get_global_rank(self.process_group, 0) if self.process_group else 0,
+                              group=self.process_group)
+        return t
+
+    def _seed_random(self, Xc, rng, n, w=None):
+        """sklearn _kmeans.py:1030-1037: K distinct rows drawn with choice(n, size=K, replace=False, p=w/sum(w)) -- p is passed
+        with unit weights too, as sklearn does (numpy draws differently without it).  Sharded: drawn on rank 0 over the points
+        of all ranks in rank order, each row contributed by its owner rank."""
+        K = self.n_clusters
+        dev = Xc.device
+        world, rank = self._world()
+        sizes = self._gather_sizes(n, dev)
+        n_tot, lo = sum(sizes), sum(sizes[:rank])
+        wall = self._gather_weights(w, sizes) if w is not None else None
+        idx = torch.empty(K, dtype=torch.int64)
+        if rank == 0:
+            wa = wall if wall is not None else np.ones(n_tot, dtype=np.float32)
+            idx[:] = torch.from_numpy(rng.choice(n_tot, size=K, replace=False, p=wa / wa.sum()).astype(np.int64))
+        idx = self._broadcast0(idx.to(dev))
+        pos = idx - lo
+        mine = (pos >= 0) & (pos < n)
+        rows = Xc[pos.clamp(0, n - 1)] * mine.to(torch.float32).unsqueeze(1)
+        if world > 1:
+            _dist().all_reduce(rows, group=self.process_group)
+        return rows.contiguous()
+
+    def _seed_plusplus(self, Xc, xt, rng, n=None, w=None):
         """k-means++ exactly as sklearn's _kmeans_plusplus consumes its random stream (sklearn 1.9.0 _kmeans.py:_kmeans_plusplus):
         first centre through `choice(n, p=w/sum(w))`, then `uniform(size=2+ln K)` per centre; candidates = searchsorted of
         u * potential in the cumulative sum of the closest squared distances; all candidates of a centre scored in ONE pass over
@@ -65,7 +116,11 @@ class KMeans:
 
         Sharded (multi-GPU): the points of all ranks form ONE sequence in rank order; every rank searches its own slice of the
         global cumulative sum, the owner contributes the candidate rows (all-reduce), potentials are all-reduced: the picks equal
-        the single-GPU picks.  The random numbers are drawn on rank 0 and broadcast.  No host synchronisation inside the loop."""
+        the single-GPU picks.  The random numbers are drawn on rank 0 and broadcast.  No host synchronisation inside the loop.
+
+        Weighted (w: this rank's (n,) fp32 weights): the first centre is choice(n, p=w/sum(w)) over the weights of all ranks
+        (all-gathered once), the potentials are sum_i w_i * closest_i (gfs_kmeans_pp_trial_weighted) and the candidates come
+        from the cumulative sum of w * closest; `closest` itself stays unweighted, as in sklearn."""
         D = Xc.shape[1]
         n = Xc.shape[0] if n is None else n
         K = self.n_clusters
@@ -74,18 +129,14 @@ class KMeans:
             raise NotImplementedError(f"k-means++ with {trials} local trials (n_clusters={K}) is not built")
         dev = Xc.device
         world, rank = self._world()
-        sizes = torch.tensor([n], dtype=torch.int64, device=dev)
-        if world > 1:
-            allsz = [torch.empty_like(sizes) for _ in range(world)]
-            _dist().all_gather(allsz, sizes, group=self.process_group)
-            sizes = torch.cat(allsz)
-        sizes = sizes.tolist()
+        sizes = self._gather_sizes(n, dev)
         n_tot, lo = sum(sizes), sum(sizes[:rank])
         # the random stream (rank 0's generator; the other ranks receive the draws)
         draws = torch.empty(1 + (K - 1) * trials, dtype=torch.float64)
+        wall = self._gather_weights(w, sizes) if w is not None else None
         if rank == 0:
-            w = np.ones(n_tot, dtype=np.float32)
-            draws[0] = float(rng.choice(n_tot, p=w / w.sum()))
+            wa = wall if wall is not None else np.ones(n_tot, dtype=np.float32)
+            draws[0] = float(rng.choice(n_tot, p=wa / wa.sum()))
             draws[1:] = torch.from_numpy(rng.uniform(size=(K - 1) * trials)) if K > 1 else draws[1:]
         draws = draws.to(dev)
         if world > 1:
@@ -108,12 +159,19 @@ class KMeans:
 
         first = draws[0].long() - lo
         centers[0] = owned_rows(first.view(1), ((first >= 0) & (first < n)).view(1))[0]
-        ops.kmeans_pp_trial(xt, n, xsq, centers[0:1].contiguous(), None, m, pots)
+        def trial(cand, closest):
+            if w is None:
+                ops.kmeans_pp_trial(xt, n, xsq, cand, closest, m, pots)
+            else:
+                ops.kmeans_pp_trial_weighted(xt, n, xsq, cand, closest, w, m, pots)
+
+        trial(centers[0:1].contiguous(), None)
         if world > 1:
             _dist().all_reduce(pots, group=self.process_group)
         closest, pot = m[0].clone(), pots[0].clone()
         for c in range(1, K):
-            cs = torch.cumsum(closest[:n].double(), 0)             # this rank's slice of the global cumulative sum, minus P[rank]
+            # this rank's slice of the global cumulative sum (of w * closest when weighted: an exact fp64 product), minus P[rank]
+            cs = torch.cumsum(closest[:n].double() if w is None else closest[:n].double() * w.double(), 0)
             tots = cs[-1:].contiguous()
             if world > 1:
                 gathered = [torch.empty_like(tots) for _ in range(world)]
@@ -126,7 +184,7 @@ class KMeans:
             pos = torch.searchsorted(cs, rv - (P[rank] - tots[rank])).clamp_max(n - 1)   # first i with cumsum[i] >= rv (side='left')
             cand = owned_rows(pos, mine)
             pots.zero_()
-            ops.kmeans_pp_trial(xt, n, xsq, cand, closest, m, pots)
+            trial(cand, closest)
             if world > 1:
                 _dist().all_reduce(pots, group=self.process_group)
             best = torch.argmin(pots[:trials]).view(1)
@@ -136,18 +194,62 @@ class KMeans:
         return centers
 
     # ------------------------------------------------------------------ fit
-    def fit(self, X, y=None, sample_weight=None):
-        if sample_weight is not None:
-            raise NotImplementedError("sample_weight is not built (get_basis.py never passes it)")
-        dev = torch.device(self.device) if self.device is not None else torch.device("cuda", torch.cuda.current_device())
-        if isinstance(X, np.ndarray):
-            Xd = torch.from_numpy(np.ascontiguousarray(X, dtype=np.float32)).to(dev, non_blocking=True)
+    def _check_weight(self, sample_weight, n):
+        """sklearn's _check_sample_weight(..., dtype=float32) plus the checks its seeding relies on; runs before the data
+        touch the device.  -> None, or the (n,) float32 weights as a CPU or CUDA tensor (a CUDA tensor stays where it is)"""
+        if sample_weight is None:
+            return None
+        if isinstance(sample_weight, torch.Tensor):
+            w = sample_weight.detach().to(torch.float32)
         else:
-            Xd = X.to(dev, torch.float32).contiguous()
+            w = torch.from_numpy(np.ascontiguousarray(np.asarray(sample_weight, dtype=np.float32)))
+        if tuple(w.shape) != (n,):
+            raise ValueError(f"sample_weight has shape {tuple(w.shape)}, expected ({n},)")
+        if not bool(torch.isfinite(w).all()):
+            raise ValueError("sample_weight must be finite")
+        if bool((w < 0).any()):
+            raise ValueError("sample_weight must be non-negative")
+        if not self.shard and not bool((w > 0).any()):
+            raise ValueError("sample_weight must contain at least one positive entry")
+        return w.contiguous()
+
+    def _n_runs(self):
+        """sklearn _kmeans.py:_check_params_vs_input: 'auto' is 10 runs for init='random', else 1; an array init runs once"""
+        array_init = isinstance(self.init, (np.ndarray, torch.Tensor))
+        if self.n_init == "auto":
+            runs = 10 if (isinstance(self.init, str) and self.init == "random") else 1
+        else:
+            runs = int(self.n_init)
+            if runs < 1:
+                raise ValueError(f"n_init={self.n_init!r} must be 'auto' or a positive integer")
+        if array_init and runs != 1:
+            warnings.warn(f"Explicit initial center position passed: performing only one init in KMeans instead of n_init={runs}.",
+                          RuntimeWarning, stacklevel=3)
+            runs = 1
+        return runs
+
+    def _as_device(self, X, dev):
+        if isinstance(X, np.ndarray):
+            return torch.from_numpy(np.ascontiguousarray(X, dtype=np.float32)).to(dev, non_blocking=True)
+        return X.to(dev, torch.float32).contiguous()
+
+    def fit(self, X, y=None, sample_weight=None):
+        """sample_weight: None or (n,) non-negative finite weights (numpy or tensor), cast to float32; with shard=True, the
+        weights of this rank's shard.  Mean-centring and the tolerance stay unweighted, as in sklearn."""
+        w_in = self._check_weight(sample_weight, X.shape[0])
+        dev = torch.device(self.device) if self.device is not None else torch.device("cuda", torch.cuda.current_device())
+        Xd = self._as_device(X, dev)
         n, D = Xd.shape
         K = self.n_clusters
         if K > 192:
             raise NotImplementedError(f"n_clusters={K} > 192 is not built")
+        runs = self._n_runs()
+        w = w_in.to(dev) if w_in is not None else None
+        if w is not None and self.shard:
+            wtot = w.double().sum().view(1)
+            self._allreduce(wtot)
+            if not float(wtot) > 0:
+                raise ValueError("sample_weight must contain at least one positive entry")
 
         # mean-centring and tolerance (global over all shards)
         stat = torch.cat([Xd.double().sum(0), (Xd.double() ** 2).sum(0), torch.tensor([float(n)], dtype=torch.float64, device=dev)])
@@ -162,19 +264,55 @@ class KMeans:
         xt = torch.zeros(D, npad, dtype=torch.float32, device=dev)
         xt[:, :n] = Xc.t()
 
-        # initial centres
-        if isinstance(self.init, str) and self.init == "k-means++":
-            centers = self._seed_plusplus(Xc, xt, self._rng(), n)
-        elif isinstance(self.init, (np.ndarray, torch.Tensor)):
-            centers = torch.as_tensor(self.init, dtype=torch.float32).to(dev) - mean32
-            if centers.shape != (K, D):
-                raise ValueError(f"init has shape {tuple(centers.shape)}, expected {(K, D)}")
-        else:
-            raise NotImplementedError(f"init={self.init!r} is not built")
+        rng = self._rng() if isinstance(self.init, str) else None
+        best = None
+        for _ in range(runs):
+            # initial centres
+            if isinstance(self.init, str) and self.init == "k-means++":
+                centers = self._seed_plusplus(Xc, xt, rng, n, w=w)
+            elif isinstance(self.init, str) and self.init == "random":
+                centers = self._seed_random(Xc, rng, n, w=w)
+            elif isinstance(self.init, (np.ndarray, torch.Tensor)):
+                centers = torch.as_tensor(self.init, dtype=torch.float32).to(dev) - mean32
+                if centers.shape != (K, D):
+                    raise ValueError(f"init has shape {tuple(centers.shape)}, expected {(K, D)}")
+            else:
+                raise NotImplementedError(f"init={self.init!r} is not built")
+            labels, centers, n_iter, lloyd_ms = self._lloyd(Xc, xt, n, centers.contiguous(), w, tol_abs)
+            inertia = self._allreduce(ops.kmeans_inertia(Xc, labels, centers, w, n_valid=n))
+            inertia = float(inertia)
+            # sklearn _kmeans.py:1534-1538: a later run wins only with a lower inertia AND a different partition
+            if best is None or (inertia < best[0] and not self._same_clustering(labels[:n], best[1][:n])):
+                best = (inertia, labels, centers, n_iter, lloyd_ms)
 
+        inertia, labels, centers, n_iter, lloyd_ms = best
+        self.labels_ = labels[:n].cpu().numpy().astype(np.int32)
+        self.lloyd_ms_ = lloyd_ms
+        self.labels_device_ = labels[:n]
+        self.cluster_centers_ = (centers + mean32).cpu().numpy()
+        self.inertia_ = inertia
+        self.n_iter_ = n_iter
+        self.n_features_in_ = D
+        self.mean_device_ = mean32                      # predict centres new data with the fit's fp32 mean ...
+        self.centers_centered_ = centers               # ... against these: cluster_centers_ - mean does not round back to them
+        return self
+
+    def _same_clustering(self, a, b):
+        """sklearn _k_means_common.pyx:_is_same_clustering (every label of a maps to one label of b), over all shards"""
+        K = self.n_clusters
+        pairs = torch.bincount(a.long() * K + b.long(), minlength=K * K).view(K, K)
+        self._allreduce(pairs)
+        return bool(((pairs > 0).sum(1) <= 1).all())
+
+    def _lloyd(self, Xc, xt, n, centers, w, tol_abs):
+        """one Lloyd run from the (centred) initial centres -> (labels (npad) int32, centres (K, D), n_iter, Lloyd ms)"""
+        K, D = self.n_clusters, Xc.shape[1]
+        dev = Xc.device
+        npad = xt.shape[1]
         # Lloyd iterations.  Per iteration: E-step (4 launches), M-step sums (2), pack (1), ONE collective of the packed
         # [sums | counts | labels changed] buffer when sharded, centre update (1) and ONE device->host read of
-        # (labels changed, centre shift, empty clusters).  All buffers are allocated once.
+        # (labels changed, centre shift, empty clusters).  All buffers are allocated once.  Weighted: the same launches, with
+        # the fp64 weight sums in the counts' slot.
         Kp = (K + 3) // 4 * 4
         ct = torch.zeros(D, Kp, dtype=torch.float32, device=dev)
         ct[:, :K] = centers.t()
@@ -183,8 +321,12 @@ class KMeans:
         labels_old = torch.full((npad,), -1, dtype=torch.int32, device=dev)
         packed = torch.empty(K * D + K + 1, dtype=torch.float64, device=dev)
         sums = packed[:K * D].view(K, D)
-        counts = torch.empty(K, dtype=torch.int64, device=dev)
-        acc_ws = ops.kmeans_accumulate_workspace(K, D, dev)
+        if w is None:
+            counts = torch.empty(K, dtype=torch.int64, device=dev)
+            acc_ws = ops.kmeans_accumulate_workspace(K, D, dev)
+        else:
+            wsums = packed[K * D:K * D + K]
+            acc_ws = ops.kmeans_accumulate_weighted_workspace(K, D, dev)
         scratch = torch.zeros(2, dtype=torch.int64, device=dev)
         result = torch.empty(3, dtype=torch.float64, device=dev)
         # E-step over the channel-major copy: tensor-core product when the shape allows, same labels as the fp32 kernel.  (The
@@ -196,18 +338,30 @@ class KMeans:
         ev0.record()
         for n_iter in range(1, self.max_iter + 1):
             labels = assign()                                          # ct holds the current centres, transposed
-            ops.kmeans_accumulate(Xc, labels, K, n_valid=n, sums=sums, counts=counts, ws=acc_ws)
-            ops.kmeans_pack(labels, labels_old, n, counts, K, D, packed, scratch)
+            if w is None:
+                ops.kmeans_accumulate(Xc, labels, K, n_valid=n, sums=sums, counts=counts, ws=acc_ws)
+                ops.kmeans_pack(labels, labels_old, n, counts, K, D, packed, scratch)
+            else:
+                ops.kmeans_accumulate_weighted(Xc, labels, w, K, n_valid=n, sums=sums, wsums=wsums, ws=acc_ws)
+                ops.kmeans_pack_weighted(labels, labels_old, n, K, D, packed, scratch)
             if self.shard:
                 _dist().all_reduce(packed, group=self.process_group)
-            ops.kmeans_update(packed, centers, K, D, Kp, centers_new, ct, result)
+            if w is None:
+                ops.kmeans_update(packed, centers, K, D, Kp, centers_new, ct, result)
+            else:
+                ops.kmeans_update_weighted(packed, centers, K, D, Kp, centers_new, ct, result)
             n_changed, shift_h, n_empty = result.tolist()
             if n_empty > 0:           # rare: sklearn moves the empty clusters onto the points farthest from their centres
                 gsums = packed[:K * D].view(K, D).clone()
-                gcounts = packed[K * D:K * D + K].round().long()
-                gsums, gcounts = self._relocate_empty(Xc, n, labels, centers, gsums, gcounts)
-                # clusters that are still empty keep the zero sum (sklearn _k_means_common.pyx:_average_centers)
-                new = torch.where(gcounts[:, None] > 0, gsums / gcounts.clamp_min(1)[:, None].double(), torch.zeros_like(gsums)).float()
+                if w is None:
+                    gcounts = packed[K * D:K * D + K].round().long()
+                    gsums, gcounts = self._relocate_empty(Xc, n, labels, centers, gsums, gcounts)
+                    # clusters that are still empty keep the zero sum (sklearn _k_means_common.pyx:_average_centers)
+                    new = torch.where(gcounts[:, None] > 0, gsums / gcounts.clamp_min(1)[:, None].double(), torch.zeros_like(gsums)).float()
+                else:
+                    gw = packed[K * D:K * D + K].clone()
+                    gsums, gw = self._relocate_empty(Xc, n, labels, centers, gsums, gw, w=w)
+                    new = torch.where(gw[:, None] > 0, gsums / torch.where(gw > 0, gw, 1.0)[:, None], torch.zeros_like(gsums)).float()
                 shift_h = float(((new - centers).double() ** 2).sum())
                 centers_new.copy_(new)
                 ct[:, :K] = new.t()
@@ -223,19 +377,20 @@ class KMeans:
         ev1.record()
         if not strict:
             labels = assign()                                          # ct already holds the final centres
-        self.labels_ = labels[:n].cpu().numpy().astype(np.int32)
-        self.lloyd_ms_ = ev0.elapsed_time(ev1)          # device time of the Lloyd loop (the .cpu() above synchronised)
-        self.labels_device_ = labels[:n]
-        self.cluster_centers_ = (centers + mean32).cpu().numpy()
-        self.n_iter_ = n_iter
-        self.n_features_in_ = D
-        return self
+        torch.cuda.synchronize(dev)
+        return labels, centers, n_iter, ev0.elapsed_time(ev1)
 
-    def _relocate_empty(self, Xc, n, labels, centers, sums, counts):
+    def _relocate_empty(self, Xc, n, labels, centers, sums, counts, w=None):
         """sklearn _k_means_common.pyx:167-211: every empty cluster is moved onto one of the points farthest from its own
         (old) centre, and that point is taken out of its old cluster's sum.  Rare path, plain device ops.  Sharded: each
         rank offers its n_empty farthest points (distance, old label, coordinates), the candidates are all-gathered and
-        every rank applies the same global choice to the (already all-reduced) sums / counts."""
+        every rank applies the same global choice to the (already all-reduced) sums / counts.
+
+        Weighted (w given, counts = the fp64 weight sums): the farthest points are still chosen by unweighted distance;
+        then sums[old] -= w x, sums[e] = w x (an fp32 product, as sklearn), counts[e] = w, counts[old] -= w.  The weight
+        travels next to each candidate row."""
+        if w is not None:
+            return self._relocate_empty_weighted(Xc, n, labels, centers, sums, counts, w)
         empty = (counts == 0).nonzero().flatten()
         ne = int(empty.numel())
         D = Xc.shape[1]
@@ -263,5 +418,98 @@ class KMeans:
             counts[old] -= 1
         return sums, counts
 
+    def _relocate_empty_weighted(self, Xc, n, labels, centers, sums, wsums, w):
+        empty = (wsums == 0).nonzero().flatten()
+        ne = int(empty.numel())
+        D = Xc.shape[1]
+        dist = ((Xc - centers[labels[:n].long()]) ** 2).sum(1)
+        m = min(ne, n)
+        vals, idxs = torch.topk(dist, m)
+        cand = torch.full((ne, 3 + D), float("-inf"), dtype=torch.float64, device=Xc.device)
+        cand[:m, 0] = vals.double()
+        cand[:m, 1] = labels[idxs].double()
+        cand[:m, 2] = w[idxs].double()
+        cand[:m, 3:] = Xc[idxs].double()
+        if self.shard:
+            world = _dist().get_world_size(self.process_group)
+            gathered = [torch.empty_like(cand) for _ in range(world)]
+            _dist().all_gather(gathered, cand, group=self.process_group)
+            cand = torch.cat(gathered, 0)
+        if float(cand[:, 0].max()) <= 0:
+            return sums, wsums
+        order = torch.argsort(cand[:, 0], descending=True, stable=True)[:ne]
+        for e, row in zip(empty.tolist(), order.tolist()):
+            old = int(cand[row, 1])
+            wx = (cand[row, 3:].float() * cand[row, 2].float()).double()
+            sums[old] -= wx
+            sums[e] = wx
+            wsums[e] = cand[row, 2]
+            wsums[old] -= cand[row, 2]
+        return sums, wsums
+
     def fit_predict(self, X, y=None, sample_weight=None):
         return self.fit(X, sample_weight=sample_weight).labels_
+
+    # ------------------------------------------------------------------ fitted-model queries
+    def _fitted_device(self):
+        if not hasattr(self, "centers_centered_"):
+            raise RuntimeError("this KMeans instance is not fitted yet: call fit first")
+        return self.centers_centered_.device
+
+    @staticmethod
+    def _like_input(X, t):
+        """numpy in -> numpy out, tensor in -> tensor on the input's device"""
+        return t.to(X.device) if isinstance(X, torch.Tensor) else t.cpu().numpy()
+
+    def _predict_device(self, X):
+        dev = self._fitted_device()
+        Xc = self._as_device(X, dev) - self.mean_device_
+        n, D = Xc.shape
+        if D != self.n_features_in_:
+            raise ValueError(f"X has {D} features, the model was fitted with {self.n_features_in_}")
+        K = self.n_clusters
+        xt = torch.zeros(D, (n + 3) // 4 * 4, dtype=torch.float32, device=dev)
+        xt[:, :n] = Xc.t()
+        ct = torch.zeros(D, (K + 3) // 4 * 4, dtype=torch.float32, device=dev)
+        ct[:, :K] = self.centers_centered_.t()
+        return Xc.contiguous(), ops.kmeans_assign(xt, ct, K)[:n]
+
+    def predict(self, X):
+        """nearest centre of each row: X is centred with the fit's fp32 mean and labelled by the pinned E-step against the
+        fit's centred fp32 centres (labels defined bit for bit by oracle.kmeans_assign_exact on the centred data)"""
+        return self._like_input(X, self._predict_device(X)[1])
+
+    def transform(self, X):
+        """(n, K) Euclidean distances to cluster_centers_ on the uncentred data, as sklearn's euclidean_distances evaluates
+        float32 input: (|x|^2 - 2 x.c) + |c|^2 in fp64, one rounding to fp32, a clip at 0, an fp32 sqrt.  Runs
+        gfs_kmeans_pp_trial (closest = NULL) over groups of 8 centres."""
+        dev = self._fitted_device()
+        Xd = self._as_device(X, dev)
+        n, D = Xd.shape
+        if D != self.n_features_in_:
+            raise ValueError(f"X has {D} features, the model was fitted with {self.n_features_in_}")
+        K = self.n_clusters
+        npad = (n + 3) // 4 * 4
+        xt = torch.zeros(D, npad, dtype=torch.float32, device=dev)
+        xt[:, :n] = Xd.t()
+        xsq = (Xd.double() ** 2).sum(1)
+        C = torch.from_numpy(np.ascontiguousarray(self.cluster_centers_, dtype=np.float32)).to(dev)
+        m = torch.empty(8, npad, dtype=torch.float32, device=dev)
+        pots = torch.zeros(8, dtype=torch.float64, device=dev)
+        out = torch.empty(n, K, dtype=torch.float32, device=dev)
+        for g in range(0, K, 8):
+            T = min(8, K - g)
+            ops.kmeans_pp_trial(xt, n, xsq, C[g:g + T].contiguous(), None, m, pots)
+            out[:, g:g + T] = m[:T, :n].t()
+        return self._like_input(X, torch.sqrt(out))
+
+    def fit_transform(self, X, y=None, sample_weight=None):
+        return self.fit(X, sample_weight=sample_weight).transform(X)
+
+    def score(self, X, y=None, sample_weight=None):
+        """-inertia of predict(X) on X (centred as in predict), weighted by sample_weight"""
+        w = self._check_weight(sample_weight, X.shape[0])
+        Xc, labels = self._predict_device(X)
+        if w is not None:
+            w = w.to(Xc.device)
+        return -float(ops.kmeans_inertia(Xc, labels, self.centers_centered_, w))

@@ -390,6 +390,82 @@ def kmeans_accumulate_workspace(K: int, D: int, device):
     return (torch.empty(P * K * D, dtype=torch.float32, device=device), torch.empty(P * K, dtype=torch.int32, device=device))
 
 
+def kmeans_accumulate_weighted(X: torch.Tensor, labels: torch.Tensor, weights: torch.Tensor, K: int, n_valid: Optional[int] = None,
+                               sums=None, wsums=None, ws=None):
+    """X (n, D) fp32 row-major, labels (n) int32, weights (n) fp32 -> sums (K, D) fp64 of x * w, wsums (K) fp64 of w
+    (deterministic; weights of 1 give kmeans_accumulate's sums bit for bit).  ws = (partial, pweight) from
+    kmeans_accumulate_weighted_workspace; wsums may be a view of the packed buffer's weight slot."""
+    _need_cuda(X, labels, weights)
+    n, D = X.shape
+    if n_valid is not None:
+        n = n_valid
+    assert X.is_contiguous() and labels.dtype == torch.int32 and weights.dtype == torch.float32 and weights.is_contiguous()
+    assert weights.numel() >= n
+    if ws is None:
+        ws = kmeans_accumulate_weighted_workspace(K, D, X.device)
+    partial, pweight = ws
+    if sums is None:
+        sums = torch.empty(K, D, dtype=torch.float64, device=X.device)
+    if wsums is None:
+        wsums = torch.empty(K, dtype=torch.float64, device=X.device)
+    assert sums.dtype == torch.float64 and sums.is_contiguous() and wsums.dtype == torch.float64 and wsums.is_contiguous()
+    _call("gfs_kmeans_accumulate_weighted", 2, _ptr(X), n, D, _ptr(labels), _ptr(weights), K, _ptr(partial), _ptr(pweight),
+          _ptr(sums), _ptr(wsums), _stream())
+    return sums, wsums
+
+
+def kmeans_accumulate_weighted_workspace(K: int, D: int, device):
+    P = lib().gfs_kmeans_partials()
+    return (torch.empty(P * K * D, dtype=torch.float32, device=device), torch.empty(P * K, dtype=torch.float64, device=device))
+
+
+def kmeans_pack_weighted(labels, labels_old, n, K, D, packed, scratch):
+    """packed[-1] = #(labels != labels_old) over the first n; packed[:K*D] (sums) and packed[K*D:K*D+K] (weight sums) are
+    filled already by kmeans_accumulate_weighted"""
+    _need_cuda(labels, labels_old, packed, scratch)
+    assert packed.dtype == torch.float64 and packed.numel() == K * D + K + 1 and scratch.numel() * scratch.element_size() >= 16
+    _call("gfs_kmeans_pack_weighted", 1, _ptr(labels), _ptr(labels_old), n, K, D, _ptr(packed), _ptr(scratch), _stream())
+
+
+def kmeans_update_weighted(packed, centers_old, K, D, Kp, centers_new, ct, result):
+    """kmeans_update dividing by the fp64 weight sums of the packed buffer as they are (no rounding to a count)"""
+    _need_cuda(packed, centers_old, centers_new, ct, result)
+    assert centers_old.is_contiguous() and centers_new.is_contiguous() and ct.is_contiguous() and result.dtype == torch.float64
+    _call("gfs_kmeans_update_weighted", 1, _ptr(packed), _ptr(centers_old), K, D, Kp, _ptr(centers_new), _ptr(ct), _ptr(result),
+          _stream())
+
+
+def kmeans_pp_trial_weighted(xt: torch.Tensor, n: int, xsq: torch.Tensor, cand: torch.Tensor, closest: Optional[torch.Tensor],
+                             weights: torch.Tensor, m_out: torch.Tensor, pots: torch.Tensor):
+    """kmeans_pp_trial with pots (T) f64 (+)= sum_i weights[i] * m_out[t, i]; m_out is the unweighted minimum"""
+    _need_cuda(xt, xsq, cand, closest, weights, m_out, pots)
+    D, npad = xt.shape
+    T = cand.shape[0]
+    assert xt.is_contiguous() and cand.is_contiguous() and cand.shape[1] == D and m_out.is_contiguous() and m_out.shape[1] == npad
+    assert m_out.shape[0] >= T and pots.dtype == torch.float64 and pots.numel() >= T and xsq.numel() >= n and xsq.dtype == torch.float64
+    assert weights.dtype == torch.float32 and weights.is_contiguous() and weights.numel() >= n
+    _call("gfs_kmeans_pp_trial_weighted", 1, _ptr(xt), npad, n, D, _ptr(xsq), _ptr(cand), T, _ptr(closest), _ptr(weights), _ptr(m_out),
+          _ptr(pots), _stream())
+
+
+def kmeans_inertia(X: torch.Tensor, labels: torch.Tensor, centers: torch.Tensor, weights: Optional[torch.Tensor] = None,
+                   n_valid: Optional[int] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """X (n, D) fp32 row-major, labels (n) int32, centers (K, D) fp32, weights (n) fp32 or None -> (1,) fp64 on the device:
+    sum_i w_i |x_i - c_{label_i}|^2 (fp32 distance chain as sklearn's, fp64 sum in a fixed order)"""
+    _need_cuda(X, labels, centers, weights)
+    n, D = X.shape
+    if n_valid is not None:
+        n = n_valid
+    K = centers.shape[0]
+    assert X.is_contiguous() and centers.is_contiguous() and centers.shape[1] == D and labels.dtype == torch.int32
+    assert labels.numel() >= n and (weights is None or (weights.dtype == torch.float32 and weights.is_contiguous() and weights.numel() >= n))
+    partial = torch.empty(lib().gfs_kmeans_inertia_partials(), dtype=torch.float64, device=X.device)
+    if out is None:
+        out = torch.empty(1, dtype=torch.float64, device=X.device)
+    _call("gfs_kmeans_inertia", 2, _ptr(X), n, D, _ptr(labels), _ptr(centers), K, _ptr(weights), _ptr(partial), _ptr(out), _stream())
+    return out
+
+
 def kmeans_pack(labels, labels_old, n, counts, K, D, packed, scratch):
     """packed[K*D:K*D+K] = counts, packed[-1] = #(labels != labels_old) over the first n; packed[:K*D] are the sums already"""
     _need_cuda(labels, labels_old, counts, packed, scratch)

@@ -222,6 +222,13 @@ int gfs_kmeans_assign_tc(const float* X, int64_t n, int64_t ld, int point_major,
 int gfs_kmeans_partials(void);
 int gfs_kmeans_accumulate(const float* X, int64_t n, int D, const int32_t* labels, int K,
                           float* partial, int32_t* pcount, double* sums, int64_t* counts, void* stream);
+/* weighted M-step sums (sklearn _k_means_lloyd.pyx:216-218): sums[l] += x * w (an fp32 product, then an fp32 add; no fused
+ * multiply-add) in the same ascending, pairwise order as gfs_kmeans_accumulate, so weights of 1 give its sums bit for bit;
+ * wsums[l] += w in fp64, ascending point order per CTA.  weights (n) fp32; partial (P, K, D) fp32 and pweight (P, K) fp64
+ * workspaces, P = gfs_kmeans_partials(); sums (K, D) and wsums (K) fp64 are reduced in CTA order.  wsums may be the weight
+ * slot packed[K*D : K*D+K] of gfs_kmeans_pack_weighted's buffer.                                                      */
+int gfs_kmeans_accumulate_weighted(const float* X, int64_t n, int D, const int32_t* labels, const float* weights, int K,
+                                   float* partial, double* pweight, double* sums, double* wsums, void* stream);
 
 /* The rest of a Lloyd iteration (sklearn _k_means_common.pyx:_average_centers, _kmeans.py:_kmeans_single_lloyd) in two launches:
  *   gfs_kmeans_pack:   packed (K*D + K + 1 doubles) = [sums (already there: pass packed as gfs_kmeans_accumulate's sums) |
@@ -233,6 +240,22 @@ int gfs_kmeans_pack(const int32_t* labels, const int32_t* labels_old, int64_t n,
                     double* packed, void* scratch16, void* stream);
 int gfs_kmeans_update(const double* packed, const float* centers_old, int K, int D, int Kp, float* centers_new, float* centers_t,
                       double* result3, void* stream);
+/* Weighted forms: packed's middle slot holds the fp64 weight sums (written by gfs_kmeans_accumulate_weighted), so
+ * gfs_kmeans_pack_weighted writes only the changed-label count into packed[K*D + K], and gfs_kmeans_update_weighted divides by
+ * the weight sums as they are (gfs_kmeans_update rounds its slot to an integer count).  A cluster is empty when its weight
+ * sum is 0, so a cluster whose members all weigh 0 is empty, as in sklearn.                                            */
+int gfs_kmeans_pack_weighted(const int32_t* labels, const int32_t* labels_old, int64_t n, int K, int D, double* packed,
+                             void* scratch16, void* stream);
+int gfs_kmeans_update_weighted(const double* packed, const float* centers_old, int K, int D, int Kp, float* centers_new,
+                               float* centers_t, double* result3, void* stream);
+
+/* inertia (sklearn _k_means_common.pyx:_inertia_dense): out[0] = sum_i w_i * |x_i - centers[labels[i]]|^2 (w_i = 1 when
+ * weights is NULL).  The squared distance is sklearn's fp32 chain over groups of 4 features; the sum is fp64 in an order
+ * fixed by n (per-CTA partials, reduced in CTA order): two calls give the same bits.  X (n, D) row-major and centers (K, D),
+ * both 16-byte aligned, D % 4 == 0, D <= 256; partial: gfs_kmeans_inertia_partials() doubles of workspace.            */
+int gfs_kmeans_inertia_partials(void);
+int gfs_kmeans_inertia(const float* X, int64_t n, int D, const int32_t* labels, const float* centers, int K,
+                       const float* weights, double* partial, double* out, void* stream);
 
 /* ---- k-means++ seeding step (sklearn _kmeans.py:_kmeans_plusplus behind get_basis.py:210, SURVEY 8f N3) ---------------
  * For T <= 8 candidate centres:  m[t][i] = min(max(float(|x_i|^2 - 2 x_i.c_t + |c_t|^2), 0), closest[i]),  pots[t] += sum_i m[t][i]
@@ -241,6 +264,10 @@ int gfs_kmeans_update(const double* packed, const float* centers_old, int K, int
  *   (= +inf: the first centre), m_out (T, npad) fp32, pots (T) fp64 ACCUMULATED into (the caller zeroes it)              */
 int gfs_kmeans_pp_trial(const float* xt, int64_t npad, int64_t n, int D, const double* xsq, const float* cand, int T,
                         const float* closest, float* m_out, double* pots, void* stream);
+/* weighted k-means++ (sklearn's `distance_to_candidates @ sample_weight`): pots[t] += sum_i weights[i] * m[t][i] in fp64 (the
+ * product of two fp32 values is exact); m_out is unchanged, closest stays unweighted.  weights (n) fp32.             */
+int gfs_kmeans_pp_trial_weighted(const float* xt, int64_t npad, int64_t n, int D, const double* xsq, const float* cand, int T,
+                                 const float* closest, const float* weights, float* m_out, double* pots, void* stream);
 
 /* =====================================================================================================================
  * TRAINING path (model.train(), train.py:614-631).  fp32 end to end, activations channel-major (C, M) with M = B*N points

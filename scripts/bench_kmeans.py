@@ -3,6 +3,8 @@
 
     python scripts/bench_kmeans.py [--n 500000] [--iters 10]          (one GPU: one shard of the 4 M / 8 split)
     torchrun --nproc-per-node N scripts/bench_kmeans.py --n 4000000   (points sharded over N GPUs, NCCL all-reduce)
+    python scripts/bench_kmeans.py --weighted [--n 4194304]          (one GPU: weighted vs unweighted Lloyd iteration,
+                                                                      the inertia pass, weighted k-means++ seeding)
 
 Prints one JSON line: ms per Lloyd iteration (E-step + M-step + all-reduce), kernel times, achieved GB/s / TFLOP/s,
 and sklearn's Lloyd iteration on a bounded sample of the host cores for comparison."""
@@ -24,6 +26,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--n", type=int, default=500000)
 ap.add_argument("--iters", type=int, default=10)
 ap.add_argument("--cpu-sample", type=int, default=200000)
+ap.add_argument("--weighted", action="store_true", help="time the sample_weight path against the unweighted one (one GPU)")
 a = ap.parse_args()
 world, rank, local = int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0))
 torch.cuda.set_device(local)
@@ -51,6 +54,86 @@ def lloyd(centers):
         sums, counts = allreduce_centroid_stats(sums, counts)
     return (sums / counts.clamp_min(1)[:, None]).float(), labels
 
+
+def bench_weighted():
+    """KMeans' Lloyd iteration as the fit issues it (E-step, M-step sums, pack, centre update, one 24-byte read), weighted and
+    unweighted alternately in rounds; the inertia pass; weighted k-means++ seeding.  Prints the card and its power limit."""
+    import subprocess
+    from gfs3d.kmeans import KMeans as GKMeans
+    w = torch.rand(n, device=dev, generator=g) * 2
+    npad = xt.shape[1]
+    ct = torch.zeros(D, Kp, device=dev)
+    ct[:, :K] = centers.t()
+    cnew, cold = torch.empty(K, D, device=dev), centers.clone()
+    packed = torch.empty(K * D + K + 1, dtype=torch.float64, device=dev)
+    counts = torch.empty(K, dtype=torch.int64, device=dev)
+    ws_u, ws_w = ops.kmeans_accumulate_workspace(K, D, dev), ops.kmeans_accumulate_weighted_workspace(K, D, dev)
+    scratch = torch.zeros(2, dtype=torch.int64, device=dev)
+    result = torch.empty(3, dtype=torch.float64, device=dev)
+    labels_old = torch.full((npad,), -1, dtype=torch.int32, device=dev)
+    sums = packed[:K * D].view(K, D)
+
+    def iteration(weighted):
+        labels = ops.kmeans_assign(xt, ct, K)
+        if weighted:
+            ops.kmeans_accumulate_weighted(X, labels, w, K, sums=sums, wsums=packed[K * D:K * D + K], ws=ws_w)
+            ops.kmeans_pack_weighted(labels, labels_old, n, K, D, packed, scratch)
+            ops.kmeans_update_weighted(packed, cold, K, D, Kp, cnew, ct, result)
+        else:
+            ops.kmeans_accumulate(X, labels, K, sums=sums, counts=counts, ws=ws_u)
+            ops.kmeans_pack(labels, labels_old, n, counts, K, D, packed, scratch)
+            ops.kmeans_update(packed, cold, K, D, Kp, cnew, ct, result)
+        result.tolist()
+        return labels
+
+    def timed(fn, reps):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(reps):
+            out = fn()
+        e1.record()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / reps, out
+
+    for flag in (False, True, False, True):
+        iteration(flag)                                    # warm-up
+    rounds = {"unweighted": [], "weighted": []}
+    for _ in range(5):
+        rounds["unweighted"].append(timed(lambda: iteration(False), a.iters)[0])
+        rounds["weighted"].append(timed(lambda: iteration(True), a.iters)[0])
+    ops.PROFILE = {}
+    iteration(False)
+    labels = iteration(True)
+    torch.cuda.synchronize()
+    entries = {k: round(sum(s_.elapsed_time(e_) for s_, e_ in v), 4) for k, v in ops.PROFILE.items()}
+    ops.PROFILE = None
+    ops.kmeans_inertia(X, labels, cnew, w)
+    inert = {"weighted_ms": timed(lambda: ops.kmeans_inertia(X, labels, cnew, w), 20)[0],
+             "unweighted_ms": timed(lambda: ops.kmeans_inertia(X, labels, cnew), 20)[0]}
+    inert["algorithmic_gbs"] = (n * D * 4 + n * 8) / inert["weighted_ms"] / 1e6
+    seeder = GKMeans(n_clusters=K, init="k-means++", random_state=0)
+    seeder._seed_plusplus(X[:40000], xt[:, :40000].contiguous(), np.random.RandomState(0), w=w[:40000].contiguous())   # warm-up
+    seed_s = {}
+    for name, ww in (("unweighted", None), ("weighted", w), ("unweighted_again", None), ("weighted_again", w)):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        seeder._seed_plusplus(X, xt, np.random.RandomState(0), w=ww)
+        torch.cuda.synchronize()
+        seed_s[name] = time.perf_counter() - t0
+    smi = subprocess.run(["nvidia-smi", "-i", str(local), "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                         capture_output=True, text=True).stdout.strip()
+    med = {k: sorted(v)[len(v) // 2] for k, v in rounds.items()}
+    print(json.dumps({"metric": "kmeans_weighted_lloyd_iteration_ms", "ms_per_iteration_median": med,
+                      "ms_per_iteration_rounds": rounds, "weighted_over_unweighted": med["weighted"] / med["unweighted"],
+                      "entry_ms_one_iteration_each": entries, "inertia": inert, "seeding_seconds": seed_s,
+                      "points": n, "centroids": K, "dim": D, "gpu": torch.cuda.get_device_name(dev),
+                      "nvidia_smi_name_power_limit": smi}))
+
+
+if a.weighted:
+    assert world == 1, "--weighted runs on one GPU"
+    bench_weighted()
+    sys.exit(0)
 
 for _ in range(3):
     centers, _ = lloyd(centers)
