@@ -107,15 +107,19 @@ __global__ void bn_act_fwd_kernel(const float* __restrict__ x, int64_t ldx, floa
 }
 
 // g = dy * act'(u), u = gamma * xhat + beta;  sums[c] = (sum g, sum g * xhat)
+// FROZEN: BatchNorm with running statistics (mean / invstd are the running ones, eval-mode nn.BatchNorm).  Its dx = gamma * invstd * g
+// does not depend on the sums, so the same loop writes dx (the backward is one pass over dy and x, no apply kernel).
+template <bool FROZEN>
 __global__ void __launch_bounds__(512)
 bn_bwd_reduce_kernel(const float* __restrict__ dy, int64_t lddy, const float* __restrict__ x, int64_t ldx, int64_t M,
                      const float* __restrict__ mean, const float* __restrict__ invstd, const float* __restrict__ gamma,
-                     const float* __restrict__ beta, float slope, double* __restrict__ part) {
+                     const float* __restrict__ beta, float slope, double* __restrict__ part, float* __restrict__ dx, int64_t lddx) {
     __shared__ double red[16];
     const int c = blockIdx.x;
-    const float mu = mean[c], is = invstd[c], ga = gamma[c], be = beta[c];
+    const float mu = mean[c], is = invstd[c], ga = gamma[c], be = beta[c], kk = ga * is;
     const float* dr = dy + (int64_t)c * lddy;
     const float* xr = x + (int64_t)c * ldx;
+    float* o = FROZEN ? dx + (int64_t)c * lddx : nullptr;
     const int64_t per = (M + gridDim.y - 1) / gridDim.y;
     const int64_t i0 = per * blockIdx.y, i1 = (i0 + per) < M ? (i0 + per) : M;
     double s = 0.0, q = 0.0;
@@ -123,6 +127,7 @@ bn_bwd_reduce_kernel(const float* __restrict__ dy, int64_t lddy, const float* __
         const float xh = (xr[i] - mu) * is;
         const float u = fmaf(ga, xh, be);
         const float g = dr[i] * (u > 0.0f ? 1.0f : slope);
+        if (FROZEN) o[i] = kk * g;
         s += g;
         q += (double)g * xh;
     }
@@ -149,11 +154,15 @@ __global__ void bn_bwd_finish_kernel(const double* __restrict__ part, int C, int
 // The same two kernels for the BatchNorm that feeds max-over-k (model/dgcnn.py:55-58,118): the incoming gradient is dy (C, Mp)
 // at the arg-max edge of every (channel, point) and zero on the other k-1 edges, so the (C, Mp*k) tensor gfs_max_over_k_bwd would
 // write is never built: the sums run over the Mp arg-max edges only, the apply pass reads dy / arg per point.
+// FROZEN (running statistics): the CTA also writes dx = gamma * invstd * g for the k edges of each point of its slice, zero except
+// at the arg-max edge, VEC edges per thread (VEC = 4: k % 4 == 0 and dx rows 16-byte aligned, one float4 store; the slice starts on
+// a point, so a group never straddles two points).  x is read at the arg-max edge only.
+template <bool FROZEN, int VEC = 1>
 __global__ void __launch_bounds__(512)
 bn_bwd_reduce_argmax_kernel(const float* __restrict__ dy, int64_t lddy, const uint8_t* __restrict__ arg, int k,
                             const float* __restrict__ x, int64_t ldx, int64_t Mp, const float* __restrict__ mean,
                             const float* __restrict__ invstd, const float* __restrict__ gamma, const float* __restrict__ beta,
-                            float slope, double* __restrict__ part) {
+                            float slope, double* __restrict__ part, float* __restrict__ dx, int64_t lddx) {
     __shared__ double red[16];
     const int c = blockIdx.x;
     const float mu = mean[c], is = invstd[c], ga = gamma[c], be = beta[c];
@@ -163,12 +172,36 @@ bn_bwd_reduce_argmax_kernel(const float* __restrict__ dy, int64_t lddy, const ui
     const int64_t per = (Mp + gridDim.y - 1) / gridDim.y;
     const int64_t i0 = per * blockIdx.y, i1 = (i0 + per) < Mp ? (i0 + per) : Mp;
     double s = 0.0, q = 0.0;
-    for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
-        const float xh = (xr[i * k + ar[i]] - mu) * is;
-        const float u = fmaf(ga, xh, be);
-        const float g = dr[i] * (u > 0.0f ? 1.0f : slope);
-        s += g;
-        q += (double)g * xh;
+    if (FROZEN) {
+        const float kk = ga * is;
+        float* o = dx + (int64_t)c * lddx;
+        const int G = k / VEC, ng = (int)(i1 - i0) * G;                     // groups per point, in the slice (E < 2^31)
+        for (int t = threadIdx.x; t < ng; t += blockDim.x) {
+            const int pl = t / G, slot0 = (t - pl * G) * VEC;
+            const int64_t p = i0 + pl, i = p * k + slot0;
+            const int hit = (int)__ldg(ar + p) - slot0;                      // arg-max edge is element `hit` of this group
+            float g = 0.0f;
+            if (hit >= 0 && hit < VEC) {
+                const float xh = (__ldg(xr + i + hit) - mu) * is;
+                const float u = fmaf(ga, xh, be);
+                g = __ldg(dr + p) * (u > 0.0f ? 1.0f : slope);
+                s += g;
+                q += (double)g * xh;
+            }
+            float out[VEC];
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) out[e] = e == hit ? kk * g : 0.0f;
+            if (VEC == 4) *reinterpret_cast<float4*>(o + i) = make_float4(out[0], out[1], out[2], out[3]);
+            else o[i] = out[0];
+        }
+    } else {
+        for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+            const float xh = (xr[i * k + ar[i]] - mu) * is;
+            const float u = fmaf(ga, xh, be);
+            const float g = dr[i] * (u > 0.0f ? 1.0f : slope);
+            s += g;
+            q += (double)g * xh;
+        }
     }
     s = block_sum(s, red);
     q = block_sum(q, red);
@@ -705,7 +738,7 @@ extern "C" int gfs_bn_act_bwd(const float* dy, int64_t lddy, const float* x, int
                 "gfs_bn_act_bwd: bad argument");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int S = M >= 65536 ? BN_SPLIT : 1;
-    bn_bwd_reduce_kernel<<<dim3(C, S), 512, 0, st>>>(dy, lddy, x, ldx, M, mean, invstd, gamma, beta, slope, workspace);
+    bn_bwd_reduce_kernel<false><<<dim3(C, S), 512, 0, st>>>(dy, lddy, x, ldx, M, mean, invstd, gamma, beta, slope, workspace, nullptr, 0);
     GFS_LAUNCH_OK("bn_bwd_reduce_kernel");
     bn_bwd_finish_kernel<<<(C + 127) / 128, 128, 0, st>>>(workspace, C, S, sum_g, sum_gx);
     GFS_LAUNCH_OK("bn_bwd_finish_kernel");
@@ -722,7 +755,8 @@ extern "C" int gfs_bn_act_bwd_argmax(const float* dy, int64_t lddy, const uint8_
                 GFS_ERR_BAD_ARG, "gfs_bn_act_bwd_argmax: bad argument");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int S = Mp >= 65536 ? BN_SPLIT : 1;
-    bn_bwd_reduce_argmax_kernel<<<dim3(C, S), 512, 0, st>>>(dy, lddy, arg, k, x, ldx, Mp, mean, invstd, gamma, beta, slope, workspace);
+    bn_bwd_reduce_argmax_kernel<false><<<dim3(C, S), 512, 0, st>>>(dy, lddy, arg, k, x, ldx, Mp, mean, invstd, gamma, beta, slope, workspace,
+                                                                nullptr, 0);
     GFS_LAUNCH_OK("bn_bwd_reduce_argmax_kernel");
     bn_bwd_finish_kernel<<<(C + 127) / 128, 128, 0, st>>>(workspace, C, S, sum_g, sum_gx);
     GFS_LAUNCH_OK("bn_bwd_finish_kernel");
@@ -741,6 +775,47 @@ extern "C" int gfs_bn_act_bwd_argmax(const float* dy, int64_t lddy, const uint8_
     return GFS_OK;
 }
 
+extern "C" int gfs_bn_act_bwd_frozen(const float* dy, int64_t lddy, const float* x, int64_t ldx, float* dx, int64_t lddx, int C, int64_t M,
+                                     const float* mean, const float* invstd, const float* gamma, const float* beta, float slope,
+                                     double* workspace, float* sum_g, float* sum_gx, void* stream) {
+    GFS_REQUIRE(dy && x && dx && mean && invstd && gamma && beta && workspace && sum_g && sum_gx, GFS_ERR_BAD_ARG,
+                "gfs_bn_act_bwd_frozen: null pointer");
+    GFS_REQUIRE(C > 0 && M > 0, GFS_ERR_BAD_ARG, "gfs_bn_act_bwd_frozen: non-positive size (C=%d M=%lld)", C, (long long)M);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int S = M >= 65536 ? BN_SPLIT : 1;
+    bn_bwd_reduce_kernel<true><<<dim3(C, S), 512, 0, st>>>(dy, lddy, x, ldx, M, mean, invstd, gamma, beta, slope, workspace, dx, lddx);
+    GFS_LAUNCH_OK("bn_bwd_reduce_kernel<frozen>");
+    bn_bwd_finish_kernel<<<(C + 127) / 128, 128, 0, st>>>(workspace, C, S, sum_g, sum_gx);
+    GFS_LAUNCH_OK("bn_bwd_finish_kernel");
+    return GFS_OK;
+}
+
+extern "C" int gfs_bn_act_bwd_argmax_frozen(const float* dy, int64_t lddy, const uint8_t* arg, int k, const float* x, int64_t ldx,
+                                            float* dx, int64_t lddx, int C, int64_t Mp, const float* mean, const float* invstd,
+                                            const float* gamma, const float* beta, float slope, double* workspace, float* sum_g,
+                                            float* sum_gx, void* stream) {
+    GFS_REQUIRE(dy && arg && x && dx && mean && invstd && gamma && beta && workspace && sum_g && sum_gx, GFS_ERR_BAD_ARG,
+                "gfs_bn_act_bwd_argmax_frozen: null pointer");
+    GFS_REQUIRE(C > 0 && Mp > 0 && k > 0 && k <= 255, GFS_ERR_BAD_ARG, "gfs_bn_act_bwd_argmax_frozen: bad size (C=%d Mp=%lld k=%d)", C,
+                (long long)Mp, k);
+    GFS_REQUIRE(Mp * k < ((int64_t)1 << 31), GFS_ERR_UNSUPPORTED, "gfs_bn_act_bwd_argmax_frozen: Mp*k = %lld edges >= 2^31 per channel",
+                (long long)Mp * k);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // the CTAs of a channel split its E = Mp*k output edges, so the split follows E (the batch-statistic reduce reads Mp values)
+    const int S = Mp * k >= 65536 ? BN_SPLIT : 1;
+    const bool vec = (k % 4 == 0) && (lddx % 4 == 0) && ((reinterpret_cast<uintptr_t>(dx) & 15) == 0);
+    if (vec)
+        bn_bwd_reduce_argmax_kernel<true, 4><<<dim3(C, S), 512, 0, st>>>(dy, lddy, arg, k, x, ldx, Mp, mean, invstd, gamma, beta, slope,
+                                                                        workspace, dx, lddx);
+    else
+        bn_bwd_reduce_argmax_kernel<true, 1><<<dim3(C, S), 512, 0, st>>>(dy, lddy, arg, k, x, ldx, Mp, mean, invstd, gamma, beta, slope,
+                                                                        workspace, dx, lddx);
+    GFS_LAUNCH_OK("bn_bwd_reduce_argmax_kernel<frozen>");
+    bn_bwd_finish_kernel<<<(C + 127) / 128, 128, 0, st>>>(workspace, C, S, sum_g, sum_gx);
+    GFS_LAUNCH_OK("bn_bwd_finish_kernel");
+    return GFS_OK;
+}
+
 extern "C" int gfs_bn_bwd_sums(const float* dy, int64_t lddy, const float* x, int64_t ldx, int C, int64_t M, const float* mean,
                                const float* invstd, const float* gamma, const float* beta, float slope, double* workspace, float* sum_g,
                                float* sum_gx, void* stream) {
@@ -748,7 +823,7 @@ extern "C" int gfs_bn_bwd_sums(const float* dy, int64_t lddy, const float* x, in
                 "gfs_bn_bwd_sums: bad argument");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int S = M >= 65536 ? BN_SPLIT : 1;
-    bn_bwd_reduce_kernel<<<dim3(C, S), 512, 0, st>>>(dy, lddy, x, ldx, M, mean, invstd, gamma, beta, slope, workspace);
+    bn_bwd_reduce_kernel<false><<<dim3(C, S), 512, 0, st>>>(dy, lddy, x, ldx, M, mean, invstd, gamma, beta, slope, workspace, nullptr, 0);
     GFS_LAUNCH_OK("bn_bwd_reduce_kernel");
     bn_bwd_finish_kernel<<<(C + 127) / 128, 128, 0, st>>>(workspace, C, S, sum_g, sum_gx);
     GFS_LAUNCH_OK("bn_bwd_finish_kernel");

@@ -54,6 +54,8 @@ SIGNATURES = {
     "gfs_edge_scatter_bn_ordered": [_p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p],
     "gfs_bn_act_bwd": [_p, _i64, _p, _i64, _p, _i64, _i, _i64, _p, _p, _p, _p, _f, _p, _p, _p, _p],
     "gfs_bn_act_bwd_argmax": [_p, _i64, _p, _i, _p, _i64, _p, _i64, _i, _i64, _p, _p, _p, _p, _f, _p, _p, _p, _p],
+    "gfs_bn_act_bwd_frozen": [_p, _i64, _p, _i64, _p, _i64, _i, _i64, _p, _p, _p, _p, _f, _p, _p, _p, _p],
+    "gfs_bn_act_bwd_argmax_frozen": [_p, _i64, _p, _i, _p, _i64, _p, _i64, _i, _i64, _p, _p, _p, _p, _f, _p, _p, _p, _p],
     "gfs_edge_gather": [_p, _p, _i, _i, _i, _p, _p],
     "gfs_edge_gather_stats": [_p, _p, _i, _i, _i, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p, _p],
     "gfs_edge_scatter": [_p, _p, _i, _i, _i, _p, _p],

@@ -596,6 +596,34 @@ def bn_act_bwd_argmax(dy, arg, k, x, mean, invstd, gamma, beta, slope):
     return dx, sg, sgx
 
 
+def bn_act_bwd_frozen(dy, x, mean, invstd, gamma, beta, slope):
+    """bn_act_bwd for a BatchNorm that normalises with fixed (running) statistics: dx = gamma * invstd * g, no batch-statistic
+    terms; (sum_g, sum_gx) = (dbeta, dgamma).  One pass over dy and x"""
+    C, M = x.shape
+    dx = torch.empty(C, M, dtype=torch.float32, device=x.device)
+    sg = torch.empty(C, dtype=torch.float32, device=x.device)
+    sgx = torch.empty(C, dtype=torch.float32, device=x.device)
+    ws = torch.empty(2 * 16 * C, dtype=torch.float64, device=x.device)
+    _call("gfs_bn_act_bwd_frozen", 2, _ptr(dy), dy.stride(0), _ptr(x), x.stride(0), _ptr(dx), M, C, M, _ptr(mean), _ptr(invstd),
+          _ptr(gamma), _ptr(beta), float(slope), _ptr(ws), _ptr(sg), _ptr(sgx), _stream())
+    return dx, sg, sgx
+
+
+def bn_act_bwd_argmax_frozen(dy, arg, k, x, mean, invstd, gamma, beta, slope):
+    """bn_act_bwd_frozen(max_over_k_bwd(dy, arg, k), x, ...) without the (C, Mp*k) gradient in between; x is read at the arg-max
+    edges only"""
+    C, E = x.shape
+    Mp = arg.shape[1]
+    assert E == Mp * k and dy.shape == arg.shape
+    dx = torch.empty(C, E, dtype=torch.float32, device=x.device)
+    sg = torch.empty(C, dtype=torch.float32, device=x.device)
+    sgx = torch.empty(C, dtype=torch.float32, device=x.device)
+    ws = torch.empty(2 * 16 * C, dtype=torch.float64, device=x.device)
+    _call("gfs_bn_act_bwd_argmax_frozen", 2, _ptr(dy), dy.stride(0), _ptr(arg), k, _ptr(x), x.stride(0), _ptr(dx), E, C, Mp, _ptr(mean),
+          _ptr(invstd), _ptr(gamma), _ptr(beta), float(slope), _ptr(ws), _ptr(sg), _ptr(sgx), _stream())
+    return dx, sg, sgx
+
+
 def bn_act_max_fwd(z, scale, shift, slope, M, k):
     """max over the k slots of act(BN(z)) and its arg-max, one pass over z (C, M*k) -> y (C, M), arg (C, M) uint8"""
     C = z.shape[0]

@@ -1,9 +1,10 @@
 """torch.autograd.Functions of the training path over the C ABI (fp32, channel-major (C, M) tensors).
 
 Reference semantics: model.train() (train.py:614) -- BatchNorm with batch statistics, LeakyReLU(0.2) / ReLU, max over k with
-gradient to the arg-max edge, gather backward = scatter-add.  Every Function's forward AND backward run in the hand-written
-kernels of csrc/gemm_f32.cu + csrc/train.cu (+ csrc/knn.cu for the graph, which is not differentiated, as in the reference
-where knn returns integer indices)."""
+gradient to the arg-max edge, gather backward = scatter-add.  A BatchNorm whose module is in eval mode inside a training model
+is frozen, as in torch: it normalises with its running statistics, which it leaves unchanged (see batch_stats).  Every
+Function's forward AND backward run in the hand-written kernels of csrc/gemm_f32.cu + csrc/train.cu (+ csrc/knn.cu for the
+graph, which is not differentiated, as in the reference where knn returns integer indices)."""
 import torch
 
 from . import ops
@@ -28,10 +29,17 @@ def from_cm(x, B, N):
     return x.reshape(C, B, N).permute(1, 0, 2).contiguous()
 
 
+def batch_stats(bn):
+    """torch's rule (nn.modules.batchnorm._BatchNorm.forward): a BatchNorm normalises with the statistics of the batch iff it is
+    in training mode or keeps no running statistics; otherwise it is frozen"""
+    return bn.training or bn.running_mean is None
+
+
 def _bn_coeffs(z, gamma, beta, running_mean, running_var, training):
     if training:
         return ops.bn_stats_coeffs(z, gamma, beta, BN_EPS)           # mean, var, invstd, scale, shift in one call
-    mean, var = running_mean.float(), running_var.float()
+    # copies: the Functions return mean / var as outputs, which must not alias the module's buffers
+    mean, var = running_mean.detach().float().clone(), running_var.detach().float().clone()
     invstd = torch.rsqrt(var + BN_EPS)
     scale = (gamma * invstd).contiguous()
     shift = (beta - mean * scale).contiguous()
@@ -39,7 +47,8 @@ def _bn_coeffs(z, gamma, beta, running_mean, running_var, training):
 
 
 class ConvBNAct(torch.autograd.Function):
-    """y = act(BN(W x + bias)); x (I, M), W (O, I).  Returns (y, batch_mean, batch_var)."""
+    """y = act(BN(W x + bias)); x (I, M), W (O, I).  Returns (y, batch_mean, batch_var).
+    training=False: BN with the running statistics (returned in place of the batch ones)."""
 
     @staticmethod
     def forward(ctx, x, W, bias, gamma, beta, running_mean, running_var, slope, training):
@@ -57,12 +66,12 @@ class ConvBNAct(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy, _dm, _dv):
         x, W, z, mean, invstd, g, b = ctx.saved_tensors
-        if not ctx.training:
-            raise NotImplementedError("backward through eval-mode BatchNorm is not built")
-        dz, sg, sgx = ops.bn_act_bwd(dy.contiguous(), z, mean, invstd, g, b, ctx.slope)
-        dW = ops.conv_wgrad(dz, x)
-        dx = ops.conv_dgrad(W, dz) if ctx.needs_input_grad[0] else None
-        dbias = dz.sum(dim=1) if ctx.has_bias else None
+        need = ctx.needs_input_grad
+        bwd = ops.bn_act_bwd if ctx.training else ops.bn_act_bwd_frozen
+        dz, sg, sgx = bwd(dy.contiguous(), z, mean, invstd, g, b, ctx.slope)
+        dW = ops.conv_wgrad(dz, x) if need[1] else None
+        dx = ops.conv_dgrad(W, dz) if need[0] else None
+        dbias = dz.sum(dim=1) if ctx.has_bias and need[2] else None
         return dx, dW, dbias, sgx, sg, None, None, None, None
 
 
@@ -80,7 +89,8 @@ class ConvOnly(torch.autograd.Function):
     def backward(ctx, dz):
         x, W = ctx.saved_tensors
         dz = dz.contiguous()
-        return (ops.conv_dgrad(W, dz) if ctx.needs_input_grad[0] else None), ops.conv_wgrad(dz, x)
+        need = ctx.needs_input_grad
+        return (ops.conv_dgrad(W, dz) if need[0] else None), (ops.conv_wgrad(dz, x) if need[1] else None)
 
 
 class ConvConstW(torch.autograd.Function):
@@ -100,10 +110,12 @@ class ConvConstW(torch.autograd.Function):
 
 class EdgeConvTrain(torch.autograd.Function):
     """One EdgeConv block (model/dgcnn.py:35-41 + :53-58 + :118) in training mode.
-    x (C, M) channel-major, idx (B, N, k) int32 -> (y (64, M), mean1, var1, mean2, var2)."""
+    x (C, M) channel-major, idx (B, N, k) int32 -> (y (64, M), mean1, var1, mean2, var2).
+    train1 / train2: BN1 / BN2 use batch statistics; False: that BN is frozen and normalises with (rm, rv), its running
+    statistics, which are then returned as its mean / var."""
 
     @staticmethod
-    def forward(ctx, x, idx, W1, g1, b1, W2, g2, b2, B, N, k):
+    def forward(ctx, x, idx, W1, g1, b1, W2, g2, b2, B, N, k, train1=True, rm1=None, rv1=None, train2=True, rm2=None, rv2=None):
         x = x.contiguous()
         C, M = x.shape
         W1f = W1.detach().float().reshape(64, 2 * C)
@@ -115,16 +127,21 @@ class EdgeConvTrain(torch.autograd.Function):
         # tf32) would be of the order of the neighbour differences themselves
         ops.gemm_f32(Wpq, C, True, x, M, False, 128, M, C, pq, 128, c_trans=True, impl=_exact())   # point-major rows for the gather
         g1f, b1f, g2f, b2f = (t.detach().contiguous().float() for t in (g1, b1, g2, b2))
-        # (64, E) pre-BN1 tensor and its batch statistics / BN coefficients in one pass (the tile is summed while on chip)
-        H, (m1, v1, is1, sc1, sh1) = ops.edge_gather_stats(pq, idx, B, N, k, g1f, b1f, BN_EPS)
+        if train1:
+            # (64, E) pre-BN1 tensor and its batch statistics / BN coefficients in one pass (the tile is summed while on chip)
+            H, (m1, v1, is1, sc1, sh1) = ops.edge_gather_stats(pq, idx, B, N, k, g1f, b1f, BN_EPS)
+        else:
+            H = ops.edge_gather(pq, idx, B, N, k)
+            m1, v1, is1, sc1, sh1 = _bn_coeffs(H, g1f, b1f, rm1, rv1, False)
         del pq
         h1 = ops.bn_act_fwd(H, sc1, sh1, 0.2)
         W2f = W2.detach().float().reshape(64, 64).contiguous()
         Z = ops.conv_fwd(W2f, h1)                                                   # (64, E), pre-BN2
-        m2, v2, is2, sc2, sh2 = _bn_coeffs(Z, g2f, b2f, None, None, True)
+        m2, v2, is2, sc2, sh2 = _bn_coeffs(Z, g2f, b2f, rm2, rv2, train2)
         y, arg = ops.bn_act_max_fwd(Z, sc2, sh2, 0.2, M, k)                         # BN2 + LeakyReLU + max over k: one pass over Z
         ctx.save_for_backward(x, idx, Wpq, W2f, H, h1, Z, m1, is1, g1f, b1f, m2, is2, g2f, b2f, arg)
         ctx.dims = (B, N, k, C, M)
+        ctx.train = (train1, train2)
         ctx.mark_non_differentiable(m1, v1, m2, v2)
         return y, m1, v1, m2, v2
 
@@ -132,29 +149,43 @@ class EdgeConvTrain(torch.autograd.Function):
     def backward(ctx, dy, *_):
         x, idx, Wpq, W2f, H, h1, Z, m1, is1, g1, b1, m2, is2, g2, b2, arg = ctx.saved_tensors
         B, N, k, C, M = ctx.dims
+        train1, train2 = ctx.train
+        need = ctx.needs_input_grad
         # dy lives at the arg-max edge only: BN2's backward reads (dy, arg) directly, the (64, E) sparse gradient is never built
-        dZ, sg2, sgx2 = ops.bn_act_bwd_argmax(dy.contiguous(), arg, k, Z, m2, is2, g2, b2, 0.2)
-        dW2 = ops.conv_wgrad(dZ, h1)
+        bwd2 = ops.bn_act_bwd_argmax if train2 else ops.bn_act_bwd_argmax_frozen
+        dZ, sg2, sgx2 = bwd2(dy.contiguous(), arg, k, Z, m2, is2, g2, b2, 0.2)
+        dW2 = ops.conv_wgrad(dZ, h1).reshape(64, 64, 1, 1) if need[5] else None
         dh1 = ops.conv_dgrad(W2f, dZ)
         del dZ
         # BN1 / LeakyReLU backward is applied inside the scatter while its tile is staged: dH (64, E) is never built
-        sg1, sgx1 = ops.bn_bwd_sums(dh1, H, m1, is1, g1, b1, 0.2)
-        if torch.are_deterministic_algorithms_enabled():
-            # reproducible bits: each dP row is summed in ascending edge order instead of by atomics (one (E, 64) buffer of
-            # per-edge terms lives until the scatter returns)
-            dpq = ops.edge_scatter_bn(dh1, H, idx, B, N, k, m1, is1, g1, b1, 0.2, sg1, sgx1, ordered=True,
-                                      rev=ops.edge_reverse_index(idx, B, N))
-        else:
-            dpq = ops.edge_scatter_bn(dh1, H, idx, B, N, k, m1, is1, g1, b1, 0.2, sg1, sgx1)   # (M, 128): scatter-add over the graph
-        del dh1
-        dWpq = torch.empty(128, C, dtype=torch.float32, device=x.device)
-        ops.gemm_f32(dpq, 128, False, x, M, True, 128, C, M, dWpq, C, splitk=ops._splitk(M), impl=_exact())
-        dx = None
-        if ctx.needs_input_grad[0]:
-            dx = torch.empty(C, M, dtype=torch.float32, device=x.device)
-            ops.gemm_f32(Wpq, C, False, dpq, 128, True, C, M, 128, dx, M, impl=_exact())
-        dW1 = torch.cat([dWpq[:64] - dWpq[64:], dWpq[64:]], dim=1).reshape(64, 2 * C, 1, 1)
-        return dx, None, dW1, sgx1, sg1, dW2.reshape(64, 64, 1, 1), sgx2, sg2, None, None, None
+        sg1 = sgx1 = None
+        if train1 or need[3] or need[4]:
+            sg1, sgx1 = ops.bn_bwd_sums(dh1, H, m1, is1, g1, b1, 0.2)
+        dx = dW1 = None
+        if need[0] or need[2]:
+            if train1:
+                ag, agx = sg1, sgx1
+            else:
+                # frozen BN1: the scatter's apply step gamma*invstd*(g - sum_g/E - xhat*sum_gx/E) is exactly gamma*invstd*g when both
+                # sums are zero (g - 0 - xhat*0 == g in fp32), which is the running-statistic backward
+                ag = agx = torch.zeros(64, dtype=torch.float32, device=x.device)
+            if torch.are_deterministic_algorithms_enabled():
+                # reproducible bits: each dP row is summed in ascending edge order instead of by atomics (one (E, 64) buffer of
+                # per-edge terms lives until the scatter returns)
+                dpq = ops.edge_scatter_bn(dh1, H, idx, B, N, k, m1, is1, g1, b1, 0.2, ag, agx, ordered=True,
+                                          rev=ops.edge_reverse_index(idx, B, N))
+            else:
+                dpq = ops.edge_scatter_bn(dh1, H, idx, B, N, k, m1, is1, g1, b1, 0.2, ag, agx)   # (M, 128): scatter-add over the graph
+            del dh1
+            if need[2]:
+                dWpq = torch.empty(128, C, dtype=torch.float32, device=x.device)
+                ops.gemm_f32(dpq, 128, False, x, M, True, 128, C, M, dWpq, C, splitk=ops._splitk(M), impl=_exact())
+            if need[0]:
+                dx = torch.empty(C, M, dtype=torch.float32, device=x.device)
+                ops.gemm_f32(Wpq, C, False, dpq, 128, True, C, M, 128, dx, M, impl=_exact())
+            if need[2]:
+                dW1 = torch.cat([dWpq[:64] - dWpq[64:], dWpq[64:]], dim=1).reshape(64, 2 * C, 1, 1)
+        return (dx, None, dW1, sgx1, sg1, dW2, sgx2, sg2) + (None,) * 9
 
 
 class AttentionTrain(torch.autograd.Function):

@@ -2,7 +2,8 @@
 
 q/k/v 1x1 maps run as ONE fused gfs_linear_bf16 call (256 -> 3*64) whose bf16 output tiles are consumed in place by
 gfs_attention_fwd, a flash-style tcgen05 kernel (csrc/attention.cu): the N x N softmax(q^T k / sqrt(d)) matrix is never
-materialised.  Eval mode only (dropout is the identity); N must be a multiple of 128.
+materialised.  Eval mode only (dropout is the identity); N must be a multiple of 128.  The training path (forward_train) applies
+dropout iff the dropout module itself is in training mode.
 """
 import torch
 import torch.nn as nn
@@ -41,7 +42,7 @@ class SelfAttention(nn.Module):
         w = torch.cat([self.q_map.weight, self.k_map.weight, self.v_map.weight], dim=0).reshape(3 * self.out_channel, self.in_channel)
         qkv = ConvOnly.apply(x_cm, w)
         keep, seed = 1.0, 0
-        if self.dropout.p > 0:
+        if self.dropout.training and self.dropout.p > 0:
             # dropout on the attention weights (model/attention.py:45) without a mask tensor: the kernels hash (seed, row, column);
             # the seed advances per call from torch's seed, so torch.manual_seed makes a run repeatable (no host sync)
             keep = 1.0 - self.dropout.p

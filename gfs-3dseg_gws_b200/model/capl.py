@@ -126,13 +126,21 @@ class mpti_net_Point_GeoAsWeight_v2(nn.Module):
 
     def _features_train(self, x, need_semantic=False):
         """training mode (model/capl.py:324-362 under model.train()): fp32, batch-statistics BatchNorm, differentiable through
-        the hand-written training kernels (gfs3d/train_ops.py).  Same return convention as _features."""
-        from gfs3d.train_ops import ConvBNAct, ConvConstW, from_cm, update_running_stats
+        the hand-written training kernels (gfs3d/train_ops.py).  Same return convention as _features.
+        A BatchNorm in eval mode is frozen (running statistics, left unchanged).  A frozen encoder -- in eval mode, no parameter
+        requiring grad, x not requiring grad -- receives no gradient, so its eval-mode outputs come from the fused inference
+        kernels (bit-identical to self.encoder(x) in eval mode): no autograd graph and no per-edge tensors."""
+        from gfs3d.train_ops import ConvBNAct, ConvConstW, batch_stats, from_cm, to_cm, update_running_stats
         if not x.is_cuda:
             raise RuntimeError("the GW model needs CUDA tensors: the hot path has no CPU fallback")
         B, _, N = x.shape
         M = B * N
-        ecs, lvl2 = self.encoder.forward_train(x)                        # channel-major (64, M) x3, (256, M)
+        enc = self.encoder
+        if not enc.training and not x.requires_grad and not any(p.requires_grad for p in enc.parameters()):
+            out = enc.forward_fused(x, want_lvl2_cm=True)
+            ecs, lvl2 = list(to_cm(out.ec).split(64, dim=0)), to_cm(out.lvl2_cm)
+        else:
+            ecs, lvl2 = enc.forward_train(x)                             # channel-major (64, M) x3, (256, M)
         lvl3 = self.base_learner.forward_train(lvl2)
         att = self.att_learner.forward_train(lvl2, B, N)
         ec = torch.cat(ecs, dim=0)                                       # (192, M)
@@ -144,8 +152,10 @@ class mpti_net_Point_GeoAsWeight_v2(nn.Module):
         assignment = cosine_feat.argmax(dim=0).reshape(B, N).int()
         conv, bn = self.fusion[0], self.fusion[1]
         w = conv.weight.reshape(conv.weight.shape[0], conv.weight.shape[1])
-        pf, m, v = ConvBNAct.apply(torch.cat([cosine_feat, semantic], dim=0), w, conv.bias, bn.weight, bn.bias, None, None, 0.2, True)
-        update_running_stats(bn, m, v, M)
+        pf, m, v = ConvBNAct.apply(torch.cat([cosine_feat, semantic], dim=0), w, conv.bias, bn.weight, bn.bias, bn.running_mean,
+                                   bn.running_var, 0.2, batch_stats(bn))
+        if bn.training:
+            update_running_stats(bn, m, v, M)
         return from_cm(pf, B, N), assignment, (from_cm(semantic, B, N) if need_semantic else None)
 
     def getFeatures(self, x, segment_label=None):

@@ -209,8 +209,9 @@ class DGCNN(nn.Module):
 
     def forward_train(self, x):
         """training mode (model.train(), train.py:614): batch-statistics BatchNorm, fp32, autograd through the hand-written
-        forward/backward kernels of gfs3d/train_ops.py.  Returns channel-major tensors: ([ec_i (64, M)], out (mlp[-1], M))."""
-        from gfs3d.train_ops import ConvBNAct, EdgeConvTrain, from_cm, to_cm, update_running_stats
+        forward/backward kernels of gfs3d/train_ops.py.  Returns channel-major tensors: ([ec_i (64, M)], out (mlp[-1], M)).
+        Each BatchNorm follows its own mode: one in eval mode is frozen (running statistics, left unchanged)."""
+        from gfs3d.train_ops import ConvBNAct, EdgeConvTrain, batch_stats, from_cm, to_cm, update_running_stats
         if not x.is_cuda:
             raise RuntimeError("DGCNN needs CUDA tensors: the hot path has no CPU fallback")
         self._check_supported()
@@ -223,16 +224,20 @@ class DGCNN(nn.Module):
             (c1, b1), (c2, b2) = blk.stages()
             idx = ops.knn(cur_bcn, self.k)                       # integer graph: not differentiated (as in the reference)
             y, m1, v1, m2, v2 = EdgeConvTrain.apply(cur_cm, idx, c1.weight, b1.weight, b1.bias, c2.weight, b2.weight, b2.bias,
-                                                    B, N, self.k)
-            update_running_stats(b1, m1, v1, M * self.k)
-            update_running_stats(b2, m2, v2, M * self.k)
+                                                    B, N, self.k, batch_stats(b1), b1.running_mean, b1.running_var,
+                                                    batch_stats(b2), b2.running_mean, b2.running_var)
+            if b1.training:
+                update_running_stats(b1, m1, v1, M * self.k)
+            if b2.training:
+                update_running_stats(b2, m2, v2, M * self.k)
             outs.append(y)
             cur_cm, cur_bcn = y, from_cm(y.detach(), B, N)
         cur = torch.cat(outs, dim=0)
         for conv, bn in self.conv.stages():
             w = conv.weight.reshape(conv.weight.shape[0], conv.weight.shape[1])
-            cur, m, v = ConvBNAct.apply(cur, w, None, bn.weight, bn.bias, None, None, 0.2, True)
-            update_running_stats(bn, m, v, M)
+            cur, m, v = ConvBNAct.apply(cur, w, None, bn.weight, bn.bias, bn.running_mean, bn.running_var, 0.2, batch_stats(bn))
+            if bn.training:
+                update_running_stats(bn, m, v, M)
         return outs, cur
 
     def forward(self, x):
@@ -278,15 +283,18 @@ class BaseLearner(nn.Module):
         return self._folded.data
 
     def forward_train(self, x_cm):
-        """x_cm (in_channels, M) -> (params[-1], M); Conv1d(+bias)+BN with ReLU between layers, batch statistics"""
-        from gfs3d.train_ops import ConvBNAct, update_running_stats
+        """x_cm (in_channels, M) -> (params[-1], M); Conv1d(+bias)+BN with ReLU between layers, batch statistics (running ones for
+        a BatchNorm in eval mode)"""
+        from gfs3d.train_ops import ConvBNAct, batch_stats, update_running_stats
         M = x_cm.shape[1]
         cur = x_cm
         for i, seq in enumerate(self.convs):
             conv, bn = seq[0], seq[1]
             w = conv.weight.reshape(conv.weight.shape[0], conv.weight.shape[1])
-            cur, m, v = ConvBNAct.apply(cur, w, conv.bias, bn.weight, bn.bias, None, None, 0.0 if i != self.num_convs - 1 else 1.0, True)
-            update_running_stats(bn, m, v, M)
+            cur, m, v = ConvBNAct.apply(cur, w, conv.bias, bn.weight, bn.bias, bn.running_mean, bn.running_var,
+                                        0.0 if i != self.num_convs - 1 else 1.0, batch_stats(bn))
+            if bn.training:
+                update_running_stats(bn, m, v, M)
         return cur
 
     def forward_fused(self, x_act, B, N, y_act=None, y_kb0=0, y_cm=None):

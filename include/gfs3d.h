@@ -319,6 +319,21 @@ int gfs_bn_act_bwd(const float* dy, int64_t lddy, const float* x, int64_t ldx, f
 int gfs_bn_act_bwd_argmax(const float* dy, int64_t lddy, const uint8_t* arg, int k, const float* x, int64_t ldx, float* dx,
                           int64_t lddx, int C, int64_t Mp, const float* mean, const float* invstd, const float* gamma,
                           const float* beta, float slope, double* workspace, float* sum_g, float* sum_gx, void* stream);
+/* Frozen BatchNorm: the backward of y = act(gamma*xhat + beta) with xhat = (x - mean)*invstd taken from the RUNNING statistics
+ * (an eval-mode nn.BatchNorm1d/2d inside a training model, model/dgcnn.py:54-58,73-74): dx = gamma*invstd*g with g = dy*act'(u),
+ * no batch-statistic terms; sum_g = dbeta, sum_gx = dgamma.  Same arguments as gfs_bn_act_bwd / gfs_bn_act_bwd_argmax.  One
+ * pass over dy and x: every CTA writes dx for its slice and its fp64 partial sums, combined per channel in index order
+ * (deterministic, no floating-point atomics).
+ *   gfs_bn_act_bwd_frozen         (C, M) tensors, as gfs_bn_act_bwd
+ *   gfs_bn_act_bwd_argmax_frozen  the BatchNorm in front of max-over-k (model/dgcnn.py:55-58,118): reads (dy, arg) per point,
+ *                                 writes the (C, Mp*k) dx, zero except at the arg-max edge; the sums run over the arg-max edges.
+ *                                 Mp*k >= 2^31 is GFS_ERR_UNSUPPORTED.                                                         */
+int gfs_bn_act_bwd_frozen(const float* dy, int64_t lddy, const float* x, int64_t ldx, float* dx, int64_t lddx, int C, int64_t M,
+                          const float* mean, const float* invstd, const float* gamma, const float* beta, float slope,
+                          double* workspace, float* sum_g, float* sum_gx, void* stream);
+int gfs_bn_act_bwd_argmax_frozen(const float* dy, int64_t lddy, const uint8_t* arg, int k, const float* x, int64_t ldx, float* dx,
+                                 int64_t lddx, int C, int64_t Mp, const float* mean, const float* invstd, const float* gamma,
+                                 const float* beta, float slope, double* workspace, float* sum_g, float* sum_gx, void* stream);
 
 /* Fusions of the per-edge BatchNorm passes of the training EdgeConv (model/dgcnn.py:53-58,118 under model.train()):
  *   gfs_bn_act_max_fwd   y[c,i] = max_slot act(z[c, i*k+slot]*scale[c] + shift[c]) and its arg-max slot, in ONE pass over z:

@@ -5,11 +5,15 @@ forward + backward + Adam, data-parallel with one flat-bucket NCCL gradient all-
     python scripts/bench_train.py [--batch 32] [--steps 10]
     torchrun --nproc-per-node N scripts/bench_train.py
     python scripts/bench_train.py --deterministic
+    python scripts/bench_train.py --frozen
 
 Prints one JSON line (ms/step max over ranks, blocks/s whole job).  Attention dropout stays ON (p = 0.1) as in training.
 --deterministic (one GPU): times the default step and the step under torch.use_deterministic_algorithms(True, warn_only=True),
 with torch's NaN fill of uninitialised memory on and off, alternately for three rounds, and reports the ordered-scatter
-entry points' times next to the atomic scatter's."""
+entry points' times next to the atomic scatter's.
+--frozen (one GPU): alternates, for three rounds, the full step, the step with every BatchNorm frozen (eval mode inside the training
+model) and the frozen-encoder step (encoder in eval mode, no encoder parameter requiring grad: the fused inference encoder runs),
+and reports for each its ms/step, its peak allocated memory and the times of the frozen-BatchNorm backward entry points."""
 import argparse
 import json
 import os
@@ -33,6 +37,7 @@ ap.add_argument("--steps", type=int, default=10)
 ap.add_argument("--warmup", type=int, default=3)
 ap.add_argument("--npts", type=int, default=2048)
 ap.add_argument("--deterministic", action="store_true", help="compare the default and the deterministic step (one GPU)")
+ap.add_argument("--frozen", action="store_true", help="compare the full, the frozen-BatchNorm and the frozen-encoder step (one GPU)")
 a = ap.parse_args()
 world, rank, local = int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0))
 torch.cuda.set_device(local)
@@ -112,6 +117,67 @@ def bench_deterministic():
                       "peak_mem_gb": torch.cuda.max_memory_allocated() / 1e9,
                       "config": "ScanNet-shaped: 21 classes, 180 GWs, base_num 15, fwd+bwd+Adam, attention dropout 0.1"}))
 
+
+def bench_frozen():
+    import subprocess
+    bns = [mod for mod in m.modules() if isinstance(mod, torch.nn.modules.batchnorm._BatchNorm)]
+
+    def set_kind(name):
+        m.train()
+        m.encoder.requires_grad_(name != "frozen_encoder")
+        if name == "bn_frozen":
+            for bn in bns:
+                bn.eval()
+        elif name == "frozen_encoder":
+            m.encoder.eval()
+
+    kinds = ("full", "bn_frozen", "frozen_encoder")
+    for name in kinds:
+        set_kind(name)
+        for i in range(a.warmup):
+            step(i)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    rounds = {name: [] for name in kinds}
+    for _ in range(3):
+        for name in kinds:
+            set_kind(name)
+            torch.cuda.synchronize()
+            e0.record()
+            for i in range(a.steps):
+                step(i)
+            e1.record()
+            torch.cuda.synchronize()
+            rounds[name].append(round(e0.elapsed_time(e1) / a.steps, 3))
+    peak, entries = {}, {}
+    for name in kinds:
+        set_kind(name)
+        opt.zero_grad(set_to_none=True)
+        torch.cuda.synchronize()
+        torch.cuda.reset_peak_memory_stats()
+        step(0)
+        torch.cuda.synchronize()
+        peak[name] = round(torch.cuda.max_memory_allocated() / 1e9, 3)
+        ops.PROFILE = {}
+        step(0)
+        torch.cuda.synchronize()
+        entries[name] = {k: round(sum(s_.elapsed_time(e_) for s_, e_ in v), 3) for k, v in ops.PROFILE.items()
+                         if k.startswith(("gfs_bn_act_bwd", "gfs_bn_bwd_sums"))}
+        ops.PROFILE = None
+    set_kind("full")
+    smi = subprocess.run(["nvidia-smi", "-i", str(local), "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                         text=True).stdout.strip()
+    print(json.dumps({"metric": "gfs_train_step_ms_frozen", "ms_per_step_rounds": rounds,
+                      "ms_per_step_median": {k: sorted(v)[1] for k, v in rounds.items()}, "peak_mem_gb": peak,
+                      "bn_backward_entry_ms_per_step": entries, "steps_per_round": a.steps, "batch": a.batch, "npts": a.npts,
+                      "gpu": torch.cuda.get_device_name(dev), "nvidia_smi_name_power_limit": smi,
+                      "config": "ScanNet-shaped: 21 classes, 180 GWs, base_num 15, fwd+bwd+Adam, attention dropout 0.1"}))
+
+
+if a.frozen:
+    if world > 1:
+        sys.exit("--frozen runs on one GPU")
+    bench_frozen()
+    sys.exit(0)
 
 if a.deterministic:
     if world > 1:
