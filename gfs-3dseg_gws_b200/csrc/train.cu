@@ -275,8 +275,9 @@ __global__ void bn_bwd_apply_kernel(const float* __restrict__ dy, int64_t lddy, 
 // ------------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128)
 edge_gather_kernel(const float* __restrict__ pq, const int32_t* __restrict__ idx, int N, int k, int64_t E, float* __restrict__ H,
-                   float2* __restrict__ part) {
+                   double2* __restrict__ part) {
     __shared__ float T[64][129];
+    __shared__ double2 upper[64];                      // the (sum, sum of squares) of the second 64 edges
     const int64_t e0 = (int64_t)blockIdx.x * 128;
     const int q = threadIdx.x & 7, sub = threadIdx.x >> 3;
 #pragma unroll 2
@@ -303,32 +304,39 @@ edge_gather_kernel(const float* __restrict__ pq, const int32_t* __restrict__ idx
         for (int c = 0; c < 64; ++c) H[(int64_t)c * E + e] = T[c][threadIdx.x];
     if (part) {
         // BatchNorm statistics of H while the tile is on chip: thread (c, half) sums 64 edges of channel c (rows past E are
-        // zero); partials [c][2 * CTA + half] are combined in index order in fp64 by bn_stats_partials_kernel (deterministic)
+        // zero), the two halves are added, and partial [c][CTA] goes to bn_stats_partials_kernel, which combines them in index
+        // order (deterministic).  The sums are fp64, as in bn_stats_kernel: var = E[v^2] - mean^2 cancels (mean / sigma)^2 of
+        // the sums' rounding, so fp32 sums of 64 edges would lose the variance of a channel whose mean is far from 0.
         const int c = threadIdx.x & 63, half = threadIdx.x >> 6;
-        float sm = 0.0f, sq = 0.0f;
+        double sm = 0.0, sq = 0.0;
 #pragma unroll 8
         for (int el = half * 64; el < half * 64 + 64; ++el) {
-            const float v = T[c][el];
+            const double v = T[c][el];
             sm += v;
-            sq = fmaf(v, v, sq);
+            sq = fma(v, v, sq);
         }
-        part[(int64_t)c * (2 * gridDim.x) + 2 * blockIdx.x + half] = make_float2(sm, sq);
+        if (half) upper[c] = make_double2(sm, sq);
+        __syncthreads();
+        if (!half) {
+            const double2 o = upper[c];
+            part[(int64_t)c * gridDim.x + blockIdx.x] = make_double2(sm + o.x, sq + o.y);
+        }
     }
 }
 
 // per-channel statistics and affine coefficients from the partial (sum, sum of squares) pairs of edge_gather_kernel
 __global__ void __launch_bounds__(256)
-bn_stats_partials_kernel(const float2* __restrict__ part, int P, int64_t M, const float* __restrict__ gamma, const float* __restrict__ beta,
+bn_stats_partials_kernel(const double2* __restrict__ part, int P, int64_t M, const float* __restrict__ gamma, const float* __restrict__ beta,
                          float eps, float* __restrict__ mean, float* __restrict__ var, float* __restrict__ invstd,
                          float* __restrict__ scale, float* __restrict__ shift) {
     __shared__ double red[16];
     const int c = blockIdx.x;
-    const float2* row = part + (int64_t)c * P;
+    const double2* row = part + (int64_t)c * P;
     double s = 0.0, q = 0.0;
     for (int i = threadIdx.x; i < P; i += blockDim.x) {       // fixed assignment + fixed-order tree: deterministic
-        const float2 v = row[i];
-        s += (double)v.x;
-        q += (double)v.y;
+        const double2 v = row[i];
+        s += v.x;
+        q += v.y;
     }
     s = block_sum(s, red);
     q = block_sum(q, red);
@@ -916,9 +924,10 @@ extern "C" int gfs_edge_gather_stats(const float* pq, const int32_t* idx, int B,
     const int64_t E = (int64_t)B * N * k;
     const unsigned grid = (unsigned)((E + 127) / 128);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    edge_gather_kernel<<<grid, 128, 0, st>>>(pq, idx, N, k, E, H, reinterpret_cast<float2*>(partials));
+    GFS_REQUIRE((reinterpret_cast<uintptr_t>(partials) & 15) == 0, GFS_ERR_BAD_ARG, "gfs_edge_gather_stats: partials must be 16-byte aligned");
+    edge_gather_kernel<<<grid, 128, 0, st>>>(pq, idx, N, k, E, H, reinterpret_cast<double2*>(partials));
     GFS_LAUNCH_OK("edge_gather_kernel");
-    bn_stats_partials_kernel<<<64, 256, 0, st>>>(reinterpret_cast<const float2*>(partials), (int)(2 * grid), E, gamma, beta, eps, mean, var,
+    bn_stats_partials_kernel<<<64, 256, 0, st>>>(reinterpret_cast<const double2*>(partials), (int)grid, E, gamma, beta, eps, mean, var,
                                                  invstd, scale, shift);
     GFS_LAUNCH_OK("bn_stats_partials_kernel");
     return GFS_OK;

@@ -688,7 +688,7 @@ def edge_gather_stats(pq, idx, B, N, k, gamma, beta, eps):
     """edge_gather + bn_stats_coeffs(H) in one pass: -> H (64, E), (mean, var, invstd, scale, shift)"""
     E = B * N * k
     H = torch.empty(64, E, dtype=torch.float32, device=pq.device)
-    part = torch.empty(64 * 2 * ((E + 127) // 128) * 2, dtype=torch.float32, device=pq.device)
+    part = torch.empty(64 * ((E + 127) // 128) * 2, dtype=torch.float64, device=pq.device)      # fp64 (sum, sum of squares) per channel and tile
     out = torch.empty(5, 64, dtype=torch.float32, device=pq.device)
     _call("gfs_edge_gather_stats", 2, _ptr(pq), _ptr(idx), B, N, k, _ptr(H), _ptr(part), _ptr(gamma), _ptr(beta), float(eps),
           _ptr(out[0]), _ptr(out[1]), _ptr(out[2]), _ptr(out[3]), _ptr(out[4]), _stream())

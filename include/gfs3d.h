@@ -370,7 +370,8 @@ int gfs_edge_scatter_bn_ordered(const float* dy, const float* x, const int32_t* 
 /* edge tensor of model/dgcnn.py:35-41 after the split first conv: H[c, e] = P[j(e), c] + Q[i(e), c]  (pq point-major (M,128)) */
 int gfs_edge_gather(const float* pq, const int32_t* idx, int B, int N, int k, float* H, void* stream);
 /* the same plus the batch statistics of H and the BatchNorm coefficients (as gfs_bn_stats_coeffs) taken while the tiles are on
- * chip: no second pass over H.  partials: 64 * 2 * ceil(E/128) float pairs (sum, sum of squares), reduced in fp64 in a fixed order */
+ * chip: no second pass over H.  partials: 16-byte aligned workspace of 64 * ceil(E/128) fp64 pairs (sum, sum of squares), i.e.
+ * 64 * 4 * ceil(E/128) floats, accumulated and reduced in fp64 in a fixed order                                             */
 int gfs_edge_gather_stats(const float* pq, const int32_t* idx, int B, int N, int k, float* H, float* partials,
                           const float* gamma, const float* beta, float eps, float* mean, float* var, float* invstd,
                           float* scale, float* shift, void* stream);
