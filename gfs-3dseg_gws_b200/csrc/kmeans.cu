@@ -134,8 +134,10 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
     }
 }
 
-__global__ void kmeans_reduce_kernel(const float* __restrict__ partial, const int32_t* __restrict__ pcount, int P, int KD, int K,
-                                     double* __restrict__ sums, int64_t* __restrict__ counts) {
+// CTA-order reduction of the per-CTA tables: sums in fp64; int32 counts into int64, or fp64 weight sums into fp64
+template <typename PartialCount, typename Count>
+__global__ void kmeans_reduce_kernel(const float* __restrict__ partial, const PartialCount* __restrict__ pcount, int P, int KD, int K,
+                                     double* __restrict__ sums, Count* __restrict__ counts) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < KD) {
         double acc = 0.0;
@@ -143,25 +145,9 @@ __global__ void kmeans_reduce_kernel(const float* __restrict__ partial, const in
         sums[i] = acc;
     }
     if (i < K) {
-        int64_t c = 0;
+        Count c = 0;
         for (int p = 0; p < P; ++p) c += pcount[(size_t)p * K + i];
         counts[i] = c;
-    }
-}
-
-// weighted: the same CTA-order fp64 reduction; the per-CTA weight sums are fp64 already
-__global__ void kmeans_reduce_weighted_kernel(const float* __restrict__ partial, const double* __restrict__ pweight, int P, int KD,
-                                              int K, double* __restrict__ sums, double* __restrict__ wsums) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < KD) {
-        double acc = 0.0;
-        for (int p = 0; p < P; ++p) acc += (double)partial[(size_t)p * KD + i];
-        sums[i] = acc;
-    }
-    if (i < K) {
-        double w = 0.0;
-        for (int p = 0; p < P; ++p) w += pweight[(size_t)p * K + i];
-        wsums[i] = w;
     }
 }
 
@@ -184,7 +170,7 @@ extern "C" int gfs_kmeans_accumulate(const float* X, int64_t n, int D, const int
     GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_kernel<false>), 220 * 1024));
     kmeans_partial_kernel<false><<<P, KM_THREADS, smem, st>>>(X, n, D, labels, nullptr, K, partial, pcount, nullptr);
     GFS_LAUNCH_OK("kmeans_partial_kernel");
-    kmeans_reduce_kernel<<<(K * D + 255) / 256, 256, 0, st>>>(partial, pcount, P, K * D, K, sums, counts);
+    kmeans_reduce_kernel<int32_t, int64_t><<<(K * D + 255) / 256, 256, 0, st>>>(partial, pcount, P, K * D, K, sums, counts);
     GFS_LAUNCH_OK("kmeans_reduce_kernel");
     return GFS_OK;
 }
@@ -205,8 +191,8 @@ extern "C" int gfs_kmeans_accumulate_weighted(const float* X, int64_t n, int D, 
     GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_kernel<true>), 220 * 1024));
     kmeans_partial_kernel<true><<<P, KM_THREADS, smem, st>>>(X, n, D, labels, weights, K, partial, nullptr, pweight);
     GFS_LAUNCH_OK("kmeans_partial_kernel<weighted>");
-    kmeans_reduce_weighted_kernel<<<(K * D + 255) / 256, 256, 0, st>>>(partial, pweight, P, K * D, K, sums, wsums);
-    GFS_LAUNCH_OK("kmeans_reduce_weighted_kernel");
+    kmeans_reduce_kernel<double, double><<<(K * D + 255) / 256, 256, 0, st>>>(partial, pweight, P, K * D, K, sums, wsums);
+    GFS_LAUNCH_OK("kmeans_reduce_kernel<weighted>");
     return GFS_OK;
 }
 
@@ -216,16 +202,15 @@ namespace gfs {
 // The rest of a Lloyd iteration as two launches (it used to be ~25 elementwise / reduction launches of the host library:
 // at the sharded size of BASELINE.json configs[3], 500 k points per GPU, those fixed costs were half of the iteration).
 //
-//   kmeans_pack_kernel    packed = [sums (K*D, written by the reduce kernel) | counts as fp64 (K) | #labels changed (1)]
-//                         -- the ONE buffer the sharded version all-reduces (get_basis.py:210; SURVEY 8e)
+//   kmeans_pack_kernel    packed = [sums (K*D, written by the reduce kernel) | weight sums as fp64 (K) | #labels changed (1)]
+//                         -- the ONE buffer the sharded version all-reduces (get_basis.py:210; SURVEY 8e).  The weight sums
+//                         are the counts (copied here; exact integers, so the all-reduce keeps them exact) or, when counts
+//                         is NULL, the fp64 sums the weighted reduce kernel already wrote into the slot.
 //   kmeans_update_kernel  sklearn _k_means_common.pyx:_average_centers + the convergence quantities of _kmeans.py:_kmeans_single_lloyd:
-//                         new = count > 0 ? sums / count : 0 (an empty cluster keeps the zero sum; the rare relocation is the
+//                         new = wsum > 0 ? sums / wsum : 0 (an empty cluster keeps the zero sum; the rare relocation is the
 //                         caller's), shift = sum (new - old)^2 (fp64, fixed order), #empty; also the transposed (D, Kp) copy of
 //                         the new centres that the next E-step reads.  result = [changed, shift, empty] (fp64) = one D2H read.
 // ---------------------------------------------------------------------------------------------------------------
-// WEIGHTED: the weight slot packed[K*D : K*D+K] is already filled (gfs_kmeans_accumulate_weighted wrote it), so only the
-// changed-label count is written; WEIGHTED update divides by the fp64 weight sums as they are (no rounding to a count).
-template <bool WEIGHTED>
 __global__ void __launch_bounds__(256)
 kmeans_pack_kernel(const int32_t* __restrict__ labels, const int32_t* __restrict__ labels_old, int64_t n, const int64_t* __restrict__ counts,
                    int K, int KD, double* __restrict__ packed, unsigned long long* __restrict__ scratch) {
@@ -243,7 +228,7 @@ kmeans_pack_kernel(const int32_t* __restrict__ labels, const int32_t* __restrict
     __syncthreads();
     if (!last) return;
     __threadfence();
-    if constexpr (!WEIGHTED)
+    if (counts)
         for (int c = threadIdx.x; c < K; c += blockDim.x) packed[KD + c] = (double)counts[c];
     if (threadIdx.x == 0) {
         packed[KD + K] = (double)atomicAdd(&scratch[0], 0ull);
@@ -252,7 +237,6 @@ kmeans_pack_kernel(const int32_t* __restrict__ labels, const int32_t* __restrict
     }
 }
 
-template <bool WEIGHTED>
 __global__ void __launch_bounds__(1024)
 kmeans_update_kernel(const double* __restrict__ packed, const float* __restrict__ centers_old, int K, int D, int Kp,
                      float* __restrict__ centers_new, float* __restrict__ ct, double* __restrict__ result) {
@@ -261,15 +245,15 @@ kmeans_update_kernel(const double* __restrict__ packed, const float* __restrict_
     double shift = 0.0;
     for (int i = threadIdx.x; i < KD; i += 1024) {
         const int c = i / D, d = i - c * D;
-        const double cnt = WEIGHTED ? packed[KD + c] : rint(packed[KD + c]);
-        const float nw = cnt > 0.0 ? (float)(packed[i] / cnt) : 0.0f;
+        const double wsum = packed[KD + c];
+        const float nw = wsum > 0.0 ? (float)(packed[i] / wsum) : 0.0f;
         const double df = (double)(nw - centers_old[i]);
         shift += df * df;
         centers_new[i] = nw;
         ct[(int64_t)d * Kp + c] = nw;
     }
     double empty = 0.0;
-    for (int c = threadIdx.x; c < K; c += 1024) empty += (WEIGHTED ? packed[KD + c] : rint(packed[KD + c])) > 0.0 ? 0.0 : 1.0;
+    for (int c = threadIdx.x; c < K; c += 1024) empty += packed[KD + c] > 0.0 ? 0.0 : 1.0;
 #pragma unroll
     for (int o = 16; o >= 1; o >>= 1) {
         shift += __shfl_xor_sync(0xffffffffu, shift, o);
@@ -299,47 +283,23 @@ kmeans_update_kernel(const double* __restrict__ packed, const float* __restrict_
 extern "C" int gfs_kmeans_pack(const int32_t* labels, const int32_t* labels_old, int64_t n, const int64_t* counts, int K, int D,
                                double* packed, void* scratch16, void* stream) {
     using namespace gfs;
-    GFS_REQUIRE(labels && labels_old && counts && packed && scratch16 && n > 0 && K > 0 && D > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_pack: bad argument");
+    GFS_REQUIRE(labels && labels_old && packed && scratch16, GFS_ERR_BAD_ARG, "gfs_kmeans_pack: null pointer");
+    GFS_REQUIRE(n > 0 && K > 0 && D > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_pack: non-positive size");
     const int64_t want = (n + 256 * 8 - 1) / (256 * 8);
     const unsigned grid = (unsigned)(want < 1 ? 1 : want > 592 ? 592 : want);
-    kmeans_pack_kernel<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(labels, labels_old, n, counts, K, K * D, packed,
-                                                                                  static_cast<unsigned long long*>(scratch16));
+    kmeans_pack_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(labels, labels_old, n, counts, K, K * D, packed,
+                                                                           static_cast<unsigned long long*>(scratch16));
     GFS_LAUNCH_OK("kmeans_pack_kernel");
-    return GFS_OK;
-}
-
-extern "C" int gfs_kmeans_pack_weighted(const int32_t* labels, const int32_t* labels_old, int64_t n, int K, int D, double* packed,
-                                        void* scratch16, void* stream) {
-    using namespace gfs;
-    GFS_REQUIRE(labels && labels_old && packed && scratch16, GFS_ERR_BAD_ARG, "gfs_kmeans_pack_weighted: null pointer");
-    GFS_REQUIRE(n > 0 && K > 0 && D > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_pack_weighted: non-positive size");
-    const int64_t want = (n + 256 * 8 - 1) / (256 * 8);
-    const unsigned grid = (unsigned)(want < 1 ? 1 : want > 592 ? 592 : want);
-    kmeans_pack_kernel<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(labels, labels_old, n, nullptr, K, K * D, packed,
-                                                                                 static_cast<unsigned long long*>(scratch16));
-    GFS_LAUNCH_OK("kmeans_pack_kernel<weighted>");
     return GFS_OK;
 }
 
 extern "C" int gfs_kmeans_update(const double* packed, const float* centers_old, int K, int D, int Kp, float* centers_new, float* centers_t,
                                  double* result3, void* stream) {
     using namespace gfs;
-    GFS_REQUIRE(packed && centers_old && centers_new && centers_t && result3 && K > 0 && D > 0 && Kp >= K, GFS_ERR_BAD_ARG,
-                "gfs_kmeans_update: bad argument");
-    kmeans_update_kernel<false><<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(packed, centers_old, K, D, Kp, centers_new, centers_t,
-                                                                                   result3);
+    GFS_REQUIRE(packed && centers_old && centers_new && centers_t && result3, GFS_ERR_BAD_ARG, "gfs_kmeans_update: null pointer");
+    GFS_REQUIRE(K > 0 && D > 0 && Kp >= K, GFS_ERR_BAD_ARG, "gfs_kmeans_update: bad size");
+    kmeans_update_kernel<<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(packed, centers_old, K, D, Kp, centers_new, centers_t, result3);
     GFS_LAUNCH_OK("kmeans_update_kernel");
-    return GFS_OK;
-}
-
-extern "C" int gfs_kmeans_update_weighted(const double* packed, const float* centers_old, int K, int D, int Kp, float* centers_new,
-                                          float* centers_t, double* result3, void* stream) {
-    using namespace gfs;
-    GFS_REQUIRE(packed && centers_old && centers_new && centers_t && result3, GFS_ERR_BAD_ARG, "gfs_kmeans_update_weighted: null pointer");
-    GFS_REQUIRE(K > 0 && D > 0 && Kp >= K, GFS_ERR_BAD_ARG, "gfs_kmeans_update_weighted: bad size");
-    kmeans_update_kernel<true><<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(packed, centers_old, K, D, Kp, centers_new, centers_t,
-                                                                                  result3);
-    GFS_LAUNCH_OK("kmeans_update_kernel<weighted>");
     return GFS_OK;
 }
 
@@ -431,7 +391,7 @@ kmeans_pp_trial_kernel(const float* __restrict__ xt, int64_t npad, int64_t n, in
 }  // namespace gfs
 
 extern "C" int gfs_kmeans_pp_trial(const float* xt, int64_t npad, int64_t n, int D, const double* xsq, const float* cand, int T,
-                                   const float* closest, float* m_out, double* pots, void* stream) {
+                                   const float* closest, const float* weights, float* m_out, double* pots, void* stream) {
     using namespace gfs;
     GFS_REQUIRE(xt && xsq && cand && m_out && pots, GFS_ERR_BAD_ARG, "gfs_kmeans_pp_trial: null pointer");
     GFS_REQUIRE(n > 0 && npad >= n && D > 0 && T > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_pp_trial: non-positive size");
@@ -440,25 +400,11 @@ extern "C" int gfs_kmeans_pp_trial(const float* xt, int64_t npad, int64_t n, int
     const size_t smem = (size_t)(D * PP_T + PP_T) * sizeof(double);
     const int64_t grid = (n + PP_THREADS - 1) / PP_THREADS;
     GFS_REQUIRE(grid < ((int64_t)1 << 31), GFS_ERR_UNSUPPORTED, "gfs_kmeans_pp_trial: n too large");
-    kmeans_pp_trial_kernel<false><<<(unsigned)grid, PP_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(xt, npad, n, D, xsq, cand, T,
-                                                                                                       closest, nullptr, m_out, pots);
+    // unit weights run the instance without the weight load and product
+    const auto kernel = weights ? kmeans_pp_trial_kernel<true> : kmeans_pp_trial_kernel<false>;
+    kernel<<<(unsigned)grid, PP_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(xt, npad, n, D, xsq, cand, T, closest, weights,
+                                                                                    m_out, pots);
     GFS_LAUNCH_OK("kmeans_pp_trial_kernel");
-    return GFS_OK;
-}
-
-extern "C" int gfs_kmeans_pp_trial_weighted(const float* xt, int64_t npad, int64_t n, int D, const double* xsq, const float* cand, int T,
-                                            const float* closest, const float* weights, float* m_out, double* pots, void* stream) {
-    using namespace gfs;
-    GFS_REQUIRE(xt && xsq && cand && weights && m_out && pots, GFS_ERR_BAD_ARG, "gfs_kmeans_pp_trial_weighted: null pointer");
-    GFS_REQUIRE(n > 0 && npad >= n && D > 0 && T > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_pp_trial_weighted: non-positive size");
-    GFS_REQUIRE(T <= PP_T, GFS_ERR_UNSUPPORTED, "gfs_kmeans_pp_trial_weighted: T=%d candidates > %d is not built", T, PP_T);
-    GFS_REQUIRE(D <= 512, GFS_ERR_UNSUPPORTED, "gfs_kmeans_pp_trial_weighted: D=%d > 512 is not built", D);
-    const size_t smem = (size_t)(D * PP_T + PP_T) * sizeof(double);
-    const int64_t grid = (n + PP_THREADS - 1) / PP_THREADS;
-    GFS_REQUIRE(grid < ((int64_t)1 << 31), GFS_ERR_UNSUPPORTED, "gfs_kmeans_pp_trial_weighted: n too large");
-    kmeans_pp_trial_kernel<true><<<(unsigned)grid, PP_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(xt, npad, n, D, xsq, cand, T,
-                                                                                                      closest, weights, m_out, pots);
-    GFS_LAUNCH_OK("kmeans_pp_trial_kernel<weighted>");
     return GFS_OK;
 }
 

@@ -34,11 +34,8 @@ SIGNATURES = {
     "gfs_kmeans_accumulate": [_p, _i64, _i, _p, _i, _p, _p, _p, _p, _p],
     "gfs_kmeans_pack": [_p, _p, _i64, _p, _i, _i, _p, _p, _p],
     "gfs_kmeans_update": [_p, _p, _i, _i, _i, _p, _p, _p, _p],
-    "gfs_kmeans_pp_trial": [_p, _i64, _i64, _i, _p, _p, _i, _p, _p, _p, _p],
+    "gfs_kmeans_pp_trial": [_p, _i64, _i64, _i, _p, _p, _i, _p, _p, _p, _p, _p],
     "gfs_kmeans_accumulate_weighted": [_p, _i64, _i, _p, _p, _i, _p, _p, _p, _p, _p],
-    "gfs_kmeans_pack_weighted": [_p, _p, _i64, _i, _i, _p, _p, _p],
-    "gfs_kmeans_update_weighted": [_p, _p, _i, _i, _i, _p, _p, _p, _p],
-    "gfs_kmeans_pp_trial_weighted": [_p, _i64, _i64, _i, _p, _p, _i, _p, _p, _p, _p, _p],
     "gfs_kmeans_inertia": [_p, _i64, _i, _p, _p, _i, _p, _p, _p, _p],
     # training path
     "gfs_gemm_f32": [_p, _i64, _i, _i64, _p, _i64, _i, _i64, _p, _i64, _i, _i64, _p, _i, _i, _i, _i, _i, _p, _i, _p],

@@ -83,13 +83,20 @@ class KMeans:
                               group=self.process_group)
         return t
 
+    def _owned_rows(self, Xc, n, pos, mine):
+        """(T, D) rows Xc[pos] where this rank owns the pick, zero elsewhere; summed over the ranks"""
+        rows = Xc[pos.clamp(0, n - 1)] * mine.to(torch.float32).unsqueeze(1)
+        if self._world()[0] > 1:
+            _dist().all_reduce(rows, group=self.process_group)
+        return rows.contiguous()
+
     def _seed_random(self, Xc, rng, n, w=None):
         """sklearn _kmeans.py:1030-1037: K distinct rows drawn with choice(n, size=K, replace=False, p=w/sum(w)) -- p is passed
         with unit weights too, as sklearn does (numpy draws differently without it).  Sharded: drawn on rank 0 over the points
         of all ranks in rank order, each row contributed by its owner rank."""
         K = self.n_clusters
         dev = Xc.device
-        world, rank = self._world()
+        _, rank = self._world()
         sizes = self._gather_sizes(n, dev)
         n_tot, lo = sum(sizes), sum(sizes[:rank])
         wall = self._gather_weights(w, sizes) if w is not None else None
@@ -99,11 +106,7 @@ class KMeans:
             idx[:] = torch.from_numpy(rng.choice(n_tot, size=K, replace=False, p=wa / wa.sum()).astype(np.int64))
         idx = self._broadcast0(idx.to(dev))
         pos = idx - lo
-        mine = (pos >= 0) & (pos < n)
-        rows = Xc[pos.clamp(0, n - 1)] * mine.to(torch.float32).unsqueeze(1)
-        if world > 1:
-            _dist().all_reduce(rows, group=self.process_group)
-        return rows.contiguous()
+        return self._owned_rows(Xc, n, pos, (pos >= 0) & (pos < n))
 
     def _seed_plusplus(self, Xc, xt, rng, n=None, w=None):
         """k-means++ exactly as sklearn's _kmeans_plusplus consumes its random stream (sklearn 1.9.0 _kmeans.py:_kmeans_plusplus):
@@ -119,8 +122,8 @@ class KMeans:
         the single-GPU picks.  The random numbers are drawn on rank 0 and broadcast.  No host synchronisation inside the loop.
 
         Weighted (w: this rank's (n,) fp32 weights): the first centre is choice(n, p=w/sum(w)) over the weights of all ranks
-        (all-gathered once), the potentials are sum_i w_i * closest_i (gfs_kmeans_pp_trial_weighted) and the candidates come
-        from the cumulative sum of w * closest; `closest` itself stays unweighted, as in sklearn."""
+        (all-gathered once), the potentials are sum_i w_i * closest_i (gfs_kmeans_pp_trial with the weights) and the candidates
+        come from the cumulative sum of w * closest; `closest` itself stays unweighted, as in sklearn."""
         D = Xc.shape[1]
         n = Xc.shape[0] if n is None else n
         K = self.n_clusters
@@ -138,10 +141,7 @@ class KMeans:
             wa = wall if wall is not None else np.ones(n_tot, dtype=np.float32)
             draws[0] = float(rng.choice(n_tot, p=wa / wa.sum()))
             draws[1:] = torch.from_numpy(rng.uniform(size=(K - 1) * trials)) if K > 1 else draws[1:]
-        draws = draws.to(dev)
-        if world > 1:
-            _dist().broadcast(draws, src=_dist().get_global_rank(self.process_group, 0) if self.process_group else 0,
-                              group=self.process_group)
+        draws = self._broadcast0(draws.to(dev))
         U = draws[1:].view(K - 1, trials)
         npad = xt.shape[1]
         xsq = torch.zeros(npad, dtype=torch.float64, device=dev)
@@ -149,23 +149,9 @@ class KMeans:
         centers = torch.empty(K, D, dtype=torch.float32, device=dev)
         m = torch.empty(8, npad, dtype=torch.float32, device=dev)
         pots = torch.zeros(8, dtype=torch.float64, device=dev)
-
-        def owned_rows(pos, mine):
-            """(T, D) rows X[pos] where this rank owns the pick, zero elsewhere; summed over the ranks"""
-            rows = Xc[pos.clamp(0, n - 1)] * mine.to(torch.float32).unsqueeze(1)
-            if world > 1:
-                _dist().all_reduce(rows, group=self.process_group)
-            return rows.contiguous()
-
         first = draws[0].long() - lo
-        centers[0] = owned_rows(first.view(1), ((first >= 0) & (first < n)).view(1))[0]
-        def trial(cand, closest):
-            if w is None:
-                ops.kmeans_pp_trial(xt, n, xsq, cand, closest, m, pots)
-            else:
-                ops.kmeans_pp_trial_weighted(xt, n, xsq, cand, closest, w, m, pots)
-
-        trial(centers[0:1].contiguous(), None)
+        centers[0] = self._owned_rows(Xc, n, first.view(1), ((first >= 0) & (first < n)).view(1))[0]
+        ops.kmeans_pp_trial(xt, n, xsq, centers[0:1].contiguous(), None, m, pots, weights=w)
         if world > 1:
             _dist().all_reduce(pots, group=self.process_group)
         closest, pot = m[0].clone(), pots[0].clone()
@@ -182,9 +168,9 @@ class KMeans:
             owner = torch.searchsorted(P, rv).clamp_max(world - 1)  # first rank whose slice reaches rv (the last one if none: numpy's clip)
             mine = owner == rank
             pos = torch.searchsorted(cs, rv - (P[rank] - tots[rank])).clamp_max(n - 1)   # first i with cumsum[i] >= rv (side='left')
-            cand = owned_rows(pos, mine)
+            cand = self._owned_rows(Xc, n, pos, mine)
             pots.zero_()
-            trial(cand, closest)
+            ops.kmeans_pp_trial(xt, n, xsq, cand, closest, m, pots, weights=w)
             if world > 1:
                 _dist().all_reduce(pots, group=self.process_group)
             best = torch.argmin(pots[:trials]).view(1)
@@ -310,9 +296,9 @@ class KMeans:
         dev = Xc.device
         npad = xt.shape[1]
         # Lloyd iterations.  Per iteration: E-step (4 launches), M-step sums (2), pack (1), ONE collective of the packed
-        # [sums | counts | labels changed] buffer when sharded, centre update (1) and ONE device->host read of
-        # (labels changed, centre shift, empty clusters).  All buffers are allocated once.  Weighted: the same launches, with
-        # the fp64 weight sums in the counts' slot.
+        # [sums | weight sums | labels changed] buffer when sharded, centre update (1) and ONE device->host read of
+        # (labels changed, centre shift, empty clusters).  All buffers are allocated once.  Unweighted, the weight sums are
+        # the counts, which pack copies into their slot; weighted, the M-step writes them there.
         Kp = (K + 3) // 4 * 4
         ct = torch.zeros(D, Kp, dtype=torch.float32, device=dev)
         ct[:, :K] = centers.t()
@@ -320,12 +306,12 @@ class KMeans:
         centers_new = torch.empty_like(centers)
         labels_old = torch.full((npad,), -1, dtype=torch.int32, device=dev)
         packed = torch.empty(K * D + K + 1, dtype=torch.float64, device=dev)
-        sums = packed[:K * D].view(K, D)
+        sums, wsums = packed[:K * D].view(K, D), packed[K * D:K * D + K]
         if w is None:
             counts = torch.empty(K, dtype=torch.int64, device=dev)
             acc_ws = ops.kmeans_accumulate_workspace(K, D, dev)
         else:
-            wsums = packed[K * D:K * D + K]
+            counts = None
             acc_ws = ops.kmeans_accumulate_weighted_workspace(K, D, dev)
         scratch = torch.zeros(2, dtype=torch.int64, device=dev)
         result = torch.empty(3, dtype=torch.float64, device=dev)
@@ -340,28 +326,17 @@ class KMeans:
             labels = assign()                                          # ct holds the current centres, transposed
             if w is None:
                 ops.kmeans_accumulate(Xc, labels, K, n_valid=n, sums=sums, counts=counts, ws=acc_ws)
-                ops.kmeans_pack(labels, labels_old, n, counts, K, D, packed, scratch)
             else:
                 ops.kmeans_accumulate_weighted(Xc, labels, w, K, n_valid=n, sums=sums, wsums=wsums, ws=acc_ws)
-                ops.kmeans_pack_weighted(labels, labels_old, n, K, D, packed, scratch)
+            ops.kmeans_pack(labels, labels_old, n, K, D, packed, scratch, counts=counts)
             if self.shard:
                 _dist().all_reduce(packed, group=self.process_group)
-            if w is None:
-                ops.kmeans_update(packed, centers, K, D, Kp, centers_new, ct, result)
-            else:
-                ops.kmeans_update_weighted(packed, centers, K, D, Kp, centers_new, ct, result)
+            ops.kmeans_update(packed, centers, K, D, Kp, centers_new, ct, result)
             n_changed, shift_h, n_empty = result.tolist()
             if n_empty > 0:           # rare: sklearn moves the empty clusters onto the points farthest from their centres
-                gsums = packed[:K * D].view(K, D).clone()
-                if w is None:
-                    gcounts = packed[K * D:K * D + K].round().long()
-                    gsums, gcounts = self._relocate_empty(Xc, n, labels, centers, gsums, gcounts)
-                    # clusters that are still empty keep the zero sum (sklearn _k_means_common.pyx:_average_centers)
-                    new = torch.where(gcounts[:, None] > 0, gsums / gcounts.clamp_min(1)[:, None].double(), torch.zeros_like(gsums)).float()
-                else:
-                    gw = packed[K * D:K * D + K].clone()
-                    gsums, gw = self._relocate_empty(Xc, n, labels, centers, gsums, gw, w=w)
-                    new = torch.where(gw[:, None] > 0, gsums / torch.where(gw > 0, gw, 1.0)[:, None], torch.zeros_like(gsums)).float()
+                gsums, gw = self._relocate_empty(Xc, n, labels, centers, sums.clone(), wsums.clone(), w)
+                # clusters that are still empty keep the zero sum (sklearn _k_means_common.pyx:_average_centers)
+                new = torch.where(gw[:, None] > 0, gsums / torch.where(gw > 0, gw, 1.0)[:, None], torch.zeros_like(gsums)).float()
                 shift_h = float(((new - centers).double() ** 2).sum())
                 centers_new.copy_(new)
                 ct[:, :K] = new.t()
@@ -380,45 +355,13 @@ class KMeans:
         torch.cuda.synchronize(dev)
         return labels, centers, n_iter, ev0.elapsed_time(ev1)
 
-    def _relocate_empty(self, Xc, n, labels, centers, sums, counts, w=None):
-        """sklearn _k_means_common.pyx:167-211: every empty cluster is moved onto one of the points farthest from its own
-        (old) centre, and that point is taken out of its old cluster's sum.  Rare path, plain device ops.  Sharded: each
-        rank offers its n_empty farthest points (distance, old label, coordinates), the candidates are all-gathered and
-        every rank applies the same global choice to the (already all-reduced) sums / counts.
-
-        Weighted (w given, counts = the fp64 weight sums): the farthest points are still chosen by unweighted distance;
-        then sums[old] -= w x, sums[e] = w x (an fp32 product, as sklearn), counts[e] = w, counts[old] -= w.  The weight
-        travels next to each candidate row."""
-        if w is not None:
-            return self._relocate_empty_weighted(Xc, n, labels, centers, sums, counts, w)
-        empty = (counts == 0).nonzero().flatten()
-        ne = int(empty.numel())
-        D = Xc.shape[1]
-        dist = ((Xc - centers[labels[:n].long()]) ** 2).sum(1)
-        m = min(ne, n)
-        vals, idxs = torch.topk(dist, m)
-        cand = torch.full((ne, 2 + D), float("-inf"), dtype=torch.float64, device=Xc.device)
-        cand[:m, 0] = vals.double()
-        cand[:m, 1] = labels[idxs].double()
-        cand[:m, 2:] = Xc[idxs].double()
-        if self.shard:
-            world = _dist().get_world_size(self.process_group)
-            gathered = [torch.empty_like(cand) for _ in range(world)]
-            _dist().all_gather(gathered, cand, group=self.process_group)
-            cand = torch.cat(gathered, 0)
-        if float(cand[:, 0].max()) <= 0:
-            return sums, counts
-        order = torch.argsort(cand[:, 0], descending=True, stable=True)[:ne]
-        for e, row in zip(empty.tolist(), order.tolist()):
-            old = int(cand[row, 1])
-            x = cand[row, 2:]
-            sums[old] -= x
-            sums[e] = x
-            counts[e] = 1
-            counts[old] -= 1
-        return sums, counts
-
-    def _relocate_empty_weighted(self, Xc, n, labels, centers, sums, wsums, w):
+    def _relocate_empty(self, Xc, n, labels, centers, sums, wsums, w):
+        """sklearn _k_means_common.pyx:167-211: every empty cluster (weight sum 0) is moved onto one of the points farthest,
+        by unweighted distance, from its own (old) centre, and that point is taken out of its old cluster: sums[old] -= w x,
+        sums[e] = w x (an fp32 product, as sklearn), wsums[e] = w, wsums[old] -= w.  w None: unit weights, for which these
+        are the counts' updates.  Rare path, plain device ops.  Sharded: each rank offers its n_empty farthest points
+        (distance, old label, weight, coordinates), the candidates are all-gathered and every rank applies the same global
+        choice to the (already all-reduced) sums / weight sums."""
         empty = (wsums == 0).nonzero().flatten()
         ne = int(empty.numel())
         D = Xc.shape[1]
@@ -428,7 +371,7 @@ class KMeans:
         cand = torch.full((ne, 3 + D), float("-inf"), dtype=torch.float64, device=Xc.device)
         cand[:m, 0] = vals.double()
         cand[:m, 1] = labels[idxs].double()
-        cand[:m, 2] = w[idxs].double()
+        cand[:m, 2] = w[idxs].double() if w is not None else 1.0
         cand[:m, 3:] = Xc[idxs].double()
         if self.shard:
             world = _dist().get_world_size(self.process_group)

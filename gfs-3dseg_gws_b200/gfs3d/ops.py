@@ -313,14 +313,17 @@ def softmax_pool(logits: torch.Tensor, feat: torch.Tensor) -> torch.Tensor:
 
 
 def kmeans_pp_trial(xt: torch.Tensor, n: int, xsq: torch.Tensor, cand: torch.Tensor, closest: Optional[torch.Tensor],
-                    m_out: torch.Tensor, pots: torch.Tensor):
-    """k-means++ step: xt (D, npad) channel-major, xsq (n) fp64, cand (T, D) -> m_out (T, npad) = min(d(x, cand_t), closest), pots (T) f64 (+)="""
-    _need_cuda(xt, xsq, cand, closest, m_out, pots)
+                    m_out: torch.Tensor, pots: torch.Tensor, weights: Optional[torch.Tensor] = None):
+    """k-means++ step: xt (D, npad) channel-major, xsq (n) fp64, cand (T, D) -> m_out (T, npad) = min(d(x, cand_t), closest),
+    pots (T) f64 (+)= sum_i weights[i] * m_out[t, i] (weights (n) fp32, None = 1)"""
+    _need_cuda(xt, xsq, cand, closest, m_out, pots, weights)
     D, npad = xt.shape
     T = cand.shape[0]
     assert xt.is_contiguous() and cand.is_contiguous() and cand.shape[1] == D and m_out.is_contiguous() and m_out.shape[1] == npad
     assert m_out.shape[0] >= T and pots.dtype == torch.float64 and pots.numel() >= T and xsq.numel() >= n and xsq.dtype == torch.float64
-    _call("gfs_kmeans_pp_trial", 1, _ptr(xt), npad, n, D, _ptr(xsq), _ptr(cand), T, _ptr(closest), _ptr(m_out), _ptr(pots), _stream())
+    assert weights is None or (weights.dtype == torch.float32 and weights.is_contiguous() and weights.numel() >= n)
+    _call("gfs_kmeans_pp_trial", 1, _ptr(xt), npad, n, D, _ptr(xsq), _ptr(cand), T, _ptr(closest), _ptr(weights), _ptr(m_out),
+          _ptr(pots), _stream())
 
 
 def kmeans_assign(xt: torch.Tensor, centers_t: torch.Tensor, K: int, want_score: bool = False, impl: Optional[str] = None):
@@ -358,10 +361,6 @@ def kmeans_assign_rows(X: torch.Tensor, centers_t: torch.Tensor, K: int) -> torc
     ws = torch.empty(nbytes, dtype=torch.uint8, device=X.device)
     _call("gfs_kmeans_assign_tc", 6, _ptr(X), n, D, 1, D, _ptr(centers_t), K, Kp, _ptr(cnorm), _ptr(labels), _ptr(ws), nbytes, _stream())
     return labels
-
-
-def kmeans_rows_eligible(D: int, Kp: int) -> bool:
-    return ROWSEL_IMPL != "fp32" and D % 64 == 0 and D <= 192 and Kp <= 192
 
 
 def kmeans_accumulate(X: torch.Tensor, labels: torch.Tensor, K: int, n_valid: Optional[int] = None, sums=None, counts=None, ws=None):
@@ -419,35 +418,6 @@ def kmeans_accumulate_weighted_workspace(K: int, D: int, device):
     return (torch.empty(P * K * D, dtype=torch.float32, device=device), torch.empty(P * K, dtype=torch.float64, device=device))
 
 
-def kmeans_pack_weighted(labels, labels_old, n, K, D, packed, scratch):
-    """packed[-1] = #(labels != labels_old) over the first n; packed[:K*D] (sums) and packed[K*D:K*D+K] (weight sums) are
-    filled already by kmeans_accumulate_weighted"""
-    _need_cuda(labels, labels_old, packed, scratch)
-    assert packed.dtype == torch.float64 and packed.numel() == K * D + K + 1 and scratch.numel() * scratch.element_size() >= 16
-    _call("gfs_kmeans_pack_weighted", 1, _ptr(labels), _ptr(labels_old), n, K, D, _ptr(packed), _ptr(scratch), _stream())
-
-
-def kmeans_update_weighted(packed, centers_old, K, D, Kp, centers_new, ct, result):
-    """kmeans_update dividing by the fp64 weight sums of the packed buffer as they are (no rounding to a count)"""
-    _need_cuda(packed, centers_old, centers_new, ct, result)
-    assert centers_old.is_contiguous() and centers_new.is_contiguous() and ct.is_contiguous() and result.dtype == torch.float64
-    _call("gfs_kmeans_update_weighted", 1, _ptr(packed), _ptr(centers_old), K, D, Kp, _ptr(centers_new), _ptr(ct), _ptr(result),
-          _stream())
-
-
-def kmeans_pp_trial_weighted(xt: torch.Tensor, n: int, xsq: torch.Tensor, cand: torch.Tensor, closest: Optional[torch.Tensor],
-                             weights: torch.Tensor, m_out: torch.Tensor, pots: torch.Tensor):
-    """kmeans_pp_trial with pots (T) f64 (+)= sum_i weights[i] * m_out[t, i]; m_out is the unweighted minimum"""
-    _need_cuda(xt, xsq, cand, closest, weights, m_out, pots)
-    D, npad = xt.shape
-    T = cand.shape[0]
-    assert xt.is_contiguous() and cand.is_contiguous() and cand.shape[1] == D and m_out.is_contiguous() and m_out.shape[1] == npad
-    assert m_out.shape[0] >= T and pots.dtype == torch.float64 and pots.numel() >= T and xsq.numel() >= n and xsq.dtype == torch.float64
-    assert weights.dtype == torch.float32 and weights.is_contiguous() and weights.numel() >= n
-    _call("gfs_kmeans_pp_trial_weighted", 1, _ptr(xt), npad, n, D, _ptr(xsq), _ptr(cand), T, _ptr(closest), _ptr(weights), _ptr(m_out),
-          _ptr(pots), _stream())
-
-
 def kmeans_inertia(X: torch.Tensor, labels: torch.Tensor, centers: torch.Tensor, weights: Optional[torch.Tensor] = None,
                    n_valid: Optional[int] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """X (n, D) fp32 row-major, labels (n) int32, centers (K, D) fp32, weights (n) fp32 or None -> (1,) fp64 on the device:
@@ -466,15 +436,17 @@ def kmeans_inertia(X: torch.Tensor, labels: torch.Tensor, centers: torch.Tensor,
     return out
 
 
-def kmeans_pack(labels, labels_old, n, counts, K, D, packed, scratch):
-    """packed[K*D:K*D+K] = counts, packed[-1] = #(labels != labels_old) over the first n; packed[:K*D] are the sums already"""
+def kmeans_pack(labels, labels_old, n, K, D, packed, scratch, counts=None):
+    """packed[-1] = #(labels != labels_old) over the first n; packed[:K*D] are the sums already.  packed[K*D:K*D+K] (the weight
+    sums) = counts (K) int64, or, with counts None, the fp64 weight sums kmeans_accumulate_weighted wrote there"""
     _need_cuda(labels, labels_old, counts, packed, scratch)
     assert packed.dtype == torch.float64 and packed.numel() == K * D + K + 1 and scratch.numel() * scratch.element_size() >= 16
     _call("gfs_kmeans_pack", 1, _ptr(labels), _ptr(labels_old), n, _ptr(counts), K, D, _ptr(packed), _ptr(scratch), _stream())
 
 
 def kmeans_update(packed, centers_old, K, D, Kp, centers_new, ct, result):
-    """new centres (K, D), their transpose ct (D, Kp) and result = [changed, shift, empty] from the (all-reduced) packed buffer"""
+    """new centres (K, D) = sums / weight sums, their transpose ct (D, Kp) and result = [changed, shift, empty] from the
+    (all-reduced) packed buffer"""
     _need_cuda(packed, centers_old, centers_new, ct, result)
     assert centers_old.is_contiguous() and centers_new.is_contiguous() and ct.is_contiguous() and result.dtype == torch.float64
     _call("gfs_kmeans_update", 1, _ptr(packed), _ptr(centers_old), K, D, Kp, _ptr(centers_new), _ptr(ct), _ptr(result), _stream())

@@ -226,28 +226,23 @@ int gfs_kmeans_accumulate(const float* X, int64_t n, int D, const int32_t* label
  * multiply-add) in the same ascending, pairwise order as gfs_kmeans_accumulate, so weights of 1 give its sums bit for bit;
  * wsums[l] += w in fp64, ascending point order per CTA.  weights (n) fp32; partial (P, K, D) fp32 and pweight (P, K) fp64
  * workspaces, P = gfs_kmeans_partials(); sums (K, D) and wsums (K) fp64 are reduced in CTA order.  wsums may be the weight
- * slot packed[K*D : K*D+K] of gfs_kmeans_pack_weighted's buffer.                                                      */
+ * slot packed[K*D : K*D+K] of gfs_kmeans_pack's buffer.                                                               */
 int gfs_kmeans_accumulate_weighted(const float* X, int64_t n, int D, const int32_t* labels, const float* weights, int K,
                                    float* partial, double* pweight, double* sums, double* wsums, void* stream);
 
 /* The rest of a Lloyd iteration (sklearn _k_means_common.pyx:_average_centers, _kmeans.py:_kmeans_single_lloyd) in two launches:
- *   gfs_kmeans_pack:   packed (K*D + K + 1 doubles) = [sums (already there: pass packed as gfs_kmeans_accumulate's sums) |
- *                      counts as fp64 | number of i < n with labels[i] != labels_old[i]] -- the ONE buffer the sharded k-means
- *                      all-reduces per iteration.  scratch16: 16 bytes, zero on first use (the kernel leaves them zero).
- *   gfs_kmeans_update: centers_new (K, D) = count > 0 ? sums / count : 0, centers_t (D, Kp) its transpose for the next E-step,
- *                      result3 = [labels changed, sum (new - old)^2 in fp64 (fixed order), empty clusters]                 */
+ *   gfs_kmeans_pack:   packed (K*D + K + 1 doubles) = [sums (already there: pass packed as the accumulate call's sums) |
+ *                      weight sums in fp64 | number of i < n with labels[i] != labels_old[i]] -- the ONE buffer the sharded
+ *                      k-means all-reduces per iteration.  counts (K) int64 from gfs_kmeans_accumulate are copied into the
+ *                      weight slot; counts = NULL: the slot holds the weight sums gfs_kmeans_accumulate_weighted wrote there.
+ *                      scratch16: 16 bytes, zero on first use (the kernel leaves them zero).
+ *   gfs_kmeans_update: centers_new (K, D) = wsum > 0 ? sums / wsum : 0, centers_t (D, Kp) its transpose for the next E-step,
+ *                      result3 = [labels changed, sum (new - old)^2 in fp64 (fixed order), empty clusters].  A cluster is
+ *                      empty when its weight sum is 0, so a cluster whose members all weigh 0 is empty, as in sklearn.     */
 int gfs_kmeans_pack(const int32_t* labels, const int32_t* labels_old, int64_t n, const int64_t* counts, int K, int D,
                     double* packed, void* scratch16, void* stream);
 int gfs_kmeans_update(const double* packed, const float* centers_old, int K, int D, int Kp, float* centers_new, float* centers_t,
                       double* result3, void* stream);
-/* Weighted forms: packed's middle slot holds the fp64 weight sums (written by gfs_kmeans_accumulate_weighted), so
- * gfs_kmeans_pack_weighted writes only the changed-label count into packed[K*D + K], and gfs_kmeans_update_weighted divides by
- * the weight sums as they are (gfs_kmeans_update rounds its slot to an integer count).  A cluster is empty when its weight
- * sum is 0, so a cluster whose members all weigh 0 is empty, as in sklearn.                                            */
-int gfs_kmeans_pack_weighted(const int32_t* labels, const int32_t* labels_old, int64_t n, int K, int D, double* packed,
-                             void* scratch16, void* stream);
-int gfs_kmeans_update_weighted(const double* packed, const float* centers_old, int K, int D, int Kp, float* centers_new,
-                               float* centers_t, double* result3, void* stream);
 
 /* inertia (sklearn _k_means_common.pyx:_inertia_dense): out[0] = sum_i w_i * |x_i - centers[labels[i]]|^2 (w_i = 1 when
  * weights is NULL).  The squared distance is sklearn's fp32 chain over groups of 4 features; the sum is fp64 in an order
@@ -258,16 +253,15 @@ int gfs_kmeans_inertia(const float* X, int64_t n, int D, const int32_t* labels, 
                        const float* weights, double* partial, double* out, void* stream);
 
 /* ---- k-means++ seeding step (sklearn _kmeans.py:_kmeans_plusplus behind get_basis.py:210, SURVEY 8f N3) ---------------
- * For T <= 8 candidate centres:  m[t][i] = min(max(float(|x_i|^2 - 2 x_i.c_t + |c_t|^2), 0), closest[i]),  pots[t] += sum_i m[t][i]
- * The distance is accumulated in fp64 and rounded once to fp32, as sklearn's _euclidean_distances_upcast does for float32 data.
+ * For T <= 8 candidate centres:  m[t][i] = min(max(float(|x_i|^2 - 2 x_i.c_t + |c_t|^2), 0), closest[i]),
+ *                                 pots[t] += sum_i w_i * m[t][i]   (sklearn's `distance_to_candidates @ sample_weight`)
+ * The distance is accumulated in fp64 and rounded once to fp32, as sklearn's _euclidean_distances_upcast does for float32 data;
+ * the potentials are fp64 (w_i * m is exact there).
  *   xt (D, npad) channel-major fp32 (the E-step's copy), xsq (n) fp64 squared norms, cand (T, D) row-major, closest (n) or NULL
- *   (= +inf: the first centre), m_out (T, npad) fp32, pots (T) fp64 ACCUMULATED into (the caller zeroes it)              */
+ *   (= +inf: the first centre), weights (n) fp32 or NULL (w_i = 1), m_out (T, npad) fp32 (unweighted), pots (T) fp64
+ *   ACCUMULATED into (the caller zeroes it)                                                                             */
 int gfs_kmeans_pp_trial(const float* xt, int64_t npad, int64_t n, int D, const double* xsq, const float* cand, int T,
-                        const float* closest, float* m_out, double* pots, void* stream);
-/* weighted k-means++ (sklearn's `distance_to_candidates @ sample_weight`): pots[t] += sum_i weights[i] * m[t][i] in fp64 (the
- * product of two fp32 values is exact); m_out is unchanged, closest stays unweighted.  weights (n) fp32.             */
-int gfs_kmeans_pp_trial_weighted(const float* xt, int64_t npad, int64_t n, int D, const double* xsq, const float* cand, int T,
-                                 const float* closest, const float* weights, float* m_out, double* pots, void* stream);
+                        const float* closest, const float* weights, float* m_out, double* pots, void* stream);
 
 /* =====================================================================================================================
  * TRAINING path (model.train(), train.py:614-631).  fp32 end to end, activations channel-major (C, M) with M = B*N points

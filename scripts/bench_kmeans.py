@@ -77,12 +77,10 @@ def bench_weighted():
         labels = ops.kmeans_assign(xt, ct, K)
         if weighted:
             ops.kmeans_accumulate_weighted(X, labels, w, K, sums=sums, wsums=packed[K * D:K * D + K], ws=ws_w)
-            ops.kmeans_pack_weighted(labels, labels_old, n, K, D, packed, scratch)
-            ops.kmeans_update_weighted(packed, cold, K, D, Kp, cnew, ct, result)
         else:
             ops.kmeans_accumulate(X, labels, K, sums=sums, counts=counts, ws=ws_u)
-            ops.kmeans_pack(labels, labels_old, n, counts, K, D, packed, scratch)
-            ops.kmeans_update(packed, cold, K, D, Kp, cnew, ct, result)
+        ops.kmeans_pack(labels, labels_old, n, K, D, packed, scratch, counts=None if weighted else counts)
+        ops.kmeans_update(packed, cold, K, D, Kp, cnew, ct, result)
         result.tolist()
         return labels
 

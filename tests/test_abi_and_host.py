@@ -167,19 +167,19 @@ def _worker(rank, world, port, out):
     bucket.zero()
     lin(xin).sum().backward()                      # second step: still accumulating into the same storage
     ok = ok and bucket.views_intact() and torch.allclose(bucket.flat[:12], torch.full((12,), 2.0 * (rank + 1)))
-    # sharded k-means++ seeding (host logic of gfs3d.kmeans.KMeans._seed_plusplus; the scoring kernel is replaced by a torch
-    # stand-in with the same contract): the picks of the 2-rank run must equal the single-process picks
+    # sharded k-means++ seeding, unweighted and weighted (host logic of gfs3d.kmeans.KMeans._seed_plusplus; the scoring kernel
+    # is replaced by a torch stand-in with the same contract): the picks of the 2-rank run must equal the single-process picks
     from gfs3d import kmeans as km_mod
     from gfs3d.kmeans import KMeans
 
-    def trial_stub(xt, n_, xsq, cand, closest, m_out, pots):
+    def trial_stub(xt, n_, xsq, cand, closest, m_out, pots, weights=None):
         X_ = xt[:, :n_].t().double()
         d = (xsq[:n_][None, :] - 2.0 * (cand.double() @ X_.t()) + (cand.double() ** 2).sum(1)[:, None]).float().clamp_min(0)
         if closest is not None:
             d = torch.minimum(d, closest[:n_][None, :])
         T = cand.shape[0]
         m_out[:T, :n_] = d
-        pots[:T] += d.double().sum(1)
+        pots[:T] += (d.double() * (1.0 if weights is None else weights[:n_].double())).sum(1)
 
     real = km_mod.ops.kmeans_pp_trial
     km_mod.ops.kmeans_pp_trial = trial_stub
@@ -188,22 +188,29 @@ def _worker(rank, world, port, out):
         Xs = torch.from_numpy(rs2.randn(403, 6).astype(np.float32))
         lo2, hi2 = shard_range(403, rank, world)
 
-        def seed(Xpart, shard):
+        def seed(Xpart, shard, w=None):
             k = KMeans(n_clusters=9, init="k-means++", shard=shard)
             npad = (Xpart.shape[0] + 3) // 4 * 4
             xt = torch.zeros(6, npad)
             xt[:, :Xpart.shape[0]] = Xpart.t()
-            return k._seed_plusplus(Xpart, xt, np.random.RandomState(17))
+            return k._seed_plusplus(Xpart, xt, np.random.RandomState(17), w=w)
         c_sharded = seed(Xs[lo2:hi2].contiguous(), True)
         c_single = seed(Xs, False)
         ok = ok and torch.equal(c_sharded, c_single)
+        # weighted: an even split (gloo's all-gather of the weights takes equal sizes only; NCCL takes uneven ones)
+        ws = torch.from_numpy(rs2.lognormal(0.0, 0.75, 402).astype(np.float32))
+        ws[::7] = 0.0
+        lo3, hi3 = shard_range(402, rank, world)
+        c_sharded = seed(Xs[lo3:hi3].contiguous(), True, ws[lo3:hi3].contiguous())
+        c_single = seed(Xs[:402], False, ws)
+        ok = ok and torch.equal(c_sharded, c_single) and not torch.equal(c_single, seed(Xs[:402], False))
     finally:
         km_mod.ops.kmeans_pp_trial = real
     out[rank] = bool(ok)
     dist.destroy_process_group()
 
 
-def test_sharded_centroid_allreduce_gloo_world2():
+def test_sharded_centroid_allreduce_and_seeding_gloo_world2():
     from gfs3d.dist import shard_range
     assert [shard_range(10, r, 4) for r in range(4)] == [(0, 3), (3, 6), (6, 8), (8, 10)]
     assert shard_range(3, 3, 4) == (3, 3)

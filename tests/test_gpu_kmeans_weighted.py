@@ -95,6 +95,24 @@ def test_weighted_relocation_vs_sklearn_fixture(golden):
     assert (km.labels_ == 7).any()
 
 
+def test_unweighted_relocation_equals_unit_weights_and_restatement(golden):
+    """the relocation fixture's problem fitted without weights (centre 7 is empty in the first iteration whatever the weights):
+    the same bits as sample_weight = 1, and the numpy restatement's result with unit weights"""
+    from gfs3d.kmeans import KMeans
+    g = golden("kmeans_weighted_relocate_n2000_k20")
+    X, _, _, _ = _problem(g)
+    from make_kmeans_weighted import lloyd_reference_weighted
+    ones = np.ones(X.shape[0], np.float32)
+    km = KMeans(n_clusters=int(g["K"]), init=g["init"], n_init=1).fit(X)
+    unit = KMeans(n_clusters=int(g["K"]), init=g["init"], n_init=1).fit(X, sample_weight=ones)
+    assert np.array_equal(km.labels_, unit.labels_) and np.array_equal(km.cluster_centers_, unit.cluster_centers_)
+    assert km.n_iter_ == unit.n_iter_ and km.inertia_ == unit.inertia_
+    labels, centers, n_iter = lloyd_reference_weighted(X, g["init"], ones)
+    inertia = ((X.astype(np.float64) - centers.astype(np.float64)[labels]) ** 2).sum()
+    _fit_checks(km, X, labels, centers, n_iter, inertia)
+    assert (km.labels_ == 7).any()
+
+
 def _init_problem(golden):
     g = golden("kmeans_weighted_init_n3000_k50")
     X, w, _, _ = _problem(g)
@@ -160,6 +178,30 @@ def test_unit_and_scaled_weights_are_bit_identical(scale):
     a = km._seed_plusplus(Xc, _xt(Xc), np.random.RandomState(9), w=None if scale == 1.0 else wd)
     b = km._seed_plusplus(Xc, _xt(Xc), np.random.RandomState(9), w=wd * scale)
     assert torch.equal(a, b)
+
+
+@pytest.mark.parametrize("n", [253, 5003])
+def test_pp_trial_null_weights_equal_unit_weights(n):
+    """gfs_kmeans_pp_trial with weights = NULL gives the distances of weights all 1 bit for bit, and their potentials: bit for
+    bit within one CTA (256 points); across CTAs the fp64 atomic adds of the CTA sums may land in any order"""
+    from gfs3d import ops
+    X, rs = _mixture(n, 192, 40, seed=41)
+    Xd = torch.from_numpy(X).cuda()
+    xt = _xt(Xd)
+    xsq = (Xd.double() ** 2).sum(1)
+    cand = Xd[torch.from_numpy(rs.choice(n, 8, replace=False)).cuda()].contiguous()
+    closest = torch.from_numpy((rs.rand(n) * 400).astype(np.float32)).cuda()
+    got = []
+    for w in (None, torch.ones(n, device="cuda")):
+        m = torch.empty(8, xt.shape[1], device="cuda")
+        pots = torch.zeros(8, dtype=torch.float64, device="cuda")
+        ops.kmeans_pp_trial(xt, n, xsq, cand, closest, m, pots, weights=w)
+        got.append((m[:, :n].clone(), pots))
+    assert torch.equal(got[0][0], got[1][0])
+    if n <= 256:
+        assert torch.equal(got[0][1], got[1][1])
+    else:
+        assert bool(((got[0][1] - got[1][1]).abs() <= 1e-12 * got[1][1]).all())
 
 
 def test_weighted_msteps_unit_weights_equal_unweighted_and_repeat():

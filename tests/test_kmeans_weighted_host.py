@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 
 
-def test_weighted_kmeans_entries_reject_bad_arguments_without_gpu():
+def test_kmeans_entries_with_weights_reject_bad_arguments_without_gpu():
     from gfs3d._lib import lib
     l = lib()
     buf = (ctypes.c_double * 64)()
@@ -16,14 +16,14 @@ def test_weighted_kmeans_entries_reject_bad_arguments_without_gpu():
     assert l.gfs_kmeans_accumulate_weighted(p, 10, 260, p, p, 3, p, p, p, p, None) == 2 and b"D=260" in err()
     assert l.gfs_kmeans_accumulate_weighted(p, 10, 256, p, p, 192, p, p, p, p, None) == 2 and b"shared memory" in err()
     assert l.gfs_kmeans_accumulate_weighted(p, 0, 8, p, p, 3, p, p, p, p, None) == 1 and b"non-positive" in err()
-    assert l.gfs_kmeans_pack_weighted(p, None, 10, 3, 8, p, p, None) == 1 and b"null pointer" in err()
-    assert l.gfs_kmeans_pack_weighted(p, p, 0, 3, 8, p, p, None) == 1 and b"non-positive" in err()
-    assert l.gfs_kmeans_update_weighted(p, p, 3, 8, 4, p, None, p, None) == 1 and b"null pointer" in err()
-    assert l.gfs_kmeans_update_weighted(p, p, 5, 8, 4, p, p, p, None) == 1 and b"bad size" in err()
-    assert l.gfs_kmeans_pp_trial_weighted(p, 12, 10, 8, p, p, 2, None, None, p, p, None) == 1 and b"null pointer" in err()
-    assert l.gfs_kmeans_pp_trial_weighted(p, 12, 10, 8, p, p, 9, None, p, p, p, None) == 2 and b"T=9" in err()
-    assert l.gfs_kmeans_pp_trial_weighted(p, 12, 10, 520, p, p, 2, None, p, p, p, None) == 2 and b"D=520" in err()
-    assert l.gfs_kmeans_pp_trial_weighted(p, 8, 10, 8, p, p, 2, None, p, p, p, None) == 1 and b"non-positive" in err()
+    assert l.gfs_kmeans_pack(p, None, 10, None, 3, 8, p, p, None) == 1 and b"null pointer" in err()
+    assert l.gfs_kmeans_pack(p, p, 0, None, 3, 8, p, p, None) == 1 and b"non-positive" in err()
+    assert l.gfs_kmeans_update(p, p, 3, 8, 4, p, None, p, None) == 1 and b"null pointer" in err()
+    assert l.gfs_kmeans_update(p, p, 5, 8, 4, p, p, p, None) == 1 and b"bad size" in err()
+    assert l.gfs_kmeans_pp_trial(p, 12, 10, 8, p, p, 2, None, p, None, p, None) == 1 and b"null pointer" in err()
+    assert l.gfs_kmeans_pp_trial(p, 12, 10, 8, p, p, 9, None, p, p, p, None) == 2 and b"T=9" in err()
+    assert l.gfs_kmeans_pp_trial(p, 12, 10, 520, p, p, 2, None, p, p, p, None) == 2 and b"D=520" in err()
+    assert l.gfs_kmeans_pp_trial(p, 8, 10, 8, p, p, 2, None, p, p, p, None) == 1 and b"non-positive" in err()
     assert l.gfs_kmeans_inertia(p, 10, 8, p, None, 3, None, p, p, None) == 1 and b"null pointer" in err()
     assert l.gfs_kmeans_inertia(p, 10, 10, p, p, 3, None, p, p, None) == 2 and b"D=10" in err()
     assert l.gfs_kmeans_inertia(p, 10, 512, p, p, 3, None, p, p, None) == 2 and b"D=512" in err()
