@@ -19,27 +19,34 @@ constexpr int KM_THREADS = 288;    // warps 0-7: one thread per feature column; 
 // weights next to its labels, the column threads add __fmul_rn(x, w) with __fadd_rn (a product, then an add: no fused
 // multiply-add, as sklearn's C), and the helper warp's lane 0 adds the weights into a per-CTA fp64 table in ascending
 // point order instead of counting.  The unweighted instance is the kernel as it was.
-template <bool WEIGHTED>
-__global__ void __launch_bounds__(KM_THREADS, 1)
-kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32_t* __restrict__ labels,
-                      const float* __restrict__ weights, int K, float* __restrict__ partial, int32_t* __restrict__ pcount,
-                      double* __restrict__ pweight) {
+//
+// SPLIT (kmeans_partial_split_kernel, for K x D tables beyond shared memory): the CTAs form groups of `slices`; a group owns
+// one contiguous point range, every CTA of it streams the whole range and keeps the table of its own contiguous slice of
+// `kslice` centres, adding only the points labelled in that slice.  Each (centre, column) sum is then the same ascending-
+// order fp32 sum the undivided table would hold.  The helper warp stages an out-of-slice label as -1.
+template <bool WEIGHTED, bool SPLIT>
+__device__ __forceinline__ void kmeans_partial_body(const float* __restrict__ X, int64_t n, int D, const int32_t* __restrict__ labels,
+                                                    const float* __restrict__ weights, int K, int slices, int kslice,
+                                                    float* __restrict__ partial, int32_t* __restrict__ pcount, double* __restrict__ pweight) {
     extern __shared__ __align__(128) unsigned char sm_raw[];
+    const int range = SPLIT ? blockIdx.x / slices : blockIdx.x, nranges = SPLIT ? gridDim.x / slices : gridDim.x;
+    const int c0 = SPLIT ? (blockIdx.x - range * slices) * kslice : 0;
+    const int kc = SPLIT ? (K - c0 < kslice ? K - c0 : kslice) : K;     // centres of this CTA's table
     float* stg = reinterpret_cast<float*>(sm_raw);                          // [2][KM_CH][D]   (first: keeps 128 B alignment)
-    float* tab = stg + 2 * KM_CH * D;                                       // [K][D]
-    int* cnt = reinterpret_cast<int*>(tab + (size_t)K * D);                 // [K]            (unweighted)
-    double* wtab = reinterpret_cast<double*>(tab + (size_t)K * D);          // [K] fp64       (weighted)
-    int* lab = WEIGHTED ? reinterpret_cast<int*>(wtab + K) : cnt + ((K + 3) & ~3);   // [2][KM_CH]
+    float* tab = stg + 2 * KM_CH * D;                                       // [kc][D]
+    int* cnt = reinterpret_cast<int*>(tab + (size_t)kc * D);                // [kc]           (unweighted)
+    double* wtab = reinterpret_cast<double*>(tab + (size_t)kc * D);         // [kc] fp64      (weighted)
+    int* lab = WEIGHTED ? reinterpret_cast<int*>(wtab + kc) : cnt + ((kc + 3) & ~3);   // [2][KM_CH]
     float* wst = reinterpret_cast<float*>(lab + 2 * KM_CH);                 // [2][KM_CH]     (weighted)
     uint64_t* full = reinterpret_cast<uint64_t*>(WEIGHTED ? reinterpret_cast<int*>(wst + 2 * KM_CH) : lab + 2 * KM_CH);  // [2]
     const int tid = threadIdx.x, lane = tid & 31;
     const bool helper = tid >= 256;
 
-    for (int i = tid; i < K * D; i += KM_THREADS) tab[i] = 0.0f;
+    for (int i = tid; i < kc * D; i += KM_THREADS) tab[i] = 0.0f;
     if constexpr (WEIGHTED) {
-        for (int i = tid; i < K; i += KM_THREADS) wtab[i] = 0.0;
+        for (int i = tid; i < kc; i += KM_THREADS) wtab[i] = 0.0;
     } else {
-        for (int i = tid; i < K; i += KM_THREADS) cnt[i] = 0;
+        for (int i = tid; i < kc; i += KM_THREADS) cnt[i] = 0;
     }
     if (tid == 0) {
         mbar_init(&full[0], 1);
@@ -48,9 +55,9 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
     }
     __syncthreads();
 
-    int64_t per = (n + gridDim.x - 1) / gridDim.x;
+    int64_t per = (n + nranges - 1) / nranges;
     per = (per + KM_CH - 1) / KM_CH * KM_CH;
-    const int64_t i0 = per * blockIdx.x;
+    const int64_t i0 = per * range;
     const int64_t i1 = (i0 + per) < n ? (i0 + per) : n;
     const int nchunks = i0 < i1 ? (int)((i1 - i0 + KM_CH - 1) / KM_CH) : 0;
 
@@ -58,7 +65,12 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
         if (c < nchunks) {
             const int64_t p0 = i0 + (int64_t)c * KM_CH;
             const int cc = (int)((i1 - p0) < KM_CH ? (i1 - p0) : KM_CH);
-            lab[(c & 1) * KM_CH + lane] = lane < cc ? labels[p0 + lane] : 0;
+            if constexpr (SPLIT) {
+                const int l = lane < cc ? labels[p0 + lane] - c0 : -1;
+                lab[(c & 1) * KM_CH + lane] = l < kc ? l : -1;
+            } else {
+                lab[(c & 1) * KM_CH + lane] = lane < cc ? labels[p0 + lane] : 0;
+            }
             if constexpr (WEIGHTED) wst[(c & 1) * KM_CH + lane] = lane < cc ? weights[p0 + lane] : 0.0f;
             if (lane == 0) {
                 const uint32_t bytes = (uint32_t)cc * (uint32_t)D * 4u;
@@ -88,7 +100,10 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
                     for (; j + 1 < cc; j += 2) {  // the same pairwise order as the unweighted instance
                         const int l0 = L[j], l1 = L[j + 1];
                         const float v0 = __fmul_rn(S[j * D], W[j]), v1 = __fmul_rn(S[(j + 1) * D], W[j + 1]);
-                        if (l0 != l1) {
+                        if (SPLIT && (l0 < 0 || l1 < 0)) {
+                            if (l0 >= 0) tab[l0 * D + d] = __fadd_rn(tab[l0 * D + d], v0);
+                            if (l1 >= 0) tab[l1 * D + d] = __fadd_rn(tab[l1 * D + d], v1);
+                        } else if (l0 != l1) {
                             const float a = tab[l0 * D + d], b = tab[l1 * D + d];
                             tab[l0 * D + d] = __fadd_rn(a, v0);
                             tab[l1 * D + d] = __fadd_rn(b, v1);
@@ -96,13 +111,16 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
                             tab[l0 * D + d] = __fadd_rn(__fadd_rn(tab[l0 * D + d], v0), v1);
                         }
                     }
-                    if (j < cc) tab[L[j] * D + d] = __fadd_rn(tab[L[j] * D + d], __fmul_rn(S[j * D], W[j]));
+                    if (j < cc && (!SPLIT || L[j] >= 0)) tab[L[j] * D + d] = __fadd_rn(tab[L[j] * D + d], __fmul_rn(S[j * D], W[j]));
                 } else {
                     int j = 0;
                     for (; j + 1 < cc; j += 2) {      // ascending point order; two independent read-modify-writes when labels differ
                         const int l0 = L[j], l1 = L[j + 1];
                         const float v0 = S[j * D], v1 = S[(j + 1) * D];
-                        if (l0 != l1) {
+                        if (SPLIT && (l0 < 0 || l1 < 0)) {
+                            if (l0 >= 0) tab[l0 * D + d] += v0;
+                            if (l1 >= 0) tab[l1 * D + d] += v1;
+                        } else if (l0 != l1) {
                             const float a = tab[l0 * D + d], b = tab[l1 * D + d];
                             tab[l0 * D + d] = a + v0;
                             tab[l1 * D + d] = b + v1;
@@ -110,28 +128,62 @@ kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32
                             tab[l0 * D + d] = (tab[l0 * D + d] + v0) + v1;
                         }
                     }
-                    if (j < cc) tab[L[j] * D + d] += S[j * D];
+                    if (j < cc && (!SPLIT || L[j] >= 0)) tab[L[j] * D + d] += S[j * D];
                 }
             }
         } else if constexpr (WEIGHTED) {
             if (lane == 0) {                      // fp64, ascending point order: no floating-point atomics
                 const float* W = wst + (c & 1) * KM_CH;
-                for (int j = 0; j < cc; ++j) wtab[L[j]] += (double)W[j];
+                for (int j = 0; j < cc; ++j)
+                    if (!SPLIT || L[j] >= 0) wtab[L[j]] += (double)W[j];
             }
-        } else if (lane < cc) {
+        } else if (lane < cc && (!SPLIT || L[lane] >= 0)) {
             atomicAdd(&cnt[L[lane]], 1);
         }
         __syncthreads();                          // chunk buffer and its labels are free again
         if (helper) issue(c + 2);
     }
     __syncthreads();
-    float* o = partial + (size_t)blockIdx.x * K * D;
-    for (int i = tid; i < K * D; i += KM_THREADS) o[i] = tab[i];
+    float* o = partial + ((size_t)range * K + c0) * D;
+    for (int i = tid; i < kc * D; i += KM_THREADS) o[i] = tab[i];
     if constexpr (WEIGHTED) {
-        for (int i = tid; i < K; i += KM_THREADS) pweight[(size_t)blockIdx.x * K + i] = wtab[i];
+        for (int i = tid; i < kc; i += KM_THREADS) pweight[(size_t)range * K + c0 + i] = wtab[i];
     } else {
-        for (int i = tid; i < K; i += KM_THREADS) pcount[(size_t)blockIdx.x * K + i] = cnt[i];
+        for (int i = tid; i < kc; i += KM_THREADS) pcount[(size_t)range * K + c0 + i] = cnt[i];
     }
+}
+
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(KM_THREADS, 1)
+kmeans_partial_kernel(const float* __restrict__ X, int64_t n, int D, const int32_t* __restrict__ labels,
+                      const float* __restrict__ weights, int K, float* __restrict__ partial, int32_t* __restrict__ pcount,
+                      double* __restrict__ pweight) {
+    kmeans_partial_body<WEIGHTED, false>(X, n, D, labels, weights, K, 1, K, partial, pcount, pweight);
+}
+
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(KM_THREADS, 1)
+kmeans_partial_split_kernel(const float* __restrict__ X, int64_t n, int D, const int32_t* __restrict__ labels,
+                            const float* __restrict__ weights, int K, int slices, int kslice, float* __restrict__ partial,
+                            int32_t* __restrict__ pcount, double* __restrict__ pweight) {
+    kmeans_partial_body<WEIGHTED, true>(X, n, D, labels, weights, K, slices, kslice, partial, pcount, pweight);
+}
+
+// shared memory of a table of kc centres, its counts or fp64 weight sums and the staging
+static size_t km_smem(int kc, int D, bool weighted) {
+    return weighted ? (size_t)(2 * KM_CH + kc) * D * sizeof(float) + (size_t)kc * sizeof(double) + 2 * KM_CH * (sizeof(int) + sizeof(float)) + 64
+                    : (size_t)(2 * KM_CH + kc) * D * sizeof(float) + (size_t)((kc + 3) & ~3) * sizeof(int) + 2 * KM_CH * sizeof(int) + 64;
+}
+constexpr size_t KM_SMEM = 220 * 1024;
+
+// centre slices per point range: 1 while the whole table fits (the single-table kernel), else the fewest that fit; the split
+// is built for the k-means shapes beyond 192 centres, K <= 512 with D <= 192 (0: not built)
+static int km_slices(int K, int D, bool weighted) {
+    if (km_smem(K, D, weighted) <= KM_SMEM) return 1;
+    if (K > 512 || D > 192) return 0;
+    for (int g = 2; g <= K; ++g)
+        if (km_smem((K + g - 1) / g, D, weighted) <= KM_SMEM) return g;
+    return 0;
 }
 
 // CTA-order reduction of the per-CTA tables: sums in fp64; int32 counts into int64, or fp64 weight sums into fp64
@@ -155,6 +207,40 @@ __global__ void kmeans_reduce_kernel(const float* __restrict__ partial, const Pa
 
 extern "C" int gfs_kmeans_partials(void) { return gfs::sm_count(); }
 
+extern "C" int gfs_kmeans_accumulate_ranges(int K, int D, int weighted) {
+    const int g = gfs::km_slices(K, D, weighted != 0);
+    return g > 0 ? gfs::sm_count() / g : 0;
+}
+
+namespace gfs {
+// One resident CTA per SM: the single-table kernel over sm_count() point ranges when the K x D table fits, else
+// kmeans_partial_split_kernel with `slices` CTAs per range (sm_count() / slices ranges); then the range-order fp64 reduction.
+template <bool WEIGHTED, typename PartialCount, typename Count>
+static int km_accumulate(const char* who, const float* X, int64_t n, int D, const int32_t* labels, const float* weights, int K,
+                         float* partial, int32_t* pcount, double* pweight, PartialCount* preduce, double* sums, Count* counts,
+                         cudaStream_t st) {
+    const int slices = km_slices(K, D, WEIGHTED);
+    GFS_REQUIRE(slices > 0, GFS_ERR_UNSUPPORTED, "%s: K*D=%d does not fit shared memory", who, K * D);
+    const int sms = sm_count();
+    GFS_REQUIRE(sms > 0, GFS_ERR_CUDA, "%s: cannot query the device", who);
+    const int P = sms / slices;
+    GFS_REQUIRE(P > 0, GFS_ERR_UNSUPPORTED, "%s: K=%d needs %d CTAs per point range, the device has %d SMs", who, K, slices, sms);
+    if (slices == 1) {
+        GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_kernel<WEIGHTED>), KM_SMEM));
+        kmeans_partial_kernel<WEIGHTED><<<P, KM_THREADS, km_smem(K, D, WEIGHTED), st>>>(X, n, D, labels, weights, K, partial, pcount, pweight);
+    } else {
+        const int kslice = (K + slices - 1) / slices;
+        GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_split_kernel<WEIGHTED>), KM_SMEM));
+        kmeans_partial_split_kernel<WEIGHTED><<<P * slices, KM_THREADS, km_smem(kslice, D, WEIGHTED), st>>>(
+            X, n, D, labels, weights, K, slices, kslice, partial, pcount, pweight);
+    }
+    GFS_LAUNCH_OK("kmeans_partial_kernel");
+    kmeans_reduce_kernel<PartialCount, Count><<<(K * D + 255) / 256, 256, 0, st>>>(partial, preduce, P, K * D, K, sums, counts);
+    GFS_LAUNCH_OK("kmeans_reduce_kernel");
+    return GFS_OK;
+}
+}  // namespace gfs
+
 extern "C" int gfs_kmeans_accumulate(const float* X, int64_t n, int D, const int32_t* labels, int K, float* partial,
                                      int32_t* pcount, double* sums, int64_t* counts, void* stream) {
     using namespace gfs;
@@ -162,17 +248,8 @@ extern "C" int gfs_kmeans_accumulate(const float* X, int64_t n, int D, const int
     GFS_REQUIRE(n > 0 && D > 0 && K > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_accumulate: non-positive size");
     GFS_REQUIRE(D <= 256 && D % 4 == 0, GFS_ERR_UNSUPPORTED, "gfs_kmeans_accumulate: D=%d must be a multiple of 4, <= 256", D);
     GFS_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15) == 0, GFS_ERR_BAD_ARG, "gfs_kmeans_accumulate: X must be 16-byte aligned");
-    const size_t smem = (size_t)(2 * KM_CH + K) * D * sizeof(float) + (size_t)((K + 3) & ~3) * sizeof(int) + 2 * KM_CH * sizeof(int) + 64;
-    GFS_REQUIRE(smem <= 220 * 1024, GFS_ERR_UNSUPPORTED, "gfs_kmeans_accumulate: K*D=%d does not fit shared memory", K * D);
-    const int P = sm_count();
-    GFS_REQUIRE(P > 0, GFS_ERR_CUDA, "gfs_kmeans_accumulate: cannot query the device");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_kernel<false>), 220 * 1024));
-    kmeans_partial_kernel<false><<<P, KM_THREADS, smem, st>>>(X, n, D, labels, nullptr, K, partial, pcount, nullptr);
-    GFS_LAUNCH_OK("kmeans_partial_kernel");
-    kmeans_reduce_kernel<int32_t, int64_t><<<(K * D + 255) / 256, 256, 0, st>>>(partial, pcount, P, K * D, K, sums, counts);
-    GFS_LAUNCH_OK("kmeans_reduce_kernel");
-    return GFS_OK;
+    return km_accumulate<false>("gfs_kmeans_accumulate", X, n, D, labels, nullptr, K, partial, pcount, nullptr, pcount, sums, counts,
+                                static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int gfs_kmeans_accumulate_weighted(const float* X, int64_t n, int D, const int32_t* labels, const float* weights, int K,
@@ -183,17 +260,8 @@ extern "C" int gfs_kmeans_accumulate_weighted(const float* X, int64_t n, int D, 
     GFS_REQUIRE(n > 0 && D > 0 && K > 0, GFS_ERR_BAD_ARG, "gfs_kmeans_accumulate_weighted: non-positive size");
     GFS_REQUIRE(D <= 256 && D % 4 == 0, GFS_ERR_UNSUPPORTED, "gfs_kmeans_accumulate_weighted: D=%d must be a multiple of 4, <= 256", D);
     GFS_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15) == 0, GFS_ERR_BAD_ARG, "gfs_kmeans_accumulate_weighted: X must be 16-byte aligned");
-    const size_t smem = (size_t)(2 * KM_CH + K) * D * sizeof(float) + (size_t)K * sizeof(double) + 2 * KM_CH * (sizeof(int) + sizeof(float)) + 64;
-    GFS_REQUIRE(smem <= 220 * 1024, GFS_ERR_UNSUPPORTED, "gfs_kmeans_accumulate_weighted: K*D=%d does not fit shared memory", K * D);
-    const int P = sm_count();
-    GFS_REQUIRE(P > 0, GFS_ERR_CUDA, "gfs_kmeans_accumulate_weighted: cannot query the device");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(kmeans_partial_kernel<true>), 220 * 1024));
-    kmeans_partial_kernel<true><<<P, KM_THREADS, smem, st>>>(X, n, D, labels, weights, K, partial, nullptr, pweight);
-    GFS_LAUNCH_OK("kmeans_partial_kernel<weighted>");
-    kmeans_reduce_kernel<double, double><<<(K * D + 255) / 256, 256, 0, st>>>(partial, pweight, P, K * D, K, sums, wsums);
-    GFS_LAUNCH_OK("kmeans_reduce_kernel<weighted>");
-    return GFS_OK;
+    return km_accumulate<true>("gfs_kmeans_accumulate_weighted", X, n, D, labels, weights, K, partial, nullptr, pweight, pweight, sums,
+                               wsums, static_cast<cudaStream_t>(stream));
 }
 
 namespace gfs {

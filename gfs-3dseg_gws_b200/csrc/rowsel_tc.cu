@@ -45,6 +45,11 @@ struct RtSmem {                   // 1024-byte aligned; every operand tile start
 static_assert(offsetof(RtSmem, B) % 1024 == 0, "dictionary tiles must be 1024-byte aligned");
 
 enum { RT_GW = 0, RT_KMEANS = 1, RT_KMEANS_PM = 2 };   // _PM: points are rows of a row-major (n, D) matrix (contiguous 128-point tiles)
+// RT_PANEL (or-ed into a layout): one panel of <= 192 words of a dictionary of up to 512 (see rt_run_wide).  The panel
+// instances reuse three arguments the single-panel ones leave unused in their layout: kb0 = the panel's first word,
+// cos_cm = the per-row scratch the panels share, kblocks != 0 on the last panel (k-means).
+constexpr int RT_PANEL = 4;
+constexpr int RT_MAXK = 512;      // widest dictionary: ceil(512 / 192) = 3 panels
 
 // dict_t (D, Gp) fp32 channel-major -> per 64-channel block: [hi tile | lo tile], 192 rows x 128 B, K-major SWIZZLE_128B.
 // Also the largest squared norm of an entry (k-means: scales the ambiguity bound).
@@ -130,6 +135,8 @@ rowsel_tc_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstride, 
                  const uint8_t* __restrict__ img, int G, int Gp, const float* __restrict__ cnorm, const float* __restrict__ cmax2,
                  uint8_t* __restrict__ cos_act, int kblocks, int kb0, float* __restrict__ cos_cm, int32_t* __restrict__ sel,
                  int32_t* __restrict__ recheck, int32_t* __restrict__ recheck_cnt) {
+    constexpr int L = MODE & 3;
+    constexpr bool PANEL = (MODE & RT_PANEL) != 0;
     pdl_enter();
     extern __shared__ unsigned char smem_raw[];
     RtSmem& sm = *reinterpret_cast<RtSmem*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
@@ -172,7 +179,7 @@ rowsel_tc_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstride, 
             const int64_t m = ((int64_t)blockIdx.x + (int64_t)lt_ * gridDim.x) * RT_ROWS + r;
             const bool valid = it < S && m < M;
             const int64_t mm = valid ? m : 0;
-            if (MODE == RT_KMEANS_PM) {
+            if (L == RT_KMEANS_PM) {
                 // point-major: the thread's 16 channels are 64 contiguous bytes of its own row
                 const float4* xp4 = reinterpret_cast<const float4*>(x + mm * D + kb_ * 64 + qt * 16);
 #pragma unroll
@@ -186,7 +193,7 @@ rowsel_tc_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstride, 
                 return;
             }
             const float* xp;
-            if (MODE == RT_GW) {
+            if (L == RT_GW) {
                 const int64_t b = mm / N;
                 xp = x + b * bstride + (mm - b * N);
             } else {
@@ -280,7 +287,7 @@ rowsel_tc_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstride, 
         const int quarter = warp & 3;
         const int row = quarter * 32 + lane;
         const uint32_t tbase = tmem + ((uint32_t)(quarter * 32) << 16);
-        const float cmax = MODE != RT_GW ? sqrtf(__ldg(cmax2)) : 0.0f;
+        const float cmax = L != RT_GW ? sqrtf(__ldg(cmax2)) : 0.0f;
         int lt = 0;
         for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++lt) {
             const int acc = lt & 1;
@@ -293,7 +300,27 @@ rowsel_tc_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstride, 
             uint32_t rr[32];
             float b1, b2;
             int i1 = 0;
-            if (MODE == RT_GW) {
+            if constexpr (PANEL && L == RT_GW) {
+                // this panel's 10 cos into the column-major scratch [|x|^2 | word 0 | word 1 | ...] (rows of M): the softmax
+                // needs every word of the row, rowsel_gw_finish_kernel takes it from there
+                const float inv = 10.0f / fmaxf(sqrtf(nrm), 1e-12f);
+                float* out = cos_cm + (int64_t)(1 + kb0) * M + m;
+                if (valid && kb0 == 0) cos_cm[m] = nrm;
+                for (int ch = 0; ch * 32 < G; ++ch) {
+                    tmem_ld32(t0 + ch * 32, rr);
+                    tmem_ld_wait32(rr);
+                    if (valid) {
+#pragma unroll
+                        for (int c = 0; c < 32; ++c)
+                            if (ch * 32 + c < G) out[(int64_t)(ch * 32 + c) * M] = __uint_as_float(rr[c]) * inv;
+                    }
+                }
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&s.acce[acc]);
+                continue;
+            }
+            if (L == RT_GW) {
                 const float inv = 10.0f / fmaxf(sqrtf(nrm), 1e-12f);
                 b1 = -INFINITY;
                 b2 = -INFINITY;
@@ -392,11 +419,31 @@ rowsel_tc_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstride, 
             __syncwarp();
             if (lane == 0) mbar_arrive(&s.acce[acc]);
             if (valid) {
+                if constexpr (PANEL) {
+                    // (best, second best, index) of the panels so far, merged in ascending panel order: the earlier panels
+                    // hold the lower indices, so an equal score keeps theirs
+                    float* rs = cos_cm + 4 * m;
+                    i1 += kb0;
+                    if (kb0 > 0) {
+                        const float pb1 = rs[0];
+                        if (b1 < pb1) {
+                            b2 = fminf(b2, pb1);
+                        } else {
+                            b2 = fminf(rs[1], b1);
+                            b1 = pb1;
+                            i1 = __float_as_int(rs[2]);
+                        }
+                    }
+                    if (!kblocks) {
+                        *reinterpret_cast<float4*>(rs) = make_float4(b1, b2, __int_as_float(i1), 0.0f);
+                        continue;
+                    }
+                }
                 sel[m] = i1;
                 // the two best scores closer than the error bound of the tensor-core product (x 3 safety, see the header):
                 // the pinned fp32 chain decides (rowsel_recheck_kernel)
                 bool amb;
-                if (MODE == RT_GW) amb = !(b1 - b2 > 5e-3f) || !(nrm > 1e-20f);
+                if (L == RT_GW) amb = !(b1 - b2 > 5e-3f) || !(nrm > 1e-20f);
                 else amb = !(b2 - b1 > 0x1p-10f * sqrtf(nrm) * cmax);
                 if (amb) recheck[atomicAdd(recheck_cnt, 1)] = (int32_t)m;
             }
@@ -418,84 +465,97 @@ rowsel_tc_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstride, 
 // (Measured alternatives, r2: four rows per warp to reuse the dictionary values divides the L2 traffic by four but leaves
 // only ~250 warps on the GPU for ~1000 ambiguous rows: slower.  The re-check is latency bound, not traffic bound.)
 constexpr int RC_WARPS = 8;
+// RT_PANEL instance (dictionaries of 193..512 words): the row is staged once, then the 192-column groups run one after
+// the other with the same chains and the same per-lane pick; a later group replaces the running best only with a strictly
+// better score, so ties still go to the lowest index over all words.
 template <int MODE>
 __global__ void __launch_bounds__(32 * RC_WARPS)
 rowsel_recheck_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstride, int D, int N, const float* __restrict__ dict_t,
                       int G, int Gp, const float* __restrict__ cnorm, const int32_t* __restrict__ recheck,
                       const int32_t* __restrict__ recheck_cnt, int32_t* __restrict__ sel) {
+    constexpr int L = MODE & 3;
+    constexpr bool PANEL = (MODE & RT_PANEL) != 0;
     pdl_enter();
     __shared__ float xs_all[RC_WARPS][256];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     float* xs = xs_all[wib];
     const int nrows = *recheck_cnt;
     const int nb = (D + 7) >> 3;
+    int g0 = 0;                                      // first column of the current group (always 0 without RT_PANEL)
     auto load = [&](float (&g)[8][6], int bk) {
 #pragma unroll
         for (int c2 = 0; c2 < 8; ++c2) {
             const int c = bk * 8 + c2;
-            const float* gp = dict_t + (int64_t)c * Gp;
+            const float* gp = dict_t + (int64_t)c * Gp + g0;
 #pragma unroll
-            for (int j = 0; j < 6; ++j) g[c2][j] = (j * 32 + lane < G && c < D) ? __ldg(gp + j * 32 + lane) : 0.0f;
+            for (int j = 0; j < 6; ++j) g[c2][j] = (g0 + j * 32 + lane < G && c < D) ? __ldg(gp + j * 32 + lane) : 0.0f;
         }
     };
     for (int w = blockIdx.x * RC_WARPS + wib; w < nrows; w += gridDim.x * RC_WARPS) {
         const int64_t m = recheck[w];
         const float* xp;
-        if (MODE == RT_GW) {
+        if (L == RT_GW) {
             const int64_t b = m / N;
             xp = x + b * bstride + (m - b * N);
-        } else if (MODE == RT_KMEANS_PM) {
+        } else if (L == RT_KMEANS_PM) {
             xp = x + m * D;                          // cstride == 1
         } else {
             xp = x + m;
         }
         float ga[8][6], gb[8][6];
+        g0 = 0;
         load(ga, 0);
         __syncwarp();
         for (int c = lane; c < D; c += 32) xs[c] = __ldg(xp + (int64_t)c * cstride);
         __syncwarp();
-        float acc[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        float nrm = 0.0f;
-        auto compute = [&](const float (&g)[8][6], int bk) {
-#pragma unroll
-            for (int c2 = 0; c2 < 8; ++c2) {
-                const int c = bk * 8 + c2;
-                if (c < D) {                         // uniform
-                    const float a = xs[c];
-                    nrm = fmaf(a, a, nrm);
-#pragma unroll
-                    for (int j = 0; j < 6; ++j)
-                        if (j * 32 + lane < G) acc[j] = fmaf(a, g[c2][j], acc[j]);
-                }
-            }
-        };
-#pragma unroll 1
-        for (int bk = 0; bk < nb; bk += 2) {
-            if (bk + 1 < nb) load(gb, bk + 1);
-            compute(ga, bk);
-            if (bk + 2 < nb) load(ga, bk + 2);
-            if (bk + 1 < nb) compute(gb, bk + 1);
-        }
-        float best = MODE == RT_GW ? -INFINITY : INFINITY;
+        float best = L == RT_GW ? -INFINITY : INFINITY;
         int bi = 0x7fffffff;
-        const float inv = 10.0f / fmaxf(sqrtf(nrm), 1e-12f);
+        for (;;) {
+            float acc[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+            float nrm = 0.0f;
+            auto compute = [&](const float (&g)[8][6], int bk) {
 #pragma unroll
-        for (int j = 0; j < 6; ++j) {
-            const int col = j * 32 + lane;
-            if (col < G) {
-                const float sc = MODE == RT_GW ? acc[j] * inv : fmaf(-2.0f, acc[j], __ldg(cnorm + col));
-                const bool better = MODE == RT_GW ? (sc > best || (sc == best && col < bi)) : (sc < best || (sc == best && col < bi));
-                if (better) {
-                    best = sc;
-                    bi = col;
+                for (int c2 = 0; c2 < 8; ++c2) {
+                    const int c = bk * 8 + c2;
+                    if (c < D) {                         // uniform
+                        const float a = xs[c];
+                        nrm = fmaf(a, a, nrm);
+#pragma unroll
+                        for (int j = 0; j < 6; ++j)
+                            if (g0 + j * 32 + lane < G) acc[j] = fmaf(a, g[c2][j], acc[j]);
+                    }
+                }
+            };
+#pragma unroll 1
+            for (int bk = 0; bk < nb; bk += 2) {
+                if (bk + 1 < nb) load(gb, bk + 1);
+                compute(ga, bk);
+                if (bk + 2 < nb) load(ga, bk + 2);
+                if (bk + 1 < nb) compute(gb, bk + 1);
+            }
+            const float inv = 10.0f / fmaxf(sqrtf(nrm), 1e-12f);
+#pragma unroll
+            for (int j = 0; j < 6; ++j) {
+                const int col = g0 + j * 32 + lane;
+                if (col < G) {
+                    const float sc = L == RT_GW ? acc[j] * inv : fmaf(-2.0f, acc[j], __ldg(cnorm + col));
+                    const bool better = L == RT_GW ? (sc > best || (sc == best && col < bi)) : (sc < best || (sc == best && col < bi));
+                    if (better) {
+                        best = sc;
+                        bi = col;
+                    }
                 }
             }
+            if constexpr (!PANEL) break;
+            g0 += RT_N;
+            if (g0 >= G) break;
+            load(ga, 0);
         }
 #pragma unroll
         for (int o = 16; o >= 1; o >>= 1) {
             const float ob = __shfl_xor_sync(0xffffffffu, best, o);
             const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            const bool better = MODE == RT_GW ? (ob > best || (ob == best && oi < bi)) : (ob < best || (ob == best && oi < bi));
+            const bool better = L == RT_GW ? (ob > best || (ob == best && oi < bi)) : (ob < best || (ob == best && oi < bi));
             if (better) {
                 best = ob;
                 bi = oi;
@@ -505,19 +565,78 @@ rowsel_recheck_kernel(const float* __restrict__ x, int64_t bstride, int64_t cstr
     }
 }
 
+// GW projection over a panelled dictionary, one thread per row, after the last panel: best / second best / first index of
+// the best over the scratch's G columns, the ambiguity test of rowsel_tc_kernel, and the softmax features (bf16 act tiles
+// at kb0 with the padding columns zero, optional (B, G, N) fp32 copy) -- the single-panel epilogue, taken from the scratch.
+__global__ void __launch_bounds__(256)
+rowsel_gw_finish_kernel(const float* __restrict__ scr, int64_t M, int N, int G, int Gp, uint8_t* __restrict__ cos_act, int kblocks,
+                        int kb0, float* __restrict__ cos_cm, int32_t* __restrict__ sel, int32_t* __restrict__ recheck,
+                        int32_t* __restrict__ recheck_cnt) {
+    pdl_enter();
+    const int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (m >= M) return;
+    const float nrm = scr[m];
+    const float* v = scr + M + m;                    // word j at v[j * M]
+    float b1 = -INFINITY, b2 = -INFINITY;
+    int i1 = 0;
+    for (int j = 0; j < G; ++j) {
+        const float t = v[(int64_t)j * M];
+        if (t > b1) {
+            b2 = b1;
+            b1 = t;
+            i1 = j;
+        } else {
+            b2 = fmaxf(b2, t);
+        }
+    }
+    const float l2e = 1.4426950408889634f, nb2 = -b1 * l2e;
+    float s0 = 0.0f, s1 = 0.0f;
+    int j = 0;
+    for (; j + 1 < G; j += 2) {
+        s0 += rt_ex2(fmaf(v[(int64_t)j * M], l2e, nb2));
+        s1 += rt_ex2(fmaf(v[(int64_t)(j + 1) * M], l2e, nb2));
+    }
+    if (j < G) s0 += rt_ex2(fmaf(v[(int64_t)j * M], l2e, nb2));
+    const float rs = 1.0f / (s0 + s1);
+    const int64_t b = m / N, n = m - b * N;
+    for (int j0 = 0; j0 < Gp; j0 += 8) {
+        float e[8];
+#pragma unroll
+        for (int c = 0; c < 8; ++c) e[c] = j0 + c < G ? rt_ex2(fmaf(v[(int64_t)(j0 + c) * M], l2e, nb2)) * rs : 0.0f;
+        if (cos_act) {
+            uint8_t* tl = cos_act + (((m >> 7) * kblocks + kb0 + (j0 >> 6)) * 16384);
+            *reinterpret_cast<uint4*>(tl + sw128((uint32_t)(m & 127), (j0 >> 3) & 7)) =
+                make_uint4(pack_bf16x2(e[0], e[1]), pack_bf16x2(e[2], e[3]), pack_bf16x2(e[4], e[5]), pack_bf16x2(e[6], e[7]));
+        }
+        if (cos_cm) {
+#pragma unroll
+            for (int c = 0; c < 8; ++c)
+                if (j0 + c < G) cos_cm[(b * G + j0 + c) * N + n] = e[c];
+        }
+    }
+    sel[m] = i1;
+    if (!(b1 - b2 > 5e-3f) || !(nrm > 1e-20f)) recheck[atomicAdd(recheck_cnt, 1)] = (int32_t)m;
+}
+
 struct RtPlan {
-    size_t off_img, off_cmax, off_cnt, off_list, total;
+    size_t off_img, off_cmax, off_cnt, off_list, off_scr, total;
 };
-static RtPlan rt_plan(int64_t rows, int D) {
+// Kp > 192 (rt_run_wide): one packed image per panel and the per-row scratch the panels share -- (best, second best, index)
+// as a float4 for k-means, |x|^2 and the 10 cos of every word (column-major, (1 + Kp) x rows fp32) for the GW projection
+static RtPlan rt_plan(int64_t rows, int D, int Kp = RT_N, bool gw = false) {
+    const int panels = Kp > RT_N ? (Kp + RT_N - 1) / RT_N : 1;
     RtPlan p;
     p.off_img = 0;
-    size_t o = (size_t)(D >> 6) * 2 * RT_BTILE;
+    size_t o = (size_t)panels * (D >> 6) * 2 * RT_BTILE;
     p.off_cmax = o;
     o += 256;
     p.off_cnt = o;
     o += 256;
     p.off_list = o;
     o += (size_t)rows * 4;
+    o = (o + 255) / 256 * 256;
+    p.off_scr = o;
+    if (panels > 1) o += gw ? (size_t)(1 + Kp) * rows * 4 : (size_t)rows * 16;
     p.total = (o + 255) / 256 * 256;
     return p;
 }
@@ -555,11 +674,69 @@ static int rt_run(const char* who, const float* x, int64_t bstride, int64_t cstr
     return GFS_OK;
 }
 
+// Dictionaries of 193..512 words: panels of 192 words, each packed into its own image.  Every panel is one persistent pass
+// of rowsel_tc_kernel over all the points with that panel resident (ceil(G / 192) passes over X); k-means merges the panels
+// row by row in ascending order inside the epilogue (the last panel writes the label and applies the ambiguity bound, with
+// max|c| over all K), the GW projection writes the scores of every word and rowsel_gw_finish_kernel takes the softmax.  The
+// re-check then evaluates the pinned chains over all the words.
+template <int L>
+static int rt_run_wide(const char* who, const float* x, int64_t bstride, int64_t cstride, int D, int N, int64_t M, const float* dict_t,
+                       int G, int Gp, const float* cnorm, void* cos_act, int kblocks, int kb0, float* cos_cm, int32_t* sel, void* workspace,
+                       int64_t workspace_bytes, cudaStream_t st) {
+    const RtPlan p = rt_plan(M, D, Gp, L == RT_GW);
+    GFS_REQUIRE(workspace && workspace_bytes >= (int64_t)p.total && (reinterpret_cast<uintptr_t>(workspace) & 255) == 0, GFS_ERR_BAD_ARG,
+                "%s: workspace of %lld bytes (256-byte aligned) needed, got %lld", who, (long long)p.total, (long long)workspace_bytes);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    float* cmax2 = reinterpret_cast<float*>(ws + p.off_cmax);
+    int32_t* cnt = reinterpret_cast<int32_t*>(ws + p.off_cnt);
+    int32_t* list = reinterpret_cast<int32_t*>(ws + p.off_list);
+    float* scr = reinterpret_cast<float*>(ws + p.off_scr);
+    const int npan = (G + RT_N - 1) / RT_N;
+    const size_t pimg = (size_t)(D >> 6) * 2 * RT_BTILE;
+    const int pk = RT_N * (D >> 3);
+    for (int q = 0; q < npan; ++q) {
+        const int off = q * RT_N, w = G - off < RT_N ? G - off : RT_N;
+        launch_pdl(rowsel_pack_kernel, dim3((unsigned)((pk + 255) / 256)), dim3(256), 0, st,
+            dict_t + off, D, w, Gp, ws + q * pimg);
+        GFS_LAUNCH_OK("rowsel_pack_kernel");
+    }
+    launch_pdl(rowsel_cmax_kernel, dim3((unsigned)(1)), dim3(32), 0, st,
+        L != RT_GW ? cnorm : nullptr, G, cmax2, cnt);
+    GFS_LAUNCH_OK("rowsel_cmax_kernel");
+    const int ntiles = (int)((M + RT_ROWS - 1) / RT_ROWS);
+    const int sms = sm_count();
+    GFS_REQUIRE(sms > 0, GFS_ERR_CUDA, "%s: cannot query the device", who);
+    const size_t smem = offsetof(RtSmem, B) + pimg + sizeof(RtCtl) + 1024;
+    GFS_REQUIRE(smem <= 227 * 1024, GFS_ERR_UNSUPPORTED, "%s: D=%d: the resident dictionary panel does not fit shared memory", who, D);
+    GFS_CUDA_OK(allow_smem(reinterpret_cast<const void*>(rowsel_tc_kernel<L | RT_PANEL>), smem));
+    for (int q = 0; q < npan; ++q) {
+        const int off = q * RT_N, w = G - off < RT_N ? G - off : RT_N;
+        launch_pdl(rowsel_tc_kernel<L | RT_PANEL>, dim3((unsigned)(ntiles < sms ? ntiles : sms)), dim3(RT_THREADS), smem, st,
+            x, bstride, cstride, D, N, M, ntiles, ws + q * pimg, w, Gp, L != RT_GW ? cnorm + off : nullptr, cmax2, nullptr,
+            q == npan - 1 ? 1 : 0, off, scr, sel, list, cnt);
+        GFS_LAUNCH_OK("rowsel_tc_kernel<panel>");
+    }
+    if (L == RT_GW) {
+        launch_pdl(rowsel_gw_finish_kernel, dim3((unsigned)((M + 255) / 256)), dim3(256), 0, st,
+            scr, M, N, G, Gp, static_cast<uint8_t*>(cos_act), kblocks, kb0, cos_cm, sel, list, cnt);
+        GFS_LAUNCH_OK("rowsel_gw_finish_kernel");
+    }
+    launch_pdl(rowsel_recheck_kernel<L | RT_PANEL>, dim3((unsigned)(sms * 2)), dim3(256), 0, st,
+        x, bstride, cstride, D, N, dict_t, G, Gp, cnorm, list, cnt, sel);
+    GFS_LAUNCH_OK("rowsel_recheck_kernel<panel>");
+    return GFS_OK;
+}
+
 }  // namespace gfs
 
 extern "C" int64_t gfs_rowsel_tc_workspace_bytes(int64_t rows, int D) {
     if (rows <= 0 || D <= 0 || D % 64 != 0 || D > 192) return 0;
     return (int64_t)gfs::rt_plan(rows, D).total;
+}
+
+extern "C" int64_t gfs_rowsel_tc_workspace_bytes_kp(int64_t rows, int D, int Kp, int gw_project) {
+    if (rows <= 0 || D <= 0 || D % 64 != 0 || D > 192 || Kp <= 0 || Kp > gfs::RT_MAXK) return 0;
+    return (int64_t)gfs::rt_plan(rows, D, Kp, gw_project != 0).total;
 }
 
 extern "C" int gfs_gw_project_tc(const float* ec, int64_t ec_bstride, int B, int D, int N, const float* gp_l2t, int G, int Gp,
@@ -570,9 +747,12 @@ extern "C" int gfs_gw_project_tc(const float* ec, int64_t ec_bstride, int B, int
     GFS_REQUIRE(B > 0 && D > 0 && N > 0 && G > 0, GFS_ERR_BAD_ARG, "gfs_gw_project_tc: non-positive size");
     GFS_REQUIRE(D % 64 == 0 && D <= 192, GFS_ERR_UNSUPPORTED, "gfs_gw_project_tc: D=%d (need a multiple of 64, <= 192; use gfs_gw_project)", D);
     GFS_REQUIRE(N % 128 == 0, GFS_ERR_UNSUPPORTED, "gfs_gw_project_tc: N=%d (need a multiple of 128; use gfs_gw_project)", N);
-    GFS_REQUIRE(G <= Gp && Gp <= RT_N && Gp % 64 == 0, GFS_ERR_UNSUPPORTED, "gfs_gw_project_tc: G=%d Gp=%d (need G <= Gp <= 192, Gp %% 64 == 0)", G, Gp);
+    GFS_REQUIRE(G <= Gp && Gp <= RT_MAXK && Gp % 64 == 0, GFS_ERR_UNSUPPORTED, "gfs_gw_project_tc: G=%d Gp=%d (need G <= Gp <= 512, Gp %% 64 == 0)", G, Gp);
     GFS_REQUIRE((reinterpret_cast<uintptr_t>(cosine_act) & 15) == 0, GFS_ERR_BAD_ARG, "gfs_gw_project_tc: cosine_act must be 16-byte aligned");
     if (cosine_act) GFS_REQUIRE(kb0 >= 0 && kb0 + Gp / 64 <= kblocks, GFS_ERR_BAD_ARG, "gfs_gw_project_tc: output blocks out of range");
+    if (Gp > RT_N)
+        return rt_run_wide<RT_GW>("gfs_gw_project_tc", ec, ec_bstride, N, D, N, (int64_t)B * N, gp_l2t, G, Gp, nullptr, cosine_act, kblocks, kb0,
+                                  cosine_cm, assignment, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
     return rt_run<RT_GW>("gfs_gw_project_tc", ec, ec_bstride, N, D, N, (int64_t)B * N, gp_l2t, G, Gp, nullptr, cosine_act, kblocks, kb0, cosine_cm,
                          assignment, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
@@ -585,11 +765,18 @@ extern "C" int gfs_kmeans_assign_tc(const float* X, int64_t n, int64_t ld, int p
     GFS_REQUIRE(point_major ? ld == D : ld >= n, GFS_ERR_BAD_ARG, "gfs_kmeans_assign_tc: leading dimension %lld does not fit the layout", (long long)ld);
     GFS_REQUIRE(n < (int64_t)1 << 31, GFS_ERR_UNSUPPORTED, "gfs_kmeans_assign_tc: n=%lld exceeds 2^31 per shard", (long long)n);
     GFS_REQUIRE(D % 64 == 0 && D <= 192, GFS_ERR_UNSUPPORTED, "gfs_kmeans_assign_tc: D=%d (need a multiple of 64, <= 192; use gfs_kmeans_assign)", D);
-    GFS_REQUIRE(K <= Kp && Kp <= RT_N, GFS_ERR_UNSUPPORTED, "gfs_kmeans_assign_tc: K=%d Kp=%d (need K <= Kp <= 192)", K, Kp);
+    GFS_REQUIRE(K <= Kp && Kp <= RT_MAXK, GFS_ERR_UNSUPPORTED, "gfs_kmeans_assign_tc: K=%d Kp=%d (need K <= Kp <= 512)", K, Kp);
     GFS_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15) == 0, GFS_ERR_BAD_ARG, "gfs_kmeans_assign_tc: X must be 16-byte aligned");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     sqnorm_kernel<<<dim3((Kp + 255) / 256, 1), 256, 0, st>>>(centers_t, 0, D, Kp, cnorm);
     GFS_LAUNCH_OK("sqnorm_kernel");
+    if (Kp > RT_N) {
+        if (point_major)
+            return rt_run_wide<RT_KMEANS_PM>("gfs_kmeans_assign_tc", X, 0, 1, D, 1, n, centers_t, K, Kp, cnorm, nullptr, 0, 0, nullptr, labels,
+                                             workspace, workspace_bytes, st);
+        return rt_run_wide<RT_KMEANS>("gfs_kmeans_assign_tc", X, 0, ld, D, 1, n, centers_t, K, Kp, cnorm, nullptr, 0, 0, nullptr, labels,
+                                      workspace, workspace_bytes, st);
+    }
     if (point_major)
         return rt_run<RT_KMEANS_PM>("gfs_kmeans_assign_tc", X, 0, 1, D, 1, n, centers_t, K, Kp, cnorm, nullptr, 0, 0, nullptr, labels, workspace,
                                     workspace_bytes, st);

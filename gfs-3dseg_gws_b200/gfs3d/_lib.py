@@ -67,7 +67,9 @@ UTILITIES = {"gfs_version": (_i, []), "gfs_last_error_string": (ctypes.c_char_p,
              "gfs_kmeans_inertia_partials": (_i, []),
              "gfs_knn_tc_workspace_bytes": (_i64, [_i, _i, _i]),
              "gfs_knn_tc_chains": (_i, [_i, _i, _i]), "gfs_knn_tc_set_split": (_i, [_i]),
-             "gfs_rowsel_tc_workspace_bytes": (_i64, [_i64, _i])}
+             "gfs_rowsel_tc_workspace_bytes": (_i64, [_i64, _i]),
+             "gfs_rowsel_tc_workspace_bytes_kp": (_i64, [_i64, _i, _i, _i]),
+             "gfs_kmeans_accumulate_ranges": (_i, [_i, _i, _i])}
 
 _lib = None
 

@@ -40,6 +40,20 @@ def label_gw_histogram(assignment: torch.Tensor, labels: torch.Tensor, num_label
     return ops.joint_histogram(labels, assignment, num_labels, G, out=out)
 
 
+def block_gw_histogram(blk: torch.Tensor, assignment: torch.Tensor, b: int, G: int) -> torch.Tensor:
+    """H[i, g] = number of points of block i (blk == i; -1 = not counted) assigned to word g, (b, G) int64.  The histogram
+    kernel holds at most 12 288 bins (b * G = 16 384 at 32 blocks of 512 words): the blocks go in groups that fit, each group
+    a pass over the labels with its own block range, so the counts are those of one call."""
+    per = max(1, ops.JOINT_HISTOGRAM_MAXBINS // G)
+    if b <= per:
+        return ops.joint_histogram(blk, assignment, b, G)
+    H = torch.zeros(b, G, dtype=torch.int64, device=assignment.device)
+    for i0 in range(0, b, per):
+        nb = min(per, b - i0)
+        ops.joint_histogram(blk - i0, assignment, nb, G, out=H[i0:i0 + nb])
+    return H
+
+
 def collect_base_class_gp_coding_sum(model, train_loader, train_class, energy):
     """train.py:156-218.  train_loader yields (input (b, d, n), target (b, n), segment_label) with ANY batch size (the
     reference needs bs = 1).  Returns (base_class_gp_coding (num_base, G) multi-hot, bg_class_coding (G,)) on the device."""
@@ -61,7 +75,7 @@ def collect_base_class_gp_coding_sum(model, train_loader, train_class, energy):
             # background: one mean one-hot vector per BLOCK (train.py:186-191) = per-block histogram / count
             blk = torch.arange(b, device=input.device, dtype=torch.int32).unsqueeze(1).expand(b, n)
             blk = torch.where(target == 0, blk, torch.full_like(blk, -1))
-            hb = ops.joint_histogram(blk, assignment, b, G)
+            hb = block_gw_histogram(blk, assignment, b, G)
             cnt = hb.sum(dim=1)
             for i in range(b):
                 if int(cnt[i]) > 0:
@@ -114,7 +128,7 @@ def get_new_proto_Geo2SemProto(val_supp_loader, model, base_num=16, novel_num=5,
             cnt = fg.sum(dim=1)
             feat = (point_feat * fg.unsqueeze(1)).sum(dim=2) / cnt.unsqueeze(1)      # mean over the foreground points
             blk = torch.arange(b, device=input.device, dtype=torch.int32).unsqueeze(1).expand(b, n)
-            hist = ops.joint_histogram(torch.where(fg, blk, torch.full_like(blk, -1)), assignment, b, G)
+            hist = block_gw_histogram(torch.where(fg, blk, torch.full_like(blk, -1)), assignment, b, G)
             for i in range(b):
                 c = int(cls_id[i])
                 new_cls_feat_dict[c].append(feat[i:i + 1])

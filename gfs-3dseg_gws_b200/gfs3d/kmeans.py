@@ -4,6 +4,11 @@ Lloyd iterations run on the GPU: gfs_kmeans_assign (fp32 pinned-order E-step) + 
 sums) per iteration; the control flow mirrors sklearn 1.9.0 (_kmeans.py:1487-1490 mean-centring, :289-296 tolerance,
 :630-759 Lloyd loop / convergence, _k_means_common.pyx:167-260 empty-cluster relocation and centre averaging).
 
+Up to 512 clusters with at most 192 features (up to 192 clusters with 193..256 features).  Beyond 192 clusters the E-step
+runs the panelled tensor-core path, which needs a multiple of 64 channels: the channel-major copies of the points and the
+centres then carry zero channels up to the next multiple of 64, which leave the pinned fp32 chains (and so the labels)
+unchanged, since fmaf(0, 0, s) == s.
+
 Multi-GPU: pass `process_group` (or have torch.distributed initialised and shard=True): X is then THIS rank's shard of
 the points; the only exchange per iteration is an NCCL all-reduce of the (K*D + K) fp64 sums/counts (+ the mean/variance
 once), every rank applies the identical centroid update.
@@ -223,12 +228,14 @@ class KMeans:
         """sample_weight: None or (n,) non-negative finite weights (numpy or tensor), cast to float32; with shard=True, the
         weights of this rank's shard.  Mean-centring and the tolerance stay unweighted, as in sklearn."""
         w_in = self._check_weight(sample_weight, X.shape[0])
+        K = self.n_clusters
+        if K > 512:
+            raise NotImplementedError(f"n_clusters={K} > 512 is not built")
+        if K > 192 and X.shape[1] > 192:
+            raise NotImplementedError(f"n_clusters={K} > 192 with {X.shape[1]} > 192 features is not built")
         dev = torch.device(self.device) if self.device is not None else torch.device("cuda", torch.cuda.current_device())
         Xd = self._as_device(X, dev)
         n, D = Xd.shape
-        K = self.n_clusters
-        if K > 192:
-            raise NotImplementedError(f"n_clusters={K} > 192 is not built")
         runs = self._n_runs()
         w = w_in.to(dev) if w_in is not None else None
         if w is not None and self.shard:
@@ -247,15 +254,15 @@ class KMeans:
         mean32 = mean.float()
         Xc = Xd - mean32
         npad = (n + 3) // 4 * 4
-        xt = torch.zeros(D, npad, dtype=torch.float32, device=dev)
-        xt[:, :n] = Xc.t()
+        xt = torch.zeros(self._e_channels(D), npad, dtype=torch.float32, device=dev)   # E-step copy; xt[:D] is the data
+        xt[:D, :n] = Xc.t()
 
         rng = self._rng() if isinstance(self.init, str) else None
         best = None
         for _ in range(runs):
             # initial centres
             if isinstance(self.init, str) and self.init == "k-means++":
-                centers = self._seed_plusplus(Xc, xt, rng, n, w=w)
+                centers = self._seed_plusplus(Xc, xt[:D], rng, n, w=w)
             elif isinstance(self.init, str) and self.init == "random":
                 centers = self._seed_random(Xc, rng, n, w=w)
             elif isinstance(self.init, (np.ndarray, torch.Tensor)):
@@ -283,6 +290,11 @@ class KMeans:
         self.centers_centered_ = centers               # ... against these: cluster_centers_ - mean does not round back to them
         return self
 
+    def _e_channels(self, D):
+        """channels of the E-step's channel-major copies: D, or D padded with zeros to a multiple of 64 for the panelled
+        tensor-core path (n_clusters > 192)"""
+        return (D + 63) // 64 * 64 if self.n_clusters > 192 else D
+
     def _same_clustering(self, a, b):
         """sklearn _k_means_common.pyx:_is_same_clustering (every label of a maps to one label of b), over all shards"""
         K = self.n_clusters
@@ -300,8 +312,8 @@ class KMeans:
         # (labels changed, centre shift, empty clusters).  All buffers are allocated once.  Unweighted, the weight sums are
         # the counts, which pack copies into their slot; weighted, the M-step writes them there.
         Kp = (K + 3) // 4 * 4
-        ct = torch.zeros(D, Kp, dtype=torch.float32, device=dev)
-        ct[:, :K] = centers.t()
+        ct = torch.zeros(xt.shape[0], Kp, dtype=torch.float32, device=dev)
+        ct[:D, :K] = centers.t()
         centers = centers.contiguous()
         centers_new = torch.empty_like(centers)
         labels_old = torch.full((npad,), -1, dtype=torch.int32, device=dev)
@@ -339,7 +351,7 @@ class KMeans:
                 new = torch.where(gw[:, None] > 0, gsums / torch.where(gw > 0, gw, 1.0)[:, None], torch.zeros_like(gsums)).float()
                 shift_h = float(((new - centers).double() ** 2).sum())
                 centers_new.copy_(new)
-                ct[:, :K] = new.t()
+                ct[:D, :K] = new.t()
             centers, centers_new = centers_new, centers
             if self.verbose:
                 print(f"Iteration {n_iter - 1}, center shift {shift_h:.6g}")
@@ -411,10 +423,11 @@ class KMeans:
         if D != self.n_features_in_:
             raise ValueError(f"X has {D} features, the model was fitted with {self.n_features_in_}")
         K = self.n_clusters
-        xt = torch.zeros(D, (n + 3) // 4 * 4, dtype=torch.float32, device=dev)
-        xt[:, :n] = Xc.t()
-        ct = torch.zeros(D, (K + 3) // 4 * 4, dtype=torch.float32, device=dev)
-        ct[:, :K] = self.centers_centered_.t()
+        De = self._e_channels(D)
+        xt = torch.zeros(De, (n + 3) // 4 * 4, dtype=torch.float32, device=dev)
+        xt[:D, :n] = Xc.t()
+        ct = torch.zeros(De, (K + 3) // 4 * 4, dtype=torch.float32, device=dev)
+        ct[:D, :K] = self.centers_centered_.t()
         return Xc.contiguous(), ops.kmeans_assign(xt, ct, K)[:n]
 
     def predict(self, X):

@@ -224,6 +224,7 @@ def attention(qkv_act: torch.Tensor, kb_q: int, B: int, N: int, scale: float, y_
 
 
 ROWSEL_IMPL = os.environ.get("GFS3D_ROWSEL", "auto")   # "auto" | "tc" | "fp32": identical assignments / labels
+ROWSEL_TC_MAXK = 512      # dictionary width of the tensor-core path (> 192: panelled); the fp32 kernels stop at 192
 
 
 def gw_project(ec: torch.Tensor, gp_l2t: torch.Tensor, G: int, cosine_act: Optional[torch.Tensor] = None, kb0: int = 0,
@@ -231,7 +232,7 @@ def gw_project(ec: torch.Tensor, gp_l2t: torch.Tensor, G: int, cosine_act: Optio
     """ec (B, D, N) cm fp32; gp_l2t (D, Gp) -> assignment (B, N) int32 [, cosine_feat (B, G, N) fp32]
 
     impl "tc": tcgen05 product + pinned fp32 re-check of near-ties (gfs_gw_project_tc); "fp32": the all-fp32 kernel
-    (gfs_gw_project); "auto": tc whenever the shape is eligible.  The assignments are identical."""
+    (gfs_gw_project, Gp <= 192); "auto": tc whenever the shape is eligible (Gp <= 512).  The assignments are identical."""
     _need_cuda(ec, gp_l2t, cosine_act)
     B, D, N = ec.shape
     assert ec.stride(2) == 1 and ec.stride(1) == N and gp_l2t.is_contiguous() and gp_l2t.shape[0] == D
@@ -239,8 +240,8 @@ def gw_project(ec: torch.Tensor, gp_l2t: torch.Tensor, G: int, cosine_act: Optio
     assign = torch.empty(B, N, dtype=torch.int32, device=ec.device)
     cm = torch.empty(B, G, N, dtype=torch.float32, device=ec.device) if want_cm else None
     impl = impl or ROWSEL_IMPL
-    if impl == "tc" or (impl == "auto" and D % 64 == 0 and D <= 192 and N % 128 == 0 and Gp <= 192 and Gp % 64 == 0):
-        nbytes = int(lib().gfs_rowsel_tc_workspace_bytes(B * N, D))
+    if impl == "tc" or (impl == "auto" and D % 64 == 0 and D <= 192 and N % 128 == 0 and Gp <= ROWSEL_TC_MAXK and Gp % 64 == 0):
+        nbytes = int(lib().gfs_rowsel_tc_workspace_bytes_kp(B * N, D, Gp, 1))
         ws = torch.empty(nbytes, dtype=torch.uint8, device=ec.device)
         _call("gfs_gw_project_tc", 4, _ptr(ec), ec.stride(0), B, D, N, _ptr(gp_l2t), G, Gp, _ptr(cosine_act),
               0 if cosine_act is None else cosine_act.shape[1], kb0, _ptr(cm), _ptr(assign), _ptr(ws), nbytes, _stream())
@@ -279,6 +280,9 @@ def refine_proto(pred_proto: torch.Tensor, proto: torch.Tensor, gened: torch.Ten
     out = torch.empty(B, CLS, D, dtype=torch.float32, device=pp.device)
     _call("gfs_refine_proto", 1, _ptr(pp), _ptr(q), _ptr(g), B, CLS, D, int(base_num), _ptr(out), _stream())
     return out
+
+
+JOINT_HISTOGRAM_MAXBINS = 12288   # na * nb of one gfs_joint_histogram_i32 call
 
 
 def joint_histogram(a: torch.Tensor, b: torch.Tensor, na: int, nb: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -330,7 +334,8 @@ def kmeans_assign(xt: torch.Tensor, centers_t: torch.Tensor, K: int, want_score:
     """xt (D, n) fp32, centers_t (D, Kp) fp32 zero padded -> labels (n) int32
 
     impl "tc": tcgen05 product + pinned fp32 re-check of near-ties (gfs_kmeans_assign_tc); "fp32": gfs_kmeans_assign;
-    "auto": tc when the shape is eligible and no scores are requested.  The labels are identical."""
+    "auto": tc when the shape is eligible (Kp <= 512) and no scores are requested; "fp32" and scores stop at Kp = 192.
+    The labels are identical."""
     _need_cuda(xt, centers_t)
     D, n = xt.shape
     assert xt.is_contiguous() and centers_t.is_contiguous() and centers_t.shape[0] == D
@@ -339,8 +344,8 @@ def kmeans_assign(xt: torch.Tensor, centers_t: torch.Tensor, K: int, want_score:
     labels = torch.empty(n, dtype=torch.int32, device=xt.device)
     score = torch.empty(n, dtype=torch.float32, device=xt.device) if want_score else None
     impl = impl or ROWSEL_IMPL
-    if (impl == "tc" or (impl == "auto" and D % 64 == 0 and D <= 192 and Kp <= 192)) and not want_score:
-        nbytes = int(lib().gfs_rowsel_tc_workspace_bytes(n, D))
+    if (impl == "tc" or (impl == "auto" and D % 64 == 0 and D <= 192 and Kp <= ROWSEL_TC_MAXK)) and not want_score:
+        nbytes = int(lib().gfs_rowsel_tc_workspace_bytes_kp(n, D, Kp, 0))
         ws = torch.empty(nbytes, dtype=torch.uint8, device=xt.device)
         _call("gfs_kmeans_assign_tc", 6, _ptr(xt), n, n, 0, D, _ptr(centers_t), K, Kp, _ptr(cnorm), _ptr(labels), _ptr(ws), nbytes, _stream())
     else:
@@ -357,7 +362,7 @@ def kmeans_assign_rows(X: torch.Tensor, centers_t: torch.Tensor, K: int) -> torc
     Kp = centers_t.shape[1]
     cnorm = torch.empty(Kp, dtype=torch.float32, device=X.device)
     labels = torch.empty(n, dtype=torch.int32, device=X.device)
-    nbytes = int(lib().gfs_rowsel_tc_workspace_bytes(n, D))
+    nbytes = int(lib().gfs_rowsel_tc_workspace_bytes_kp(n, D, Kp, 0))
     ws = torch.empty(nbytes, dtype=torch.uint8, device=X.device)
     _call("gfs_kmeans_assign_tc", 6, _ptr(X), n, D, 1, D, _ptr(centers_t), K, Kp, _ptr(cnorm), _ptr(labels), _ptr(ws), nbytes, _stream())
     return labels
@@ -385,7 +390,8 @@ def kmeans_accumulate(X: torch.Tensor, labels: torch.Tensor, K: int, n_valid: Op
 
 
 def kmeans_accumulate_workspace(K: int, D: int, device):
-    P = lib().gfs_kmeans_partials()
+    """(partial (P*K*D) fp32, pcount (P*K) int32) for the P point ranges of gfs_kmeans_accumulate's grid"""
+    P = lib().gfs_kmeans_accumulate_ranges(K, D, 0)
     return (torch.empty(P * K * D, dtype=torch.float32, device=device), torch.empty(P * K, dtype=torch.int32, device=device))
 
 
@@ -414,7 +420,7 @@ def kmeans_accumulate_weighted(X: torch.Tensor, labels: torch.Tensor, weights: t
 
 
 def kmeans_accumulate_weighted_workspace(K: int, D: int, device):
-    P = lib().gfs_kmeans_partials()
+    P = lib().gfs_kmeans_accumulate_ranges(K, D, 1)
     return (torch.empty(P * K * D, dtype=torch.float32, device=device), torch.empty(P * K, dtype=torch.float64, device=device))
 
 

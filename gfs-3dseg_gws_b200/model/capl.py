@@ -57,10 +57,10 @@ class mpti_net_Point_GeoAsWeight_v2(nn.Module):
         if self._folded.key != key:
             G = self.gp.shape[0]
             sem = self.feat_dim
-            if sem != 192 or self.encoder.n_edgeconv * 64 != self.gp.shape[1] or G > 192:
+            if sem != 192 or self.encoder.n_edgeconv * 64 != self.gp.shape[1] or G > 512:
                 raise NotImplementedError(
                     f"head shapes (feat_dim={sem}, GW basis {tuple(self.gp.shape)}) are outside what the sm_100a head is built for "
-                    "(feat_dim 192, <=192 geometric words of width 64*n_edgeconv)")
+                    "(feat_dim 192, <=512 geometric words of width 64*n_edgeconv)")
             with torch.no_grad():
                 Gp = (G + 63) // 64 * 64
                 gp_l2 = F.normalize(self.gp.detach().float().to(device), p=2, dim=1)            # (G, D)

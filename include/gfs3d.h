@@ -207,9 +207,14 @@ int gfs_kmeans_assign(const float* xt, int64_t n, int D, const float* centers_t,
 /* The same two results on tcgen05 (gfs-3dseg_gws_b200/csrc/rowsel_tc.cu): bf16 hi/lo split product with fp32 accumulation in
  * TMEM; rows whose best and second best score are closer than the product's error bound are re-evaluated with the pinned fp32
  * chain, so the assignment / label is the one gfs_gw_project / gfs_kmeans_assign return, bit for bit; the GW softmax features
- * (bf16 act tiles, 2e-2 tolerance) come from the tensor-core values.  D % 64 == 0, D <= 192, <= 192 entries; GW: N % 128 == 0.
- * workspace: gfs_rowsel_tc_workspace_bytes(rows, D) bytes, 256-byte aligned (packed dictionary image, re-check list).        */
+ * (bf16 act tiles, 2e-2 tolerance) come from the tensor-core values.  D % 64 == 0, D <= 192, <= 512 entries; GW: N % 128 == 0.
+ * Up to 192 entries the dictionary stays resident in shared memory; 193..512 run in panels of 192 entries, one pass over the
+ * points per panel, with the panels merged in ascending order (ties still go to the lowest index over all entries).
+ * workspace: gfs_rowsel_tc_workspace_bytes_kp(rows, D, Kp, gw_project) bytes, 256-byte aligned (packed dictionary images,
+ * re-check list and, for Kp > 192, the panels' per-row scratch: 16 bytes a row for k-means, (1 + Kp) floats a row for the GW
+ * projection).  gfs_rowsel_tc_workspace_bytes(rows, D) is the same size for Kp <= 192.                                     */
 int64_t gfs_rowsel_tc_workspace_bytes(int64_t rows, int D);
+int64_t gfs_rowsel_tc_workspace_bytes_kp(int64_t rows, int D, int Kp, int gw_project);
 int gfs_gw_project_tc(const float* ec, int64_t ec_bstride, int B, int D, int N, const float* gp_l2t, int G, int Gp,
                       void* cosine_act, int kblocks, int kb0, float* cosine_cm, int32_t* assignment,
                       void* workspace, int64_t workspace_bytes, void* stream);
@@ -218,14 +223,18 @@ int gfs_gw_project_tc(const float* ec, int64_t ec_bstride, int B, int D, int N, 
 int gfs_kmeans_assign_tc(const float* X, int64_t n, int64_t ld, int point_major, int D, const float* centers_t, int K, int Kp,
                          float* cnorm, int32_t* labels, void* workspace, int64_t workspace_bytes, void* stream);
 /* deterministic centroid sums over X (n, D) row-major: partial (P, K, D) fp32 + pcount (P, K) int32 workspaces with
- * P = gfs_kmeans_partials() (one per SM); sums (K, D) fp64 and counts (K) int64 are reduced in a fixed order.       */
+ * P = gfs_kmeans_accumulate_ranges(K, D, 0) point ranges; sums (K, D) fp64 and counts (K) int64 are reduced in a fixed order.
+ * P = gfs_kmeans_partials() (one range per SM) while the K x D fp32 table fits shared memory; a larger table (K = 512 at
+ * D = 192) is split over the fewest CTAs per range that fit, each adding the points of its slice of centres in ascending
+ * order, so the sums are those one undivided table would hold.                                                        */
 int gfs_kmeans_partials(void);
+int gfs_kmeans_accumulate_ranges(int K, int D, int weighted);
 int gfs_kmeans_accumulate(const float* X, int64_t n, int D, const int32_t* labels, int K,
                           float* partial, int32_t* pcount, double* sums, int64_t* counts, void* stream);
 /* weighted M-step sums (sklearn _k_means_lloyd.pyx:216-218): sums[l] += x * w (an fp32 product, then an fp32 add; no fused
  * multiply-add) in the same ascending, pairwise order as gfs_kmeans_accumulate, so weights of 1 give its sums bit for bit;
  * wsums[l] += w in fp64, ascending point order per CTA.  weights (n) fp32; partial (P, K, D) fp32 and pweight (P, K) fp64
- * workspaces, P = gfs_kmeans_partials(); sums (K, D) and wsums (K) fp64 are reduced in CTA order.  wsums may be the weight
+ * workspaces, P = gfs_kmeans_accumulate_ranges(K, D, 1); sums (K, D) and wsums (K) fp64 are reduced in range order.  wsums may be the weight
  * slot packed[K*D : K*D+K] of gfs_kmeans_pack's buffer.                                                               */
 int gfs_kmeans_accumulate_weighted(const float* X, int64_t n, int D, const int32_t* labels, const float* weights, int K,
                                    float* partial, double* pweight, double* sums, double* wsums, void* stream);

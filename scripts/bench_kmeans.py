@@ -5,6 +5,8 @@
     torchrun --nproc-per-node N scripts/bench_kmeans.py --n 4000000   (points sharded over N GPUs, NCCL all-reduce)
     python scripts/bench_kmeans.py --weighted [--n 4194304]          (one GPU: weighted vs unweighted Lloyd iteration,
                                                                       the inertia pass, weighted k-means++ seeding)
+    python scripts/bench_kmeans.py --clusters 150,256,512 --n 4000000  (one GPU: Lloyd iteration and E-step alone per K, the
+                                                                      GW projection at G = 150 / 256 / 512 over 32 x 2048 rows)
 
 Prints one JSON line: ms per Lloyd iteration (E-step + M-step + all-reduce), kernel times, achieved GB/s / TFLOP/s,
 and sklearn's Lloyd iteration on a bounded sample of the host cores for comparison."""
@@ -27,6 +29,8 @@ ap.add_argument("--n", type=int, default=500000)
 ap.add_argument("--iters", type=int, default=10)
 ap.add_argument("--cpu-sample", type=int, default=200000)
 ap.add_argument("--weighted", action="store_true", help="time the sample_weight path against the unweighted one (one GPU)")
+ap.add_argument("--clusters", default=None, help="comma-separated K: time one Lloyd iteration (E + M) and the E-step alone per K, "
+                "and the GW projection at the same widths (one GPU)")
 a = ap.parse_args()
 world, rank, local = int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0))
 torch.cuda.set_device(local)
@@ -127,6 +131,69 @@ def bench_weighted():
                       "points": n, "centroids": K, "dim": D, "gpu": torch.cuda.get_device_name(dev),
                       "nvidia_smi_name_power_limit": smi}))
 
+
+def bench_clusters(ks):
+    """K beyond 192 runs the panelled E-step (ceil(K / 192) passes over X) and, past the shared-memory table, the centre-split
+    M-step.  Per K: KMeans' E-step (gfs_kmeans_assign_tc) alone and a whole Lloyd iteration as the fit issues it (E-step,
+    M-step sums, pack, centre update, one read); then gfs_gw_project_tc with act tiles at B x N = 32 x 2048 and G = K.
+    X (n x 192 fp32, 3 GB at 4 M points) is far larger than L2.  Prints the card and its power limit."""
+    import subprocess
+    import torch.nn.functional as F
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                         capture_output=True, text=True).stdout.strip()
+
+    def timed(fn, reps):
+        fn()
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(reps):
+            fn()
+        e1.record()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / reps
+
+    out = {"metric": "kmeans_wide_dictionary_ms", "points": n, "dim": D, "gpu": torch.cuda.get_device_name(dev),
+           "nvidia_smi_name_power_limit_max_sm_clock": smi, "kmeans": {}, "gw_project": {}}
+    for k in ks:
+        kp = (k + 3) // 4 * 4
+        c = X[torch.randperm(n, device=dev, generator=g)[:k]].clone()
+        ct = torch.zeros(D, kp, device=dev)
+        ct[:, :k] = c.t()
+        packed = torch.empty(k * D + k + 1, dtype=torch.float64, device=dev)
+        sums = packed[:k * D].view(k, D)
+        counts = torch.empty(k, dtype=torch.int64, device=dev)
+        ws = ops.kmeans_accumulate_workspace(k, D, dev)
+        scratch = torch.zeros(2, dtype=torch.int64, device=dev)
+        result = torch.empty(3, dtype=torch.float64, device=dev)
+        cnew, lold = torch.empty_like(c), torch.full((n,), -1, dtype=torch.int32, device=dev)
+
+        def iteration():
+            labels = ops.kmeans_assign(xt, ct, k)
+            ops.kmeans_accumulate(X, labels, k, sums=sums, counts=counts, ws=ws)
+            ops.kmeans_pack(labels, lold, n, k, D, packed, scratch, counts=counts)
+            ops.kmeans_update(packed, c, k, D, kp, cnew, ct.clone(), result)
+            result.tolist()
+        labels = ops.kmeans_assign(xt, ct, k)
+        e_ms = timed(lambda: ops.kmeans_assign(xt, ct, k), a.iters)
+        m_ms = timed(lambda: ops.kmeans_accumulate(X, labels, k, sums=sums, counts=counts, ws=ws), a.iters)
+        out["kmeans"][k] = {"lloyd_iteration_ms": timed(iteration, a.iters), "estep_ms": e_ms, "mstep_ms": m_ms,
+                            "estep_passes_over_x": (kp + 191) // 192 if kp > 192 else 1}
+    B, N = 32, 2048
+    ec = torch.randn(B, D, N, device=dev, generator=g)
+    for G in ks:
+        Gp = (G + 63) // 64 * 64
+        gp_l2t = torch.zeros(D, Gp, device=dev)
+        gp_l2t[:, :G] = F.normalize(torch.randn(G, D, device=dev, generator=g), dim=1).t()
+        act = ops.new_act(B * N, 3 + Gp // 64, dev)
+        out["gw_project"][G] = {"ms": timed(lambda: ops.gw_project(ec, gp_l2t, G, cosine_act=act, kb0=3), 20), "rows": B * N}
+    print(json.dumps(out))
+
+
+if a.clusters:
+    assert world == 1, "--clusters runs on one GPU"
+    bench_clusters([int(v) for v in a.clusters.split(",")])
+    sys.exit(0)
 
 if a.weighted:
     assert world == 1, "--weighted runs on one GPU"
